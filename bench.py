@@ -2,6 +2,7 @@
 """bench.py — env-steps/sec of the batched gripper environment (BASELINE.json metric) on N B200s of one node.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5] [--scene acorn] [--envs 4096]
+                   [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], `--config 2`): acorn_env (stand-in mesh, see DESIGN.md), 4 096 environments per GPU,
 actions U(-1,1)^6 from a seeded generator, physics + reward + observation, auto-reset on.  One "step" = one VecEnv.step over
@@ -68,7 +69,11 @@ def parse():
     ap.add_argument("--policy", action="store_true", default=None, help="actions from the tensor-core policy forward on the previous observation "
                     "(device-resident rollout loop, BASELINE.json configs[3]) instead of a random tape")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target wall time of the CPU sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0's environments) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     preset = CONFIGS[a.config or 2]
     for k, v in preset.items():
         if getattr(a, k) is None:
@@ -199,6 +204,35 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------------------------- our arm
+DUMP_ROWS, DUMP_IMAGES = 65536, 256  # environments whose records / images --dump-outputs writes: <= 14 + 2 x 21 MB as float32
+
+
+def dump_outputs(out_dir, sim, action):
+    """Writes what the last sim.step returned to its caller as float32 / float64 DIR/<name>.npy: the per-environment records
+    of up to DUMP_ROWS environments, the observations of up to DUMP_IMAGES, and the terminal observations of up to
+    DUMP_IMAGES of the environments that finished in that step (terminal_obs_env: their indices), each a fixed seeded
+    sample when there are more.  `action` is the policy's action of that step (None when the actions came from the tape,
+    which is an input)."""
+    import torch
+    N = sim.num_envs
+    rng = np.random.default_rng(0)
+
+    def sample(idx, n):
+        return np.sort(rng.choice(idx, n, replace=False)) if len(idx) > n else idx
+
+    rows, imgs = sample(np.arange(N), DUMP_ROWS), sample(np.arange(N), DUMP_IMAGES)
+    fin = sample(np.nonzero(sim.done.cpu().numpy())[0], DUMP_IMAGES)
+    rows, imgs, fin_t = [torch.as_tensor(i, device=sim.device) for i in (rows, imgs, fin)]
+    out = {"obs": sim.obs[imgs], "terminal_obs": sim.terminal_obs[fin_t], "reward": sim.reward[rows], "done": sim.done[rows],
+           "achieved_goal": sim.achieved_goal[rows], "desired_goal": sim.desired_goal[rows], "info": sim.info[rows]}
+    if action is not None:
+        out["action"] = action[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "terminal_obs_env.npy"), fin.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -272,6 +306,8 @@ def run_ours(args):
     dev_ms = float(step_ms.sum())
     kernel_ms = sim.step_kernel_ms(reset=True)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sim, pol_act if args.policy else None)
     sub_k_h, chain_k_h = sub_k.cpu().numpy(), chain_k.cpu().numpy()
     q = max(1, K // 4)  # the last quarter of the timed window
     # ---- policy forward alone on the last observation (tensor roofline): CUDA events on the launching stream, L2 flushed

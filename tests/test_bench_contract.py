@@ -46,6 +46,41 @@ def test_action_tapes():
     np.testing.assert_array_equal(bench.shape_actions(u.copy(), "uniform"), u)
 
 
+def test_dump_outputs_writes_float32_samples_of_the_last_step(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import types
+    import numpy as np
+    import torch
+    import bench
+    monkeypatch.setattr(bench, "DUMP_ROWS", 100)
+    N, g = 900, torch.Generator().manual_seed(0)
+    sim = types.SimpleNamespace(num_envs=N, device=torch.device("cpu"), reward=torch.rand(N, generator=g), done=(torch.arange(N) % 3 == 0).to(torch.uint8),
+                                obs=torch.randint(0, 256, (N, 5, 64, 64), generator=g, dtype=torch.uint8),
+                                terminal_obs=torch.randint(1, 256, (N, 5, 64, 64), generator=g, dtype=torch.uint8),
+                                achieved_goal=torch.rand(N, 2, generator=g), desired_goal=torch.rand(N, 2, generator=g), info=torch.rand(N, 40, generator=g))
+    action = torch.rand(N, 6, generator=g)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), sim, action)
+    names = ["achieved_goal", "action", "desired_goal", "done", "info", "obs", "reward", "terminal_obs", "terminal_obs_env"]
+    assert sorted(p.stem for p in (tmp_path / "a").iterdir()) == names
+    out = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in names}
+    for n in names:
+        assert out[n].dtype == (np.float64 if n == "terminal_obs_env" else np.float32)
+        np.testing.assert_array_equal(out[n], np.load(tmp_path / "b" / (n + ".npy")))  # the sample is fixed
+    assert out["obs"].shape == (256, 5, 64, 64) and out["info"].shape == (100, 40) and out["action"].shape == (100, 6)
+    rows = [int(np.nonzero((sim.info.numpy() == r).all(1))[0][0]) for r in out["info"]]
+    assert rows == sorted(set(rows))
+    np.testing.assert_array_equal(out["reward"], sim.reward.numpy()[rows])
+    np.testing.assert_array_equal(out["action"], action.numpy()[rows])
+    # terminal observations: a sample of the 300 environments that finished in that step, with their indices
+    fin = out["terminal_obs_env"].astype(np.int64)
+    assert len(fin) == 256 and np.all(fin % 3 == 0) and np.all(np.diff(fin) > 0)
+    np.testing.assert_array_equal(out["terminal_obs"], sim.terminal_obs.numpy()[fin])
+    sim.done.zero_()
+    bench.dump_outputs(str(tmp_path / "c"), sim, None)
+    assert np.load(tmp_path / "c" / "terminal_obs.npy").shape == (0, 5, 64, 64) and not (tmp_path / "c" / "action.npy").exists()
+
+
 def test_gpu_arm_has_no_cpu_fallback():
     import torch
     if torch.cuda.is_available():

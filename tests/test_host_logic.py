@@ -1,7 +1,7 @@
 """CPU: host-side logic of the VecEnv mirror (no GPU, no native calls): the lazily built `infos` (robot_env.py:226-241
 keys, SB3's terminal_observation / TimeLimit.truncated / Monitor episode record), the spaces (sensor.py:12-54,
 actuator.py:217-247), the target direction (robot_env.py:30-33, 46-54) and compute_reward (robot_env.py:243-273,
-reward.py:18-41) against the reference's own Reward class where it can be imported."""
+reward.py:18-41) against stored outputs of the reference's own Reward class."""
 import numpy as np
 import pytest
 
@@ -89,17 +89,10 @@ def test_compute_reward_matches_the_reference_reward_class():
     backwards = dict(info, final_obj_pos=np.array([0.03, 0.0, 0.0]))
     env.config = make_config()
     assert env.compute_reward(info["achieved_goal"], info["desired_goal"], backwards) == 0.0
-    # the reference's own Reward.agent_reward on the same numbers (imported by file path; skipped where /root/reference is absent)
-    import importlib.util, os, sys, types
-    ref = "/root/reference/simulation/environment/reward.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present on this machine")
-    for name in ("simulation", "simulation.utils"):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    spec = importlib.util.spec_from_file_location("simulation.utils.utils", "/root/reference/simulation/utils/utils.py")
-    utils = importlib.util.module_from_spec(spec); spec.loader.exec_module(utils); sys.modules["simulation.utils.utils"] = utils
-    spec = importlib.util.spec_from_file_location("_ref_reward", ref)
-    mod = importlib.util.module_from_spec(spec); spec.loader.exec_module(mod)
-    rw = mod.Reward(robot=None, config=make_config())
-    want = rw.agent_reward(info["init_obj_pos"], info["final_obj_pos"], info["target_dir"], info["gripper_open"], info["controls"], info["object_grasped"])
-    assert abs(want - r) < 1e-9
+    # the reference's own Reward.agent_reward outputs on 64 seeded inputs (tests/golden/unit_vectors.npz, tools/gen_golden.py)
+    u = np.load(__import__("os").path.join(__import__("os").path.dirname(__file__), "golden", "unit_vectors.npz"))
+    for i in range(len(u["rw_out"])):
+        env.target_direction = u["rw_dir"][i]
+        row = dict(info, init_obj_pos=u["rw_init"][i], final_obj_pos=u["rw_final"][i], gripper_open=bool(u["rw_open"][i]),
+                   controls=u["rw_ctrl"][i], object_grasped=int(u["rw_grasp"][i]))
+        assert abs(env.compute_reward(info["achieved_goal"], info["desired_goal"], row) - u["rw_out"][i]) < 1e-9, i
