@@ -195,6 +195,44 @@ GRS_API int32_t grl_gae(const float* rewards_dev, const uint8_t* dones_dev, cons
 GRS_API int32_t grl_adam_step(float* params_dev, const float* grads_dev, float* exp_avg_dev, float* exp_avg_sq_dev, int64_t count, int32_t step,
                               float lr, float beta1, float beta2, float eps, float grad_scale, float weight_decay, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Device-resident replay buffer with HER "future" relabelling: replaces SB3's HerReplayBuffer (host RAM, one python
+ * compute_reward call per relabelled row) under SAC.train (train_agent.py:61-88).  Errors are reported through grl_last_error().
+ *
+ * One ring of capacity + 1 slots per environment, slot-major [S][N]; a slot holds obs u8[C][H][W], next_obs u8[C][H][W],
+ * action f32[A], reward f32, done u8 and the step's info row f32[GRS_INFO_STRIDE].  All environments add in lock-step.
+ *
+ * grl_replay_create: C*H*W must be a multiple of 16.  her_reward: the simulator's her_buffer (the reward carries
+ *   exp(-|dg - ag|), recomputed for relabelled goals).  seed feeds the sampling hash.  NULL on bad sizes or no CUDA device.
+ * grl_replay_begin: records obs_dev u8[N][C][H][W], the observations the next actions are taken on (after grs_reset, and once
+ *   before the first add); closes every open episode at its newest stored transition without marking it done.
+ * grl_replay_add: one vectorised step, read from the simulator's buffers after grs_step: next_obs = terminal_obs where done,
+ *   else obs; then obs (the reset observation where done) becomes the pending observation of the next slot.
+ * grl_replay_size: complete transitions per environment, min(added, capacity).
+ * grl_replay_sample: `batch` transitions, a pure function of the buffer, seed, `draw`, batch and her_ratio.  Environment and
+ *   transition uniform among the complete ones; with probability her_ratio the desired goal is replaced by the achieved goal
+ *   (info[GRS_INFO_ACHIEVED]) of a transition drawn uniformly from the same episode at or after the sampled one (the episode ends
+ *   at its done transition, or at the newest stored one while it runs), and with her_reward the reward becomes
+ *   reward - h(ag, dg_old) + h(ag, dg_new), h(a, d) = 1 / exp(|d - a|) (0 for transitions with FLAGS bit 1).  A step
+ *   with FLAGS bit 1 (non-finite state, recorded with non-finite positions) is never a goal source and is not relabelled itself.  Outputs are
+ *   device arrays obs, next_obs u8[B][C][H][W] (16-byte aligned), actions f32[B][A], reward f32[B], done u8[B], desired_goal,
+ *   achieved_goal f32[B][2]; info f32[B][GRS_INFO_STRIDE], index i64[B] (flat slot * N + env) and goal_index i64[B] (flat index
+ *   of the goal's transition, -1 when not relabelled) may be NULL.  Fails on an empty buffer, batch <= 0 or her_ratio outside
+ *   [0, 1].
+ * grl_replay_buffer: named storage views "obs", "next_obs", "actions", "reward", "done", "info" ([S][N][...], S = capacity + 1). */
+typedef struct grl_replay grl_replay;
+GRS_API grl_replay* grl_replay_create(int32_t capacity, int32_t num_envs, int32_t channels, int32_t height, int32_t width, int32_t action_dim,
+                                      int32_t her_reward, uint32_t seed, int32_t device);
+GRS_API void grl_replay_destroy(grl_replay* rb);
+GRS_API int32_t grl_replay_begin(grl_replay* rb, const uint8_t* obs_dev, void* stream);
+GRS_API int32_t grl_replay_add(grl_replay* rb, const float* actions_dev, const float* reward_dev, const uint8_t* done_dev, const float* info_dev,
+                               const uint8_t* obs_dev, const uint8_t* terminal_obs_dev, void* stream);
+GRS_API int64_t grl_replay_size(const grl_replay* rb);
+GRS_API int32_t grl_replay_sample(grl_replay* rb, int32_t batch, float her_ratio, uint64_t draw, uint8_t* obs_dev, uint8_t* next_obs_dev,
+                                  float* actions_dev, float* reward_dev, uint8_t* done_dev, float* desired_goal_dev, float* achieved_goal_dev,
+                                  float* info_dev, int64_t* index_dev, int64_t* goal_index_dev, void* stream);
+GRS_API int32_t grl_replay_buffer(grl_replay* rb, const char* name, void** ptr, uint64_t* bytes);
+
 #ifdef __cplusplus
 }
 #endif

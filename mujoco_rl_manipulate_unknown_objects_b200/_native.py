@@ -38,6 +38,8 @@ SYMBOLS += ["grp_last_error", "grp_create", "grp_destroy", "grp_num_params", "gr
             "grp_buffer", "grp_shape", "grp_launch_count", "grp_stream"]
 
 SYMBOLS += ["grl_last_error", "grl_gae", "grl_adam_step"]
+SYMBOLS += ["grl_replay_create", "grl_replay_destroy", "grl_replay_begin", "grl_replay_add", "grl_replay_size", "grl_replay_sample",
+            "grl_replay_buffer"]
 
 _lib = None
 
@@ -110,6 +112,15 @@ def load():
     L.grl_last_error.restype = C.c_char_p
     L.grl_gae.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, C.c_float, C.c_float, vp]
     L.grl_adam_step.argtypes = [vp, vp, vp, vp, i64, i32, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, vp]
+    L.grl_replay_create.restype = vp
+    L.grl_replay_create.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.c_uint32, i32]
+    L.grl_replay_destroy.argtypes = [vp]
+    L.grl_replay_begin.argtypes = [vp, vp, vp]
+    L.grl_replay_add.argtypes = [vp] + [vp] * 6 + [vp]
+    L.grl_replay_size.restype = i64
+    L.grl_replay_size.argtypes = [vp]
+    L.grl_replay_sample.argtypes = [vp, i32, C.c_float, u64] + [vp] * 10 + [vp]
+    L.grl_replay_buffer.argtypes = [vp, C.c_char_p, C.POINTER(vp), C.POINTER(u64)]
     _lib = L
     return L
 

@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgripper_sim_b200.so")
-SOURCES = ["gripper_sim.cu", "policy_kernels.cu", "train_kernels.cu", "mjcf_compiler.cpp", "dev_model.cpp"]
+SOURCES = ["gripper_sim.cu", "policy_kernels.cu", "train_kernels.cu", "replay_kernels.cu", "mjcf_compiler.cpp", "dev_model.cpp"]
 HEADERS = ["model.h", "sim_kernels.cuh", "env_kernels.cuh", "env_lockstep.cuh", "render_kernels.cuh",
            os.path.join("..", "..", "include", "b200_gripper_sim.h")]
 # -prec-div=false / -prec-sqrt=false / -ftz=true: divisions and square roots are the hardware's 2-ulp approximations and

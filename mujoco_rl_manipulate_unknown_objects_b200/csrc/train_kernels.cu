@@ -1,6 +1,7 @@
-// Rollout post-processing and optimiser step of the on-device PPO loop (SURVEY.md §8f N1, BASELINE.json configs[3]).
-// The reference trains with SB3's SAC whose replay buffer and Adam step live on the host side of a single environment
-// (train_agent.py:82-88); these two kernels replace that round trip for the device-resident rollout storage:
+// Rollout post-processing and optimiser step of the on-device learners (SURVEY.md §8f N1, BASELINE.json configs[3]).
+// The reference trains with SB3's SAC, whose Adam step runs on the host side of a single environment (train_agent.py:82-88);
+// its replay buffer has a device-resident counterpart in replay_kernels.cu.  The two kernels here serve the PPO rollout
+// storage (k_gae) and every flat-bucket optimiser, PPO's and SAC's (k_adam):
 //
 //   k_gae   : generalised advantage estimation + returns over the [T][N] rollout storage, one thread per environment walking
 //             its T transitions backwards (coalesced across N), plus the sum / sum of squares of the advantages (double
@@ -72,6 +73,7 @@ __global__ void k_adam(float* __restrict__ p, const float* __restrict__ g, float
 }  // namespace
 
 extern "C" const char* grl_last_error(void) { return t_err.c_str(); }
+int grl_set_error(const std::string& m) { return tfail(m); }  // shared with replay_kernels.cu
 
 extern "C" int32_t grl_gae(const float* rewards_dev, const uint8_t* dones_dev, const float* values_dev, float* adv_dev, float* ret_dev, double* moments_dev,
                            int32_t T, int32_t N, float gamma, float lam, void* stream) {

@@ -122,11 +122,15 @@ class RolloutWorker:
         self.noise = torch.zeros_like(self.actions)
         self.sim.reset()
 
-    def collect(self, n_steps, deterministic=False, storage=None, random_actions=False):
+    def collect(self, n_steps, deterministic=False, storage=None, random_actions=False, replay=None):
         """n_steps vectorised transitions.  storage (optional dict of preallocated tensors [T, N, ...]: obs, actions, rewards,
-        dones, mu, log_std, noise) receives the trajectory.  Returns RolloutStats (local; call .all_reduce())."""
+        dones, mu, log_std, noise) receives the trajectory.  replay (optional DeviceReplayBuffer over this worker's
+        environments) receives every transition right after the step; a buffer not yet begun records the current observations
+        first (replay.begin()).  Returns RolloutStats (local; call .all_reduce())."""
         t = self.sim._torch
         stats = RolloutStats(self.device)
+        if replay is not None and not replay.begun:
+            replay.begin(self.sim.obs)
         for k in range(n_steps):
             if storage is not None:
                 storage["obs"][k].copy_(self.sim.obs)
@@ -137,6 +141,9 @@ class RolloutWorker:
                     self.noise.normal_(generator=self.gen)
                 self.policy.forward(self.sim.obs, deterministic=deterministic, noise=None if deterministic else self.noise, out=self.actions)
             self.sim.step(self.actions)
+            if replay is not None:
+                s = self.sim
+                replay.add(self.actions, s.reward, s.done, s.info, s.obs, s.terminal_obs)
             stats.update(self.sim.info, self.sim.reward, self.sim.done)
             if storage is not None:
                 storage["actions"][k].copy_(self.actions)
