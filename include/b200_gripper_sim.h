@@ -170,7 +170,7 @@ GRS_API int32_t grp_get_params(const grp_policy* p, float* params_host, int64_t 
  * stream: cudaStream_t as void* (NULL = the handle's own stream). */
 GRS_API int32_t grp_forward(grp_policy* p, const uint8_t* obs_dev, float* actions_dev, const float* noise_dev, int32_t n, void* stream);
 /* named device buffers: "mu", "log_std" f32[max_envs][A]; "features" bf16[max_envs][576] (512 CNN + 2 direct + padding);
- * "act1" "act2" "act3" "h1" "h2" bf16 intermediate activations (NHWC) */
+ * "act1" "act2" "act3" bf16 intermediate activations of the last forward (NHWC) */
 GRS_API int32_t grp_buffer(grp_policy* p, const char* name, void** ptr, uint64_t* bytes);
 /* {C, H, W, o1h, o1w, o2h, o2w, o3h, o3w, A} */
 GRS_API int32_t grp_shape(const grp_policy* p, int32_t* out10);

@@ -5,15 +5,18 @@
 //   obs u8 [N,C,H,W] --/255--> conv 8x8 s4 (C-1 -> 32) ReLU -> conv 4x4 s2 (32 -> 64) ReLU -> conv 3x3 s1 (64 -> 64) ReLU
 //   -> flatten -> linear (-> 512) ReLU -> concat obs[:, C-1, 0, 0:2]/255 (514) -> 256 ReLU -> 256 ReLU -> mu | log_std -> tanh
 //
-// Kernels of one forward (default path, the reference's 64 x 64 x 4 observation):
-//   k_conv1_ws          conv1 WITHOUT im2col: the tensor core reads the fp16 image through a no-swizzle shared-memory descriptor,
-//                       16 MMAs (M 128, N 96 = W | Wa | Wb) per image; warp-specialised (TMA producer, converters, issuer, epilogue)
-//   k_conv_direct<2|3>  conv2 / conv3 WITHOUT im2col: the previous layer's padded, pre-swizzled activations arrive by one bulk copy per
-//                       image pair and every k-block is a start address inside that copy (k_conv23_fused: both in one kernel)
-//   k_layer<DENSE>      the linear layer (+ the two direct features): the generic implicit-GEMM layer described next
-//   k_mlp_fused         latent_pi.0, latent_pi.2 and the mu | log_std head; hidden activations TMEM -> registers -> shared memory
-// k_layer<MODE, BN, EPI> is round 1's generic layer (still used for the linear layer, for other observation shapes and behind the
-// GRP_* switches): an implicit GEMM  D[128 x BN] += A[128 x 64] * W[BN x 64]^T per k-block, with
+// One forward is five kernels.  Which conv kernels run depends only on the observation shape, fixed at grp_create:
+//   64 x 64 observations with 4 image planes (the reference's full observation), the descriptor-addressed chain:
+//     k_conv1_ws          conv1 WITHOUT im2col: the tensor core reads the fp16 image through a no-swizzle shared-memory descriptor,
+//                         16 MMAs (M 128, N 96 = W | Wa | Wb) per image; warp-specialised (TMA producer, converters, issuer, epilogue)
+//     k_conv_direct<2|3>  conv2 / conv3 WITHOUT im2col: the previous layer's padded, pre-swizzled activations arrive by one bulk copy
+//                         per image pair and every k-block is a start address inside that copy
+//   any other shape (e.g. full_observation=False: 3 image planes), the generic chain:
+//     k_layer<CONV1 | CONV2 | CONV3>  the implicit-GEMM layer described below, gathering its A operand from dense NHWC activations
+//   every shape:
+//     k_layer<DENSE>      the linear layer (+ the two direct features)
+//     k_mlp_fused         latent_pi.0, latent_pi.2 and the mu | log_std head; hidden activations TMEM -> registers -> shared memory
+// k_layer<MODE, BN, EPI> is round 1's generic layer: an implicit GEMM  D[128 x BN] += A[128 x 64] * W[BN x 64]^T per k-block, with
 //   * A gathered by the CTA's threads straight from the previous layer's activations (im2col on the fly, NHWC bf16; the
 //     first layer reads the uint8 observation planes and converts) into the canonical K-major SWIZZLE_128B shared-memory
 //     layout that tcgen05.mma reads through a shared-memory descriptor,
@@ -21,8 +24,8 @@
 //   * one elected thread issuing tcgen05.mma.cta_group::1.kind::f16 (M=128, N=BN, K=16) into a TMEM accumulator and
 //     tcgen05.commit-ing each stage to an mbarrier, so the gather of k-block i+1.. overlaps the MMAs of k-block i
 //     (3-stage ring),
-//   * the epilogue reading the accumulator back with tcgen05.ld (32 lanes x 32 columns per warp), applying
-//     scale/bias/ReLU (or the squashed-Gaussian head) and writing bf16 NHWC rows for the next layer.
+//   * the epilogue reading the accumulator back with tcgen05.ld (32 lanes x 16 columns per warp at a time), applying
+//     scale/bias/ReLU and writing bf16 NHWC rows for the next layer.
 // No cuBLAS / cuDNN / CUTLASS calls; descriptor bit layouts follow the PTX ISA (matrix-descriptor and instruction-descriptor
 // tables for tcgen05.mma).
 #include <cuda_bf16.h>
@@ -31,8 +34,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <memory>
 #include <stdexcept>
@@ -44,11 +45,11 @@
 namespace grp {
 
 enum Mode { DENSE = 0, CONV1 = 1, CONV2 = 2, CONV3 = 3 };
-enum Epi { EPI_RELU = 0, EPI_FEATURES = 1, EPI_HEAD = 2 };
+enum Epi { EPI_RELU = 0, EPI_FEATURES = 1 };
 
 constexpr int BM = 128;      // rows of A per CTA = TMEM lanes = UMMA M
 constexpr int BK = 64;       // bf16 elements per k-block = one 128-byte swizzle row
-__host__ __device__ constexpr int stages_of(int mode) { return mode >= 0 ? 3 : 3; }
+constexpr int LAYER_STAGES = 3;  // k_layer's ring of staged k-blocks
 constexpr int THREADS = 128;
 constexpr int FEAT_LD = 576;  // 512 CNN features + 2 direct features, zero padded to a multiple of BK
 constexpr int HEAD_N = 16;    // mu rows 0..A-1, log_std rows 8..8+A-1
@@ -63,10 +64,6 @@ struct LayerArgs {
   int C, H, W_;              // observation planes (CONV1, EPI_FEATURES)
   int ih, iw, oh, ow;        // input / output feature-map size of a convolution
   const unsigned char* obs;  // EPI_FEATURES: the two direct features come from obs[:, C-1, 0, 0:2]
-  // EPI_HEAD
-  float *mu, *log_std, *action;
-  const float* noise;        // [M][adim] standard normal, or NULL for the deterministic action
-  int adim;
 };
 
 // ------------------------------------------------------------------------------------------------ PTX wrappers
@@ -137,6 +134,20 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float* v) {
 #pragma unroll
   for (int i = 0; i < 16; i++) v[i] = __uint_as_float(r[i]);
 }
+// the same for 32 consecutive columns
+__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
+  uint32_t r[32];
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]),
+        "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]),
+        "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+      : "r"(taddr)
+      : "memory");
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 32; i++) v[i] = __uint_as_float(r[i]);
+}
 
 // shared-memory matrix descriptor: K-major operand, SWIZZLE_128B (rows of 128 bytes, 8-row groups 1024 bytes apart)
 __device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t saddr) {
@@ -204,12 +215,12 @@ __device__ __forceinline__ uint4 u8x8_to_f16x8(uint2 raw) {
 
 template <int BN>
 __host__ __device__ constexpr int tmem_cols() { return BN <= 32 ? 32 : BN <= 64 ? 64 : BN <= 128 ? 128 : 256; }
-template <int MODE, int BN>
-__host__ __device__ constexpr size_t layer_smem_bytes() { return (size_t)stages_of(MODE) * (BM * 128 + BN * 128) + 1024; }
+template <int BN>
+__host__ __device__ constexpr size_t layer_smem_bytes() { return (size_t)LAYER_STAGES * (BM * 128 + BN * 128) + 1024; }
 
 template <int MODE, int BN, int EPI>
 __global__ void __launch_bounds__(THREADS) k_layer(const LayerArgs a) {
-  constexpr int STAGES = stages_of(MODE);
+  constexpr int STAGES = LAYER_STAGES;
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t bar_stage[STAGES];
   __shared__ uint64_t bar_done;
@@ -281,29 +292,18 @@ __global__ void __launch_bounds__(THREADS) k_layer(const LayerArgs a) {
     constexpr int PRE = 4;
     const unsigned char* obs = reinterpret_cast<const unsigned char*>(a.A);
     const int plane = a_kb_offset<CONV1>(a, 1);
-    // the reference's observation (64 x 64 planes, 4 image channels) on a full tile: every load is base + immediate
-    const bool fast = a.iw == 64 && a.ih == 64 && nkb == PRE && m0 + BM <= a.M;
 #pragma unroll 1
     for (int kb0 = 0; kb0 < nkb; kb0 += PRE) {
       uint2 raw[PRE][BM * 8 / THREADS];
-      if (fast) {
-        const unsigned char* p = obs + rbase[0];
 #pragma unroll
-        for (int i = 0; i < BM * 8 / THREADS; i++)
+      for (int i = 0; i < BM * 8 / THREADS; i++) {
+        const int base = rbase[i];
 #pragma unroll
-          for (int j = 0; j < PRE; j++)
-            raw[j][i] = make_uint2(__ldg(reinterpret_cast<const uint32_t*>(p + i * 64 + j * 4096)), __ldg(reinterpret_cast<const uint32_t*>(p + i * 64 + j * 4096 + 4)));
-      } else {
-#pragma unroll
-        for (int i = 0; i < BM * 8 / THREADS; i++) {
-          const int base = rbase[i];
-#pragma unroll
-          for (int j = 0; j < PRE; j++) {
-            raw[j][i] = make_uint2(0, 0);
-            if (base >= 0 && kb0 + j < nkb) {
-              const unsigned char* src = obs + base + (kb0 + j) * plane;
-              raw[j][i] = make_uint2(__ldg(reinterpret_cast<const uint32_t*>(src)), __ldg(reinterpret_cast<const uint32_t*>(src + 4)));
-            }
+        for (int j = 0; j < PRE; j++) {
+          raw[j][i] = make_uint2(0, 0);
+          if (base >= 0 && kb0 + j < nkb) {
+            const unsigned char* src = obs + base + (kb0 + j) * plane;
+            raw[j][i] = make_uint2(__ldg(reinterpret_cast<const uint32_t*>(src)), __ldg(reinterpret_cast<const uint32_t*>(src + 4)));
           }
         }
       }
@@ -371,171 +371,39 @@ __global__ void __launch_bounds__(THREADS) k_layer(const LayerArgs a) {
   // ---- epilogue: thread t of warp w owns accumulator row 32*w + t
   const int row = m0 + warp * 32 + lane;
   const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);
-  if (EPI == EPI_HEAD) {
-    float v[16];
-    tmem_ld16(trow, v);
-    if (row < a.M) {
-      for (int k = 0; k < a.adim; k++) {
-        const float mu = v[k] + sbias[k];
-        float ls = v[8 + k] + sbias[8 + k];
-        ls = fminf(fmaxf(ls, -20.0f), 2.0f);  // stable-baselines3 sac/policies.py LOG_STD_MIN / LOG_STD_MAX
-        float pre = mu;
-        if (a.noise) pre += __expf(ls) * a.noise[(size_t)row * a.adim + k];
-        a.mu[(size_t)row * a.adim + k] = mu;
-        a.log_std[(size_t)row * a.adim + k] = ls;
-        a.action[(size_t)row * a.adim + k] = tanhf(pre);
-      }
-    }
-  } else {
 #pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 16) {
-      float v[16];
-      tmem_ld16(trow + c0, v);
-      if (row < a.M) {
-        uint32_t o[8];
-        float bv[16];  // four 16-byte broadcast loads instead of sixteen scalar ones
+  for (int c0 = 0; c0 < BN; c0 += 16) {
+    float v[16];
+    tmem_ld16(trow + c0, v);
+    if (row < a.M) {
+      uint32_t o[8];
+      float bv[16];  // four 16-byte broadcast loads instead of sixteen scalar ones
 #pragma unroll
-        for (int k = 0; k < 4; k++) *reinterpret_cast<float4*>(bv + 4 * k) = *reinterpret_cast<const float4*>(sbias + c0 + 4 * k);
+      for (int k = 0; k < 4; k++) *reinterpret_cast<float4*>(bv + 4 * k) = *reinterpret_cast<const float4*>(sbias + c0 + 4 * k);
 #pragma unroll
-        for (int k = 0; k < 8; k++) {
-          const float x = fmaxf(fmaf(v[2 * k], a.scale, bv[2 * k]), 0.0f);
-          const float y = fmaxf(fmaf(v[2 * k + 1], a.scale, bv[2 * k + 1]), 0.0f);
-          o[k] = pack_bf16(x, y);
-        }
-        uint4* dst = reinterpret_cast<uint4*>(a.out + (size_t)row * a.ldo + n0 + c0);
-        dst[0] = make_uint4(o[0], o[1], o[2], o[3]);
-        dst[1] = make_uint4(o[4], o[5], o[6], o[7]);
+      for (int k = 0; k < 8; k++) {
+        const float x = fmaxf(fmaf(v[2 * k], a.scale, bv[2 * k]), 0.0f);
+        const float y = fmaxf(fmaf(v[2 * k + 1], a.scale, bv[2 * k + 1]), 0.0f);
+        o[k] = pack_bf16(x, y);
       }
+      uint4* dst = reinterpret_cast<uint4*>(a.out + (size_t)row * a.ldo + n0 + c0);
+      dst[0] = make_uint4(o[0], o[1], o[2], o[3]);
+      dst[1] = make_uint4(o[4], o[5], o[6], o[7]);
     }
-    if (EPI == EPI_FEATURES && blockIdx.y == 0 && row < a.M) {
-      // feature_extractor.py:42,48 — the two direct features ride behind the 512 CNN features (then zero padding)
-      const unsigned char* p = a.obs + ((size_t)row * a.C + (a.C - 1)) * a.H * a.W_;
-      uint4* dst = reinterpret_cast<uint4*>(a.out + (size_t)row * a.ldo + 512);
-      dst[0] = make_uint4(pack_bf16((float)p[0] * (1.0f / 255.0f), (float)p[1] * (1.0f / 255.0f)), 0, 0, 0);
+  }
+  if (EPI == EPI_FEATURES && blockIdx.y == 0 && row < a.M) {
+    // feature_extractor.py:42,48 — the two direct features ride behind the 512 CNN features (then zero padding)
+    const unsigned char* p = a.obs + ((size_t)row * a.C + (a.C - 1)) * a.H * a.W_;
+    uint4* dst = reinterpret_cast<uint4*>(a.out + (size_t)row * a.ldo + 512);
+    dst[0] = make_uint4(pack_bf16((float)p[0] * (1.0f / 255.0f), (float)p[1] * (1.0f / 255.0f)), 0, 0, 0);
 #pragma unroll
-      for (int k = 1; k < (FEAT_LD - 512) / 8; k++) dst[k] = make_uint4(0, 0, 0, 0);
-    }
+    for (int k = 1; k < (FEAT_LD - 512) / 8; k++) dst[k] = make_uint4(0, 0, 0, 0);
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem, tmem_cols<BN>());
 }
 
-
-// ------------------------------------------------------------------------------------------------ conv1, one image per CTA
-// The reference's observation (64 x 64, 4 image planes = one contiguous 16 KB block of the [n][C][64][64] uint8 tensor) is
-// brought into shared memory by ONE bulk asynchronous copy (cp.async.bulk, the TMA engine's 1-D path) that completes on an
-// mbarrier.  The 225 output pixels of the image are two 128-row MMA tiles (TMEM columns 0-31 and 32-63); thread t of the 256
-// builds the K row of output pixel t from shared memory, one K half (two input channels) at a time (16 chunks of 8 pixels:
-// shared loads at compile-time offsets, byte permutes, HSUB2; no global address arithmetic, no global latency); the MMAs of a
-// half run while the next half is being converted.
-constexpr int C1_THREADS = 256;                // thread t: output pixel t (tile 0: pixels 0..127, tile 1: 128..224 + padding)
-constexpr int C1_IMG = 4 * 64 * 64;            // staged uint8 planes
-constexpr int C1_A = 2 * 2 * BM * 128;         // two tiles x two k-blocks of A (one K half at a time), K-major SWIZZLE_128B
-constexpr int C1_W = 4 * 32 * 128;             // four k-blocks of W (32 output channels)
-constexpr size_t C1_SMEM = C1_IMG + C1_A + C1_W + 1024;
-
-__global__ void __launch_bounds__(C1_THREADS) k_conv1_image(const LayerArgs a) {
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ uint64_t bar_img, bar_mma;
-  __shared__ uint32_t tmem_base_s;
-  __shared__ float sbias[32];
-  const int tid = threadIdx.x, warp = tid >> 5;
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* sA = smem;                  // [tile 2][k-block of the current half 2][128 rows x 128 B]
-  uint8_t* sB = smem + C1_A;           // 4 x [32 rows x 128 B]
-  uint8_t* img = smem + C1_A + C1_W;   // [4][64][64] uint8
-  if (tid < 32) sbias[tid] = __ldg(a.bias + tid);
-  if (tid == 0) {
-    mbar_init(&bar_img, 1);
-    mbar_init(&bar_mma, 1);
-    fence_barrier_init();
-  }
-  __syncwarp();
-  if (warp == 0) tmem_alloc(&tmem_base_s, 64);  // columns 0..31: tile 0, 32..63: tile 1
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  const uint32_t tmem = tmem_base_s;
-  const int n = blockIdx.x;
-  // ---- stage: the image (bulk copy) and the whole weight matrix (16-byte asynchronous copies, swizzled)
-  if (tid == 0) {
-    const unsigned char* src = reinterpret_cast<const unsigned char*>(a.A) + (size_t)n * a.C * 4096;
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&bar_img)), "r"(C1_IMG) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(img)), "l"(src), "r"(C1_IMG), "r"(smem_u32(&bar_img)) : "memory");
-  }
-#pragma unroll
-  for (int i = 0; i < 4 * 32 * 8 / C1_THREADS; i++) {
-    const int c = i * C1_THREADS + tid, kb = c >> 8, row = (c >> 3) & 31, ch = c & 7;
-    cp_async16(smem_u32(sB + kb * 32 * 128 + row * 128 + ((ch ^ (row & 7)) << 4)), a.W + (size_t)row * a.K + kb * BK + ch * 8, true);
-  }
-  cp_async_commit();
-  mbar_wait(&bar_img, 0);
-  cp_async_wait<0>();
-  constexpr uint32_t idesc = instr_desc_f16(BM, 32, false);
-  const int per = 15 * 15;
-  const int tile = tid >> 7, row = tid & 127, p = tid;  // output pixel of this thread
-  const bool valid = p < per;
-  const int oy = valid ? p / 15 : 0, ox = valid ? p - oy * 15 : 0;
-  const uint8_t* src = img + (4 * oy) * 64 + 4 * ox;
-  uint8_t* dst = sA + tile * 2 * BM * 128 + row * 128;
-  const int sw = row & 7;
-#pragma unroll 1
-  for (int half = 0; half < 2; half++) {
-    if (half) {  // the MMAs of the first K half read the A buffers that are about to be overwritten
-      mbar_wait(&bar_mma, 0);
-      tc_fence_after();
-    }
-#pragma unroll
-    for (int kk = 0; kk < 2; kk++) {
-      const int kb = half * 2 + kk;
-#pragma unroll
-      for (int ky = 0; ky < 8; ky++) {
-        uint2 raw = make_uint2(0, 0);
-        if (valid) raw = make_uint2(*reinterpret_cast<const uint32_t*>(src + kb * 4096 + ky * 64), *reinterpret_cast<const uint32_t*>(src + kb * 4096 + ky * 64 + 4));
-        *reinterpret_cast<uint4*>(dst + kk * BM * 128 + ((ky ^ sw) << 4)) = u8x8_to_f16x8(raw);
-      }
-    }
-    fence_async_smem();
-    __syncthreads();
-    if (tid == 0) {
-      tc_fence_after();
-#pragma unroll
-      for (int t = 0; t < 2; t++)
-#pragma unroll
-        for (int kk = 0; kk < 2; kk++) {
-          const uint32_t aaddr = smem_u32(sA + (t * 2 + kk) * BM * 128), baddr = smem_u32(sB + (half * 2 + kk) * 32 * 128);
-#pragma unroll
-          for (int k = 0; k < BK / 16; k++) umma_bf16(tmem + t * 32, smem_desc_sw128(aaddr + k * 32), smem_desc_sw128(baddr + k * 32), idesc, (half | kk | k) != 0);
-        }
-      umma_commit(&bar_mma);
-    }
-  }
-  mbar_wait(&bar_mma, 1);
-  tc_fence_after();
-  // ---- epilogue: thread `row` of warp w (w % 4 selects the 32-lane TMEM slice) owns accumulator row `row` of its tile
-  const uint32_t trow = tmem + tile * 32 + ((uint32_t)((warp & 3) * 32) << 16);
-#pragma unroll
-  for (int c0 = 0; c0 < 32; c0 += 16) {
-    float v[16];
-    tmem_ld16(trow + c0, v);
-    if (valid) {
-      uint32_t o[8];
-#pragma unroll
-      for (int k = 0; k < 8; k++)
-        o[k] = pack_bf16(fmaxf(v[2 * k] * a.scale + sbias[c0 + 2 * k], 0.0f), fmaxf(v[2 * k + 1] * a.scale + sbias[c0 + 2 * k + 1], 0.0f));
-      uint4* out = reinterpret_cast<uint4*>(a.out + ((size_t)n * per + p) * 32 + c0);
-      out[0] = make_uint4(o[0], o[1], o[2], o[3]);
-      out[1] = make_uint4(o[4], o[5], o[6], o[7]);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem, 64);
-}
 
 // ------------------------------------------------------------------------------------------------ conv1 without im2col
 // The 8x8 stride-4 convolution read straight off the image by the tensor core's shared-memory descriptor — no im2col copy.
@@ -554,13 +422,8 @@ __global__ void __launch_bounds__(C1_THREADS) k_conv1_image(const LayerArgs a) {
 // m + 1 (a register shuffle from the next lane: rows are lanes) to column block 1 of row m.  16 MMAs per image; the image is read
 // from shared memory once per 96 output columns (one N = 32 MMA per product was bound by the tensor core's operand reads,
 // 240 KB per image); ONE fp16 copy of the image, one 16-byte store per 8-pixel chunk instead of 7 200 im2col chunks per image.
-// Persistent: one CTA per SM loops over images; two stages of image copies and of TMEM accumulators, so the conversion of
-// image i + 1 and the epilogue of image i - 1 overlap the MMAs of image i; raw bytes are prefetched two images ahead.
-constexpr int CD_THREADS = 512;                   // worker threads (convert + epilogue)
-constexpr int CD_CHUNKS = 2048 / CD_THREADS;      // eight-pixel chunks per worker and image
 constexpr int CD_STAGE = 4 * 64 * 64 * 2 + 1024;  // the fp16 copy of the four planes + slack (group 15 of the last plane reads 512 B past it)
 constexpr int CD_W = 4 * 96 * 128;                // 4 k-blocks (= input channels) x [96 rows = W | Wa | Wb] x 128 B, SWIZZLE_128B
-constexpr size_t CD_SMEM = CD_W + 2 * CD_STAGE + 1024;
 
 // shared-memory matrix descriptor: K-major operand, no swizzle (8 x 16-byte core matrices; LBO = K step, SBO = 8-row group step)
 __device__ __forceinline__ uint64_t smem_desc_nosw(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
@@ -571,157 +434,10 @@ __device__ __forceinline__ uint64_t smem_desc_nosw(uint32_t saddr, uint32_t lbo_
   d |= (uint64_t)1 << 46;
   return d;
 }
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float* v) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(taddr) : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 8; i++) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]),
-        "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]),
-        "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; i++) v[i] = __uint_as_float(r[i]);
-}
 
-template <bool DEDICATED>  // true: an extra warp issues the MMAs; false: thread 0 does
-__global__ void __launch_bounds__(CD_THREADS + (DEDICATED ? 32 : 0), 1) k_conv1_direct(const LayerArgs a, int nimg) {
-  constexpr int NT = CD_THREADS + (DEDICATED ? 32 : 0), ISSUER = DEDICATED ? CD_THREADS : 0;
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ uint64_t bar_mma[2];
-  __shared__ uint32_t tmem_base_s;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* sB = smem;            // [4 k-blocks][96 rows: W | Wa | Wb][128 B]
-  uint8_t* st0 = smem + CD_W;    // stage s: the fp16 image at st0 + s * CD_STAGE
-  if (tid == 0) {
-    mbar_init(&bar_mma[0], 1);
-    mbar_init(&bar_mma[1], 1);
-    fence_barrier_init();
-  }
-  __syncwarp();
-  if (warp == 0) tmem_alloc(&tmem_base_s, 256);  // stage s: columns 128 s .. 128 s + 95
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  const uint32_t tmem = tmem_base_s;
-  for (int i = tid; i < 4 * 96 * 8; i += NT) {  // rows 0-31 W, 32-63 Wa, 64-95 Wb: three consecutive [32][K] matrices behind a.W
-    const int kb = i / 768, c = i - kb * 768, row = c >> 3, ch = c & 7;
-    cp_async16(smem_u32(sB + kb * 96 * 128 + row * 128 + ((ch ^ (row & 7)) << 4)), a.W + (size_t)row * a.K + kb * BK + ch * 8, true);
-  }
-  cp_async_commit();
-  // the slack behind the copies is read by the junk rows of the MMAs (results never used): keep it finite
-  for (int i = tid; i < 2 * 1024 / 16; i += NT) *reinterpret_cast<uint4*>(st0 + (i >> 6) * CD_STAGE + (CD_STAGE - 1024) + (i & 63) * 16) = make_uint4(0, 0, 0, 0);
-  const unsigned char* obs = reinterpret_cast<const unsigned char*>(a.A);
-  const size_t img_bytes = (size_t)a.C * 4096;
-  // raw bytes of the next two images of this CTA, in registers
-  uint2 rawA[CD_CHUNKS], rawB[CD_CHUNKS];
-  const int stride = gridDim.x;
-  const bool worker = tid < CD_THREADS;  // the extra warp (if any) only issues the MMAs
-  auto load_raw = [&](uint2 (&raw)[CD_CHUNKS], int n) {
-    if (n < nimg && worker) {
-      const uint2* src = reinterpret_cast<const uint2*>(obs + (size_t)n * img_bytes);
-#pragma unroll
-      for (int j = 0; j < CD_CHUNKS; j++) raw[j] = __ldg(src + tid + CD_THREADS * j);
-    }
-  };
-  load_raw(rawA, blockIdx.x);
-  load_raw(rawB, blockIdx.x + stride);
-  cp_async_wait<0>();
-  constexpr uint32_t idesc = instr_desc_f16(BM, 96, false);
-  // epilogue role of this thread: accumulator row m = 32 (warp % 4) + lane = 8 oy + r, output channels 8 (warp / 4) .. + 7 of the
-  // two output pixels ox = 2r and 2r + 1
-  const int eq = (warp >> 2) & 3, em = 32 * (warp & 3) + lane, eoy = em >> 3, er = em & 7;
-  const bool evalid = eoy < 15;
-  float eb[8];  // this thread's biases, in registers (a shared-memory load per accumulator element made the epilogue MIO-bound)
-#pragma unroll
-  for (int k = 0; k < 8; k++) eb[k] = __ldg(a.bias + eq * 8 + k);
-  const float escale = a.scale;
-  // one image: convert into stage s, start its MMAs, then finish the previous image (other stage) while they run
-  auto step = [&](uint2 (&raw)[CD_CHUNKS], const int s, const int n, const int it) {
-    const bool have = n < nimg;
-    if (have && worker) {
-      // stage s is free: the MMAs of image it - 2 were waited for by the epilogue of iteration it - 1
-      uint8_t* E = st0 + s * CD_STAGE;
-#pragma unroll
-      for (int j = 0; j < CD_CHUNKS; j++) *reinterpret_cast<uint4*>(E + (tid + CD_THREADS * j) * 16) = u8x8_to_f16x8(raw[j]);  // the copy is dense: chunk q at byte 16 q
-      load_raw(raw, n + 2 * stride);  // in flight for two iterations
-      fence_async_smem();
-    }
-    __syncthreads();
-    if (have && tid == ISSUER) {
-      // 16 MMAs (M = 128, N = 96, K = 16); every descriptor is a constant 16-byte-unit offset away from the stage's first one
-      tc_fence_after();
-      const uint64_t a0 = smem_desc_nosw(smem_u32(st0 + s * CD_STAGE), 128, 512), b0 = smem_desc_sw128(smem_u32(sB));
-      const uint32_t alo = (uint32_t)a0, ahi = (uint32_t)(a0 >> 32), blo = (uint32_t)b0, bhi = (uint32_t)(b0 >> 32), td = tmem + s * 128;
-#pragma unroll
-      for (int c = 0; c < 4; c++)
-#pragma unroll
-        for (int kyp = 0; kyp < 4; kyp++) {
-          if ((c | kyp) == 0) umma_bf16_lo<0>(td, alo + ((c * 8192 + kyp * 256) >> 4), ahi, blo + ((c * 96 * 128 + kyp * 32) >> 4), bhi, idesc);
-          else umma_bf16_lo<1>(td, alo + ((c * 8192 + kyp * 256) >> 4), ahi, blo + ((c * 96 * 128 + kyp * 32) >> 4), bhi, idesc);
-        }
-      umma_commit(&bar_mma[s]);
-    }
-    if (it > 0 && worker) {  // epilogue of the previous image (other stage) while this image's MMAs run
-      const int ps = s ^ 1, pn = n - stride;
-      mbar_wait(&bar_mma[ps], ((it - 1) >> 1) & 1);
-      tc_fence_after();
-      float ve[8], va[8], vb[8];
-      {
-        const uint32_t tb = tmem + ps * 128 + eq * 8 + ((uint32_t)(32 * (warp & 3)) << 16);
-        tmem_ld8(tb, ve);
-        tmem_ld8(tb + 32, va);
-        tmem_ld8(tb + 64, vb);
-      }
-#pragma unroll
-      for (int k = 0; k < 8; k++) va[k] += __shfl_down_sync(0xffffffffu, vb[k], 1);  // odd(r) = chunk r x Wa + chunk r + 1 x Wb (row m + 1; r = 7 has no odd pixel)
-      if (evalid) {
-        uint32_t oe[4], oo[4];
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-          oe[k] = pack_bf16(fmaxf(fmaf(ve[2 * k], escale, eb[2 * k]), 0.0f), fmaxf(fmaf(ve[2 * k + 1], escale, eb[2 * k + 1]), 0.0f));
-          oo[k] = pack_bf16(fmaxf(fmaf(va[2 * k], escale, eb[2 * k]), 0.0f), fmaxf(fmaf(va[2 * k + 1], escale, eb[2 * k + 1]), 0.0f));
-        }
-        if (a.ldo == 32) {  // dense [225][32] rows (the gather-based conv2)
-          __nv_bfloat16* row = a.out + ((size_t)pn * 225 + eoy * 15 + 2 * er) * 32 + eq * 8;
-          *reinterpret_cast<uint4*>(row) = make_uint4(oe[0], oe[1], oe[2], oe[3]);
-          if (er < 7) *reinterpret_cast<uint4*>(row + 32) = make_uint4(oo[0], oo[1], oo[2], oo[3]);
-        } else {
-          // the layout conv2's descriptor reads: [15][16 px][32 ch], 128-byte lines of two pixels (2r, 2r + 1), chunk j of line l at j ^ (l & 7)
-          const int l = eoy * 8 + er;
-          uint8_t* line = reinterpret_cast<uint8_t*>(a.out) + (size_t)pn * 16384 + l * 128;
-          *reinterpret_cast<uint4*>(line + ((eq ^ (l & 7)) << 4)) = make_uint4(oe[0], oe[1], oe[2], oe[3]);
-          if (er < 7) *reinterpret_cast<uint4*>(line + (((4 + eq) ^ (l & 7)) << 4)) = make_uint4(oo[0], oo[1], oo[2], oo[3]);
-        }
-      }
-      tc_fence_before();
-    }
-  };
-  // the extra pass behind the last image runs its epilogue; iterations come in pairs so that stage and register set are static
-#pragma unroll 1
-  for (int n = blockIdx.x, it = 0; n < nimg + stride; n += 2 * stride, it += 2) {
-    step(rawA, 0, n, it);
-    if (n < nimg) step(rawB, 1, n + stride, it + 1);
-  }
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem, 256);
-}
-
-// The same convolution, warp-specialised: converting the next image, multiplying the current one and writing out the previous
-// one are three different sets of warps that meet only at mbarriers, instead of one set of warps doing the three jobs one after
-// the other between block barriers (k_conv1_direct: 46 % of its stall samples sat at __syncthreads, tensor pipe active 34 %).
+// Warp-specialised: converting the next image, multiplying the current one and writing out the previous one are three different
+// sets of warps that meet only at mbarriers.  With one set of warps doing the three jobs one after the other between block
+// barriers, 46 % of the stall samples sat at __syncthreads and the tensor pipe was active 34 % of the time.
 //   warp  17     producer: the image's four uint8 planes (16 KB, contiguous) by cp.async.bulk into a 4-deep raw ring — 64 KB per SM in
 //                flight from HBM: with register prefetch two images ahead the kernel was bound by memory latency (1.7 TB/s)
 //   warps 0-7    converters: raw ring -> fp16 copy of image k in stage k % 3, fence.proxy.async, one arrive per warp on full[stage]
@@ -1022,178 +738,6 @@ __global__ void __launch_bounds__(DC_THREADS, 1) k_conv_direct(const LayerArgs a
   if (warp == 0) tmem_dealloc(tmem, 128);
 }
 
-// ------------------------------------------------------------------------------------------------ conv2 + conv3 in one kernel
-// conv2's output never leaves the SM: its epilogue writes act2 (two images, 16 KB) into shared memory in exactly the padded,
-// swizzled layout conv3's descriptors read, and the same MMA-issuer thread then runs conv3 on it.  Both weight matrices are resident
-// (64 + 72 KB).  That removes act2's trip through L2 / HBM (8 KB per observation each way) and one launch with its fixed cost.
-//   warp 8   producer: act1 image pairs by cp.async.bulk into a 2-deep ring
-//   warp 9   issuer, per pair k: conv2(k) [32 MMAs -> accumulator k % 2], then conv3(k - 1) [36 MMAs on the act2 buffer -> accumulator
-//            2 + (k - 1) % 2]; tcgen05.commit hands back the act1 stage / the act2 buffer and publishes the accumulators
-//   warps 0-7 epilogue, per pair k: conv2 accumulator -> bias, ReLU, bf16 -> act2 buffer (fence.proxy.async, arrive), then the conv3
-//            accumulator of pair k - 1 -> act3 in HBM (dense rows for the linear layer)
-constexpr int C23_STAGES = 2;
-constexpr size_t C23_W2 = 8 * 64 * 128, C23_W3 = 9 * 64 * 128, C23_PAIR1 = 32768, C23_PAIR2 = 16384;
-constexpr size_t C23_SMEM = C23_W2 + C23_W3 + C23_STAGES * C23_PAIR1 + C23_PAIR2 + 4096 + 1024;
-
-struct Conv23Args {
-  const uint8_t* act1;                       // [n][15][16 px][32 ch] padded, pre-swizzled (conv1's output)
-  const __nv_bfloat16 *W2, *W3;              // [64][512], [64][576] K-major
-  const float *b2, *b3;
-  __nv_bfloat16* act3;                       // [n][16][64]
-};
-
-__global__ void __launch_bounds__(DC_THREADS, 1) k_conv23_fused(const Conv23Args a, int nimg) {
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ uint64_t bar_full[C23_STAGES], bar_empty[C23_STAGES], bar_t2full[2], bar_t2empty[2], bar_t3full[2], bar_t3empty[2], bar_a2full, bar_a2empty;
-  __shared__ uint32_t tmem_base_s;
-  __shared__ __align__(16) float sb2[64], sb3[64];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* sW2 = smem;
-  uint8_t* sW3 = sW2 + C23_W2;
-  uint8_t* sA1 = sW3 + C23_W3;                       // C23_STAGES x act1 pair; the junk groups of the last stage read on into sA2
-  uint8_t* sA2 = sA1 + C23_STAGES * C23_PAIR1;       // act2 pair [2][8][8 px][64 ch] (+ 4 KB behind it for conv3's junk groups)
-  if (tid < 64) { sb2[tid] = __ldg(a.b2 + tid); sb3[tid] = __ldg(a.b3 + tid); }
-  if (tid == 0) {
-    for (int i = 0; i < C23_STAGES; i++) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
-    for (int i = 0; i < 2; i++) { mbar_init(&bar_t2full[i], 1); mbar_init(&bar_t2empty[i], 8); mbar_init(&bar_t3full[i], 1); mbar_init(&bar_t3empty[i], 8); }
-    mbar_init(&bar_a2full, 8); mbar_init(&bar_a2empty, 1);
-    fence_barrier_init();
-  }
-  __syncwarp();
-  if (warp == 0) tmem_alloc(&tmem_base_s, 256);  // columns 0-63, 64-127: conv2 accumulators; 128-191, 192-255: conv3
-  for (int i = tid; i < 8 * 64 * 8; i += DC_THREADS) {
-    const int kb = i >> 9, row = (i >> 3) & 63, ch = i & 7;
-    cp_async16(smem_u32(sW2 + kb * 64 * 128 + row * 128 + ((ch ^ (row & 7)) << 4)), a.W2 + (size_t)row * 512 + kb * BK + ch * 8, true);
-  }
-  for (int i = tid; i < 9 * 64 * 8; i += DC_THREADS) {
-    const int kb = i >> 9, row = (i >> 3) & 63, ch = i & 7;
-    cp_async16(smem_u32(sW3 + kb * 64 * 128 + row * 128 + ((ch ^ (row & 7)) << 4)), a.W3 + (size_t)row * 576 + kb * BK + ch * 8, true);
-  }
-  cp_async_commit();
-  for (int i = tid; i < (int)(C23_PAIR2 + 4096) / 16; i += DC_THREADS) *reinterpret_cast<uint4*>(sA2 + i * 16) = make_uint4(0, 0, 0, 0);  // padding lines stay zero
-  cp_async_wait<0>();
-  fence_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  const uint32_t tmem = tmem_base_s;
-  const int npair = (nimg + 1) >> 1;
-  if (warp == 8) {
-    if (lane == 0) {
-      int k = 0;
-      for (int pr = blockIdx.x; pr < npair; pr += gridDim.x, k++) {
-        const int s = k % C23_STAGES;
-        mbar_wait(&bar_empty[s], ((k / C23_STAGES) & 1) ^ 1);
-        const uint32_t bytes = (2 * pr + 1 < nimg) ? (uint32_t)C23_PAIR1 : (uint32_t)C23_PAIR1 / 2;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&bar_full[s])), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(smem_u32(sA1 + s * C23_PAIR1)), "l"(a.act1 + (size_t)pr * C23_PAIR1), "r"(bytes), "r"(smem_u32(&bar_full[s])) : "memory");
-      }
-    }
-  } else if (warp == 9) {
-    if (lane == 0) {
-      constexpr uint32_t idesc = instr_desc_f16(BM, 64, true);
-      const uint64_t w2 = smem_desc_sw128(smem_u32(sW2)), w3 = smem_desc_sw128(smem_u32(sW3));
-      uint64_t a2d = smem_desc_sw128(smem_u32(sA2));  // conv3: 8-row groups one padded image row (1024 B) apart = the default SBO
-      auto conv3 = [&](int k) {  // on the act2 buffer written by the epilogue of pair k
-        const int t = k & 1;
-        mbar_wait(&bar_t3empty[t], ((k >> 1) & 1) ^ 1);
-        mbar_wait(&bar_a2full, k & 1);
-        tc_fence_after();
-#pragma unroll
-        for (int kb = 0; kb < 9; kb++)
-#pragma unroll
-          for (int k16 = 0; k16 < 4; k16++)
-            umma_bf16(tmem + 128 + t * 64, a2d + (uint64_t)((((kb / 3) * 8 + (kb % 3)) * 128 + k16 * 32) >> 4), w3 + (uint64_t)((kb * 64 * 128 + k16 * 32) >> 4), idesc, (kb | k16) != 0);
-        umma_commit(&bar_a2empty);
-        umma_commit(&bar_t3full[t]);
-      };
-      int k = 0;
-      for (int pr = blockIdx.x; pr < npair; pr += gridDim.x, k++) {
-        const int s = k % C23_STAGES, t = k & 1;
-        mbar_wait(&bar_t2empty[t], ((k >> 1) & 1) ^ 1);
-        mbar_wait(&bar_full[s], (k / C23_STAGES) & 1);
-        tc_fence_after();
-        uint64_t a1d = smem_desc_sw128(smem_u32(sA1 + s * C23_PAIR1));
-        a1d = (a1d & ~((uint64_t)0x3FFF << 32)) | ((uint64_t)(2048 >> 4) << 32);  // conv2: 8-row groups two image rows apart
-#pragma unroll
-        for (int kb = 0; kb < 8; kb++)
-#pragma unroll
-          for (int k16 = 0; k16 < 4; k16++)
-            umma_bf16(tmem + t * 64, a1d + (uint64_t)(((kb >> 1) * 1024 + (kb & 1) * 128 + k16 * 32) >> 4), w2 + (uint64_t)((kb * 64 * 128 + k16 * 32) >> 4), idesc, (kb | k16) != 0);
-        umma_commit(&bar_empty[s]);
-        umma_commit(&bar_t2full[t]);
-        if (k > 0) conv3(k - 1);
-      }
-      if (k > 0) conv3(k - 1);
-    }
-  } else {
-    // accumulator row m = 32 (warp % 4) + lane = 64 * image-in-pair + 8 * oy + ox, columns 32 (warp / 4) .. + 31
-    const int half = warp >> 2, m = 32 * (warp & 3) + lane, img = m >> 6, oy = (m >> 3) & 7, ox = m & 7;
-    const uint32_t tlane = (uint32_t)(32 * (warp & 3)) << 16;
-    auto epi3 = [&](int k, int pr) {  // conv3 accumulator of pair k -> act3
-      const int t = k & 1, n = 2 * pr + img;
-      mbar_wait(&bar_t3full[t], (k >> 1) & 1);
-      tc_fence_after();
-      float v[32];
-      tmem_ld32(tmem + 128 + t * 64 + half * 32 + tlane, v);
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bar_t3empty[t]);
-      if (oy < 4 && ox < 4 && n < nimg) {
-        float eb[32];
-#pragma unroll
-        for (int i = 0; i < 8; i++) *reinterpret_cast<float4*>(eb + 4 * i) = *reinterpret_cast<const float4*>(sb3 + half * 32 + 4 * i);
-        uint32_t o[16];
-#pragma unroll
-        for (int i = 0; i < 16; i++) o[i] = pack_bf16(fmaxf(v[2 * i] + eb[2 * i], 0.0f), fmaxf(v[2 * i + 1] + eb[2 * i + 1], 0.0f));
-        uint4* dst = reinterpret_cast<uint4*>(a.act3 + ((size_t)n * 16 + oy * 4 + ox) * 64 + half * 32);
-#pragma unroll
-        for (int j = 0; j < 4; j++) dst[j] = make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
-      }
-    };
-    int k = 0, prev_pr = 0;
-    for (int pr = blockIdx.x; pr < npair; pr += gridDim.x, k++) {
-      const int t = k & 1;
-      mbar_wait(&bar_t2full[t], (k >> 1) & 1);
-      tc_fence_after();
-      float v[32];
-      tmem_ld32(tmem + t * 64 + half * 32 + tlane, v);
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bar_t2empty[t]);
-      uint32_t o[16];
-      {
-        float eb[32];
-#pragma unroll
-        for (int i = 0; i < 8; i++) *reinterpret_cast<float4*>(eb + 4 * i) = *reinterpret_cast<const float4*>(sb2 + half * 32 + 4 * i);
-#pragma unroll
-        for (int i = 0; i < 16; i++) o[i] = pack_bf16(fmaxf(v[2 * i] + eb[2 * i], 0.0f), fmaxf(v[2 * i + 1] + eb[2 * i + 1], 0.0f));
-      }
-      mbar_wait(&bar_a2empty, (k & 1) ^ 1);  // conv3 of the previous pair has read the act2 buffer
-      if (oy < 6 && ox < 6) {
-        // [8][8 px][64 ch] lines of 128 bytes per image, chunk j of line l at position j ^ (l & 7) (what conv3's descriptor reads)
-        const int l = oy * 8 + ox;
-        uint8_t* line = sA2 + img * 8192 + l * 128;
-#pragma unroll
-        for (int j = 0; j < 4; j++) *reinterpret_cast<uint4*>(line + (((half * 4 + j) ^ (l & 7)) << 4)) = make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
-      }
-      fence_async_smem();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bar_a2full);
-      if (k > 0) epi3(k - 1, prev_pr);
-      prev_pr = pr;
-    }
-    if (k > 0) epi3(k - 1, prev_pr);
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem, 256);
-}
-
 // ------------------------------------------------------------------------------------------------ actor MLP in one kernel
 // latent_pi.0 (576 -> 256, ReLU), latent_pi.2 (256 -> 256, ReLU) and the mu | log_std head (256 -> 16) for a tile of 128
 // observations, without the two trips of the hidden activations through HBM and without two of the three launches (the three
@@ -1419,11 +963,12 @@ struct grp_policy {
   // device copies: bf16 K-major weights in gather order, fp32 biases
   __nv_bfloat16 *w1 = nullptr, *w2 = nullptr, *w3 = nullptr, *wfc = nullptr, *wp0 = nullptr, *wp1 = nullptr, *wh = nullptr;
   float *b1 = nullptr, *b2 = nullptr, *b3 = nullptr, *bfc = nullptr, *bp0 = nullptr, *bp1 = nullptr, *bh = nullptr;
-  // activations (bf16 NHWC) and outputs
-  __nv_bfloat16 *act1 = nullptr, *act2 = nullptr, *act3 = nullptr, *feat = nullptr, *h1 = nullptr, *h2 = nullptr;
-  __nv_bfloat16 *act1_dense = nullptr, *act2_dense = nullptr;  // grp_buffer("act1" / "act2") when the descriptor-addressed chain left them padded + swizzled
-  bool direct_last = false;   // layout of act1 / act2 after the last forward
-  bool act2_valid = true;     // false when conv2 + conv3 ran fused (act2 never reached HBM)
+  // true: 64 x 64 observations with 4 image planes run k_conv1_ws -> k_conv_direct<2|3>, and act1 / act2 are padded + swizzled;
+  // false: k_layer<CONV1|CONV2|CONV3>, and act1 / act2 are dense NHWC
+  bool direct = false;
+  // activations (bf16) and outputs
+  __nv_bfloat16 *act1 = nullptr, *act2 = nullptr, *act3 = nullptr, *feat = nullptr;
+  __nv_bfloat16 *act1_dense = nullptr, *act2_dense = nullptr;  // grp_buffer("act1" / "act2") of the descriptor-addressed chain
   int last_n = 0;
   float *mu = nullptr, *log_std = nullptr;
   std::vector<void*> owned;
@@ -1490,41 +1035,35 @@ extern "C" grp_policy* grp_create(int32_t max_envs, int32_t channels, int32_t he
     if (major != 10) throw std::runtime_error("the policy kernels use tcgen05 / TMEM and need an sm_100-class GPU");
     auto p = std::make_unique<grp_policy>();
     p->sh = s; p->max_envs = max_envs; p->device = device;
+    p->direct = s.H == 64 && s.W == 64 && s.cin == 4;
     CU(cudaSetDevice(device));
     CU(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking));
     const size_t N = max_envs;
     p->params.assign(layout_of(s).total, 0.0f);
-    p->w1 = palloc<__nv_bfloat16>(p.get(), 3 * 32 * (size_t)s.cin * 64); /* W | Wa | Wb (k_conv1_direct) */ p->b1 = palloc<float>(p.get(), 32);
+    p->w1 = palloc<__nv_bfloat16>(p.get(), 3 * 32 * (size_t)s.cin * 64); /* W | Wa | Wb (k_conv1_ws) */ p->b1 = palloc<float>(p.get(), 32);
     p->w2 = palloc<__nv_bfloat16>(p.get(), 64 * 512); p->b2 = palloc<float>(p.get(), 64);
     p->w3 = palloc<__nv_bfloat16>(p.get(), 64 * 576); p->b3 = palloc<float>(p.get(), 64);
     p->wfc = palloc<__nv_bfloat16>(p.get(), 512 * (size_t)s.nflat); p->bfc = palloc<float>(p.get(), 512);
     p->wp0 = palloc<__nv_bfloat16>(p.get(), 256 * (size_t)FEAT_LD); p->bp0 = palloc<float>(p.get(), 256);
     p->wp1 = palloc<__nv_bfloat16>(p.get(), 256 * 256); p->bp1 = palloc<float>(p.get(), 256);
     p->wh = palloc<__nv_bfloat16>(p.get(), HEAD_N * 256); p->bh = palloc<float>(p.get(), HEAD_N);
-    p->act1 = palloc<__nv_bfloat16>(p.get(), std::max(N * s.o1h * s.o1w * 32, (N + 2) * 8192));  // dense [225][32] or padded [15][16][32] per image
-    p->act2 = palloc<__nv_bfloat16>(p.get(), std::max(N * s.o2h * s.o2w * 64, (N + 2) * 4096));  // dense [36][64] or padded [8][8][64] per image
+    // direct: padded [15][16][32] and [8][8][64] per image (+ two images of slack); otherwise dense [o1h][o1w][32] and [o2h][o2w][64]
+    p->act1 = palloc<__nv_bfloat16>(p.get(), p->direct ? (N + 2) * 8192 : N * s.o1h * s.o1w * 32);
+    p->act2 = palloc<__nv_bfloat16>(p.get(), p->direct ? (N + 2) * 4096 : N * s.o2h * s.o2w * 64);
     p->act3 = palloc<__nv_bfloat16>(p.get(), N * s.nflat);
     p->feat = palloc<__nv_bfloat16>(p.get(), N * FEAT_LD);
-    p->h1 = palloc<__nv_bfloat16>(p.get(), N * 256);
-    p->h2 = palloc<__nv_bfloat16>(p.get(), N * 256);
     p->mu = palloc<float>(p.get(), N * s.adim);
     p->log_std = palloc<float>(p.get(), N * s.adim);
-#define SET_SMEM(M_, BN_, E_) CU(cudaFuncSetAttribute(k_layer<M_, BN_, E_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)layer_smem_bytes<M_, BN_>()))
+#define SET_SMEM(M_, BN_, E_) CU(cudaFuncSetAttribute(k_layer<M_, BN_, E_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)layer_smem_bytes<BN_>()))
     SET_SMEM(CONV1, 32, EPI_RELU);
-    CU(cudaFuncSetAttribute(k_conv1_image, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C1_SMEM));
     CU(cudaFuncSetAttribute(k_mlp_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MF_SMEM));
-    CU(cudaFuncSetAttribute(k_conv23_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C23_SMEM));
     CU(cudaFuncSetAttribute(k_conv_direct<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dc_smem<2>()));
     CU(cudaFuncSetAttribute(k_conv_direct<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dc_smem<3>()));
     CU(cudaFuncSetAttribute(k_conv1_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CW_SMEM));
-    CU(cudaFuncSetAttribute(k_conv1_direct<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CD_SMEM));
-    CU(cudaFuncSetAttribute(k_conv1_direct<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CD_SMEM));
     CU(cudaDeviceGetAttribute(&p->num_sms, cudaDevAttrMultiProcessorCount, device));
     SET_SMEM(CONV2, 64, EPI_RELU);
     SET_SMEM(CONV3, 64, EPI_RELU);
     SET_SMEM(DENSE, 128, EPI_FEATURES);
-    SET_SMEM(DENSE, 128, EPI_RELU);
-    SET_SMEM(DENSE, HEAD_N, EPI_HEAD);
 #undef SET_SMEM
     return p.release();
   } catch (const std::exception& e) {
@@ -1634,20 +1173,23 @@ extern "C" int32_t grp_get_params(const grp_policy* p, float* host, int64_t coun
   return 0;
 }
 
+// Every kernel of the forward is launched with programmatic dependent launch: it may begin while the previous one on the stream
+// is still running, and waits for it at griddepcontrol.wait before it reads that kernel's output (see k_layer).
+template <class... Params, class... Args>
+static void launch_pdl(grp_policy* p, void (*kernel)(Params...), dim3 grid, int threads, size_t smem, cudaStream_t st, Args... args) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid; cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  CU(cudaLaunchKernelEx(&cfg, kernel, args...));
+  p->launches++;
+}
+
 template <int MODE, int BN, int EPI>
 static void launch_layer(grp_policy* p, const LayerArgs& a, int n_total, cudaStream_t st) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((a.M + BM - 1) / BM, n_total / BN);
-  cfg.blockDim = dim3(THREADS);
-  cfg.dynamicSmemBytes = layer_smem_bytes<MODE, BN>();
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;  // PDL: see griddepcontrol in k_layer
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  CU(cudaLaunchKernelEx(&cfg, k_layer<MODE, BN, EPI>, a));
-  p->launches++;
+  launch_pdl(p, k_layer<MODE, BN, EPI>, dim3((a.M + BM - 1) / BM, n_total / BN), THREADS, layer_smem_bytes<BN>(), st, a);
 }
 
 extern "C" int32_t grp_forward(grp_policy* p, const uint8_t* obs_dev, float* actions_dev, const float* noise_dev, int32_t n, void* stream) {
@@ -1659,142 +1201,44 @@ extern "C" int32_t grp_forward(grp_policy* p, const uint8_t* obs_dev, float* act
     CU(cudaSetDevice(p->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
     const Shape& s = p->sh;
-    // GRP_EVENTS=1 (development aid): an event after every launch; grp_forward then blocks and prints the time between them
-    static const bool ev_on = getenv("GRP_EVENTS") != nullptr;
-    cudaEvent_t evs[9]; int nev = 0;
-    auto mark = [&]() { if (ev_on && nev < 9) { cudaEventCreate(&evs[nev]); cudaEventRecord(evs[nev], st); nev++; } };
-    struct EvPrint { bool on; cudaEvent_t* e; int* n; ~EvPrint() { if (!on || *n < 2) return; cudaEventSynchronize(e[*n - 1]); fprintf(stderr, "[grp_forward]");
-      for (int i = 1; i < *n; i++) { float ms = 0; cudaEventElapsedTime(&ms, e[i - 1], e[i]); fprintf(stderr, " %.1f us", ms * 1e3f); } fprintf(stderr, "\n"); for (int i = 0; i < *n; i++) cudaEventDestroy(e[i]); } } evp{ev_on, evs, &nev};
-    mark();
+    p->last_n = n;
+    const dim3 pairs(std::min((n + 1) / 2, p->num_sms));  // k_conv_direct: persistent CTAs over image pairs
     LayerArgs a{};
-    // conv1: uint8 planes -> [n*o1h*o1w][32]
+    // conv1: uint8 planes -> act1
     a.A = obs_dev; a.W = p->w1; a.bias = p->b1; a.out = p->act1;
     a.M = n * s.o1h * s.o1w; a.K = s.cin * 64; a.ldo = 32; a.scale = 1.0f / 255.0f;
     a.C = s.C; a.H = s.H; a.W_ = s.W; a.ih = s.H; a.iw = s.W; a.oh = s.o1h; a.ow = s.o1w;
-    const bool image_kernel = s.H == 64 && s.W == 64 && s.cin == 4 && !getenv("GRP_CONV1_GENERIC");
-    const char* c1 = getenv("GRP_CONV1");  // development switch: "image" = im2col per image, "generic" = gather layer; default = descriptor-addressed
-    const char* cc = getenv("GRP_CONV23");  // "gather" = im2col-on-the-fly conv2 / conv3 (k_layer); default = descriptor-addressed when conv1 is
-    const bool direct1 = image_kernel && !(c1 && (!strcmp(c1, "image") || !strcmp(c1, "generic")));  // "sync" is a direct variant too
-    const bool direct23 = direct1 && !(cc && !strcmp(cc, "gather"));
-    p->direct_last = direct23; p->last_n = n;
-    if (direct23) a.ldo = 0;  // conv1 leaves act1 in the padded, swizzled layout conv2's descriptor reads
-    if (direct1) {
-      // no im2col: the tensor core reads the (fp16) image rows through its shared-memory descriptor (k_conv1_direct)
-      cudaLaunchConfig_t cfg{};
-      const bool dedicated = getenv("GRP_CONV1_ISSUER") && atoi(getenv("GRP_CONV1_ISSUER")) != 0;
-      if (!(c1 && !strcmp(c1, "sync"))) {  // default: warp-specialised; GRP_CONV1=sync selects the block-barrier version
-        cfg.gridDim = dim3(std::min(n, p->num_sms)); cfg.blockDim = dim3(CW_THREADS); cfg.dynamicSmemBytes = CW_SMEM; cfg.stream = st;
-        cudaLaunchAttribute attrw[1];
-        attrw[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attrw[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attrw; cfg.numAttrs = 1;
-        CU(cudaLaunchKernelEx(&cfg, k_conv1_ws, a, (int)n));
-        p->launches++;
-      } else {
-      cfg.gridDim = dim3(std::min(n, p->num_sms)); cfg.blockDim = dim3(CD_THREADS + (dedicated ? 32 : 0)); cfg.dynamicSmemBytes = CD_SMEM; cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr; cfg.numAttrs = 1;
-      if (dedicated) CU(cudaLaunchKernelEx(&cfg, k_conv1_direct<true>, a, (int)n));
-      else CU(cudaLaunchKernelEx(&cfg, k_conv1_direct<false>, a, (int)n));
-      p->launches++;
-      }
-    } else if (image_kernel && !(c1 && !strcmp(c1, "generic"))) {
-      // one image per CTA, planes staged by a bulk copy (k_conv1_image); any other observation shape takes the generic layer
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(n); cfg.blockDim = dim3(C1_THREADS); cfg.dynamicSmemBytes = C1_SMEM; cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr; cfg.numAttrs = 1;
-      CU(cudaLaunchKernelEx(&cfg, k_conv1_image, a));
-      p->launches++;
+    if (p->direct) {
+      a.ldo = 0;  // act1 in the padded, swizzled layout k_conv_direct<2>'s descriptor reads
+      launch_pdl(p, k_conv1_ws, dim3(std::min(n, p->num_sms)), CW_THREADS, CW_SMEM, st, a, (int)n);
     } else {
       launch_layer<CONV1, 32, EPI_RELU>(p, a, 32, st);
     }
-    mark();
-    auto launch_direct = [&](auto kernel, size_t smem_bytes, const LayerArgs& la) {
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(std::min((n + 1) / 2, p->num_sms)); cfg.blockDim = dim3(DC_THREADS); cfg.dynamicSmemBytes = smem_bytes; cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr; cfg.numAttrs = 1;
-      CU(cudaLaunchKernelEx(&cfg, kernel, la, (int)n));
-      p->launches++;
-    };
-    // GRP_CONV23=fused: conv2 + conv3 in one kernel, act2 stays on the SM.  Measured equal to the two kernels (46 us against 26.6 + 26.6
-    // event-timed, the forward 0.115 ms either way: both are bound by the rate of N = 64 MMAs, not by act2's traffic), so the default
-    // stays the split pair, whose intermediate the tests can read.
-    const bool fused23 = direct23 && cc && !strcmp(cc, "fused");
-    if (fused23) {
-      Conv23Args ca{};
-      ca.act1 = reinterpret_cast<const uint8_t*>(p->act1); ca.W2 = p->w2; ca.W3 = p->w3; ca.b2 = p->b2; ca.b3 = p->b3; ca.act3 = p->act3;
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(std::min((n + 1) / 2, p->num_sms)); cfg.blockDim = dim3(DC_THREADS); cfg.dynamicSmemBytes = C23_SMEM; cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr; cfg.numAttrs = 1;
-      CU(cudaLaunchKernelEx(&cfg, k_conv23_fused, ca, (int)n));
-      p->launches++;
-      mark(); mark();
-    } else {
     // conv2
     a = LayerArgs{};
     a.A = p->act1; a.W = p->w2; a.bias = p->b2; a.out = p->act2;
     a.M = n * s.o2h * s.o2w; a.K = 512; a.ldo = 64; a.scale = 1.0f;
     a.ih = s.o1h; a.iw = s.o1w; a.oh = s.o2h; a.ow = s.o2w;
-    if (direct23) launch_direct(k_conv_direct<2>, dc_smem<2>(), a);
+    if (p->direct) launch_pdl(p, k_conv_direct<2>, pairs, DC_THREADS, dc_smem<2>(), st, a, (int)n);
     else launch_layer<CONV2, 64, EPI_RELU>(p, a, 64, st);
-    mark();
     // conv3
     a = LayerArgs{};
     a.A = p->act2; a.W = p->w3; a.bias = p->b3; a.out = p->act3;
     a.M = n * s.o3h * s.o3w; a.K = 576; a.ldo = 64; a.scale = 1.0f;
     a.ih = s.o2h; a.iw = s.o2w; a.oh = s.o3h; a.ow = s.o3w;
-    if (direct23) launch_direct(k_conv_direct<3>, dc_smem<3>(), a);
+    if (p->direct) launch_pdl(p, k_conv_direct<3>, pairs, DC_THREADS, dc_smem<3>(), st, a, (int)n);
     else launch_layer<CONV3, 64, EPI_RELU>(p, a, 64, st);
-    mark();
-    }
-    p->act2_valid = !fused23;
     // linear -> 512 features + the two direct features
     a = LayerArgs{};
     a.A = p->act3; a.W = p->wfc; a.bias = p->bfc; a.out = p->feat;
     a.M = n; a.K = s.nflat; a.lda = s.nflat; a.ldo = FEAT_LD; a.scale = 1.0f;
     a.C = s.C; a.H = s.H; a.W_ = s.W; a.obs = obs_dev;
     launch_layer<DENSE, 128, EPI_FEATURES>(p, a, 512, st);
-    mark();
-    const char* mlp = getenv("GRP_MLP");  // "layers" = one kernel per layer (writes h1 / h2); default = fused
-    if (!(mlp && !strcmp(mlp, "layers"))) {
-      MlpArgs ma{};
-      ma.feat = p->feat; ma.W0 = p->wp0; ma.W1 = p->wp1; ma.Wh = p->wh; ma.b0 = p->bp0; ma.b1 = p->bp1; ma.bh = p->bh;
-      ma.M = n; ma.adim = s.adim; ma.mu = p->mu; ma.log_std = p->log_std; ma.action = actions_dev; ma.noise = noise_dev;
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3((n + BM - 1) / BM); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = MF_SMEM; cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr; cfg.numAttrs = 1;
-      CU(cudaLaunchKernelEx(&cfg, k_mlp_fused, ma));
-      p->launches++;
-      mark();
-      return 0;
-    }
-    // latent_pi
-    a = LayerArgs{};
-    a.A = p->feat; a.W = p->wp0; a.bias = p->bp0; a.out = p->h1;
-    a.M = n; a.K = FEAT_LD; a.lda = FEAT_LD; a.ldo = 256; a.scale = 1.0f;
-    launch_layer<DENSE, 128, EPI_RELU>(p, a, 256, st);
-    a.A = p->h1; a.W = p->wp1; a.bias = p->bp1; a.out = p->h2; a.K = 256; a.lda = 256;
-    launch_layer<DENSE, 128, EPI_RELU>(p, a, 256, st);
-    // mu | log_std -> squashed Gaussian action
-    a = LayerArgs{};
-    a.A = p->h2; a.W = p->wh; a.bias = p->bh;
-    a.M = n; a.K = 256; a.lda = 256; a.scale = 1.0f;
-    a.mu = p->mu; a.log_std = p->log_std; a.action = actions_dev; a.noise = noise_dev; a.adim = s.adim;
-    launch_layer<DENSE, HEAD_N, EPI_HEAD>(p, a, HEAD_N, st);
+    // latent_pi and the mu | log_std head -> squashed Gaussian action
+    MlpArgs ma{};
+    ma.feat = p->feat; ma.W0 = p->wp0; ma.W1 = p->wp1; ma.Wh = p->wh; ma.b0 = p->bp0; ma.b1 = p->bp1; ma.bh = p->bh;
+    ma.M = n; ma.adim = s.adim; ma.mu = p->mu; ma.log_std = p->log_std; ma.action = actions_dev; ma.noise = noise_dev;
+    launch_pdl(p, k_mlp_fused, dim3((n + BM - 1) / BM), THREADS, MF_SMEM, st, ma);
     return 0;
   } catch (const std::exception& e) {
     g_err = e.what();
@@ -1814,10 +1258,9 @@ extern "C" int32_t grp_buffer(grp_policy* p, const char* name, void** ptr, uint6
   else if (k == "features") { d = p->feat; sz = N * FEAT_LD * 2; }
   else if (k == "act1" || k == "act2") {
     const int layer = k == "act1" ? 1 : 2;
-    if (layer == 2 && !p->act2_valid) { g_err = "act2 does not exist after a forward with the fused conv2 + conv3 kernel (GRP_CONV23=split|gather keeps it)"; return 1; }
     sz = layer == 1 ? N * s.o1h * s.o1w * 32 * 2 : N * s.o2h * s.o2w * 64 * 2;
     d = layer == 1 ? (void*)p->act1 : (void*)p->act2;
-    if (p->direct_last) {  // the last forward left them padded + swizzled: hand out a dense copy
+    if (p->direct) {  // the buffer is padded + swizzled: hand out a dense copy
       __nv_bfloat16*& dense = layer == 1 ? p->act1_dense : p->act2_dense;
       try {
         CU(cudaSetDevice(p->device));
@@ -1831,8 +1274,6 @@ extern "C" int32_t grp_buffer(grp_policy* p, const char* name, void** ptr, uint6
     }
   }
   else if (k == "act3") { d = p->act3; sz = N * (size_t)s.nflat * 2; }
-  else if (k == "h1") { d = p->h1; sz = N * 256 * 2; }
-  else if (k == "h2") { d = p->h2; sz = N * 256 * 2; }
   else { g_err = "unknown buffer name '" + k + "'"; return 1; }
   *ptr = d;
   if (bytes) *bytes = sz;

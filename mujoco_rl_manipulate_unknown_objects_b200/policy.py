@@ -81,7 +81,7 @@ class GripperPolicy:
         return raw.view(dtype).reshape(shape)
 
     def buffer(self, name, shape, dtype):
-        """Intermediate activation ("act1", "act2", "act3", "h1", "h2": bf16 NHWC) as a torch tensor (tests)."""
+        """Intermediate activation of the last forward ("act1", "act2", "act3": bf16 NHWC) as a torch tensor (tests)."""
         return self._tensor(name, shape, dtype)
 
     # ------------------------------------------------------------------ parameters
