@@ -147,6 +147,30 @@ GRS_API uint64_t grs_launch_count(const grs_sim* sim);
 GRS_API float grs_step_kernel_ms(grs_sim* sim, int32_t reset_counters);
 
 /* ---------------------------------------------------------------------------------------------------------------
+ * Asynchronous step in the style of EnvPool (DESIGN.md §3.1 "Asynchronous step").  Each environment is RETURNED (its
+ * outputs were handed out, it waits for an action), PENDING (action sent, step not started), PARKED (step partly done,
+ * its state in HBM) or READY (step done, outputs not handed out yet).  Outputs stay in the grs_buffer arrays, row = id.
+ * Needs auto_reset=1.  While asynchronous mode is on, grs_step, grs_step_host, grs_reset, grs_reset_host, grs_substep,
+ * grs_set_state and grs_debug_step fail.  send and recv do not synchronise with the host: invalid ids set a sticky error
+ * that the next grs_async_status or grs_async_end reports (and clears). */
+/* EnvPool async_reset: every environment becomes READY with its current outputs, in id order; the first
+ * num_envs / batch recv calls return them without stepping.  1 <= batch <= num_envs. */
+GRS_API int32_t grs_async_begin(grs_sim* sim, int32_t batch, void* stream);
+/* EnvPool send(action, env_id): actions_dev f32[n][action_dim], env_ids_dev int32[n]; each id must be RETURNED and
+ * appear once; it becomes PENDING. */
+GRS_API int32_t grs_async_send(grs_sim* sim, const float* actions_dev, const int32_t* env_ids_dev, int32_t n, void* stream);
+/* EnvPool recv(): writes `batch` environment ids to out_ids_dev (int32) in completion order (FIFO across calls) and marks
+ * them RETURNED.  With fewer than `batch` READY it first steps every PENDING and PARKED environment until `batch` are
+ * READY; environments still mid-step then are PARKED at a substep boundary.  Missing ids (too few in flight) read -1. */
+GRS_API int32_t grs_async_recv(grs_sim* sim, int32_t* out_ids_dev, void* stream);
+/* leaves asynchronous mode; fails while any environment is PENDING, PARKED or READY */
+GRS_API int32_t grs_async_end(grs_sim* sim);
+/* synchronises; counts[0..3] = environments RETURNED / PENDING / PARKED / READY, counts[4] = sticky error bits
+ * (1: a sent id was not RETURNED or was duplicated, 2: a sent id was out of range, 4: a recv found fewer than batch);
+ * non-zero error bits make the call fail with their description */
+GRS_API int32_t grs_async_status(grs_sim* sim, int64_t counts[5]);
+
+/* ---------------------------------------------------------------------------------------------------------------
  * Policy inference during rollouts (tensor cores: tcgen05 + TMEM).  Replaces, for a whole batch of observations,
  * `model.predict(obs, deterministic=...)` (reference eval_agent.py:57, SB3 SACPolicy._predict) = preprocess_obs (/255)
  * -> AugmentedNatureCNN.forward (reference models/feature_extractor.py:39-49) -> actor latent_pi [256,256]

@@ -33,7 +33,7 @@ SYMBOLS = ["grs_last_error", "grs_default_config", "grs_create", "grs_destroy", 
            "grs_obs_shape", "grs_stream", "grs_reset", "grs_step", "grs_step_host", "grs_reset_host", "grs_substep",
            "grs_buffer", "grs_get_state", "grs_set_state", "grs_max_contacts", "grs_get_contacts", "grs_debug_step",
            "grs_model_get", "grs_model_get_int", "grs_model_names", "grs_compile_only", "grs_render", "grs_launch_count",
-           "grs_step_kernel_ms"]
+           "grs_step_kernel_ms", "grs_async_begin", "grs_async_send", "grs_async_recv", "grs_async_end", "grs_async_status"]
 SYMBOLS += ["grp_last_error", "grp_create", "grp_destroy", "grp_num_params", "grp_set_params", "grp_get_params", "grp_forward",
             "grp_buffer", "grp_shape", "grp_launch_count", "grp_stream"]
 
@@ -94,6 +94,11 @@ def load():
     L.grs_launch_count.argtypes = [vp]
     L.grs_step_kernel_ms.restype = C.c_float
     L.grs_step_kernel_ms.argtypes = [vp, i32]
+    L.grs_async_begin.argtypes = [vp, i32, vp]
+    L.grs_async_send.argtypes = [vp, vp, vp, i32, vp]
+    L.grs_async_recv.argtypes = [vp, vp, vp]
+    L.grs_async_end.argtypes = [vp]
+    L.grs_async_status.argtypes = [vp, C.POINTER(i64)]
     L.grp_last_error.restype = C.c_char_p
     L.grp_create.restype = vp
     L.grp_create.argtypes = [i32, i32, i32, i32, i32, i32]

@@ -288,10 +288,37 @@ __device__ __forceinline__ unsigned long long global_ns() {
   return t;
 }
 
+// ---- asynchronous step (EnvPool send / recv; DESIGN.md §3.1 "Asynchronous step").  Every environment of a pool is in one
+// of four states.  A launch of the ASYNC instantiation integrates the pending and parked environments until `need` more of
+// them have finished; an environment still mid-step at that point is parked at a substep boundary: its state row (which
+// already holds qpos, qvel, ctrl, warm start and the env flags) plus a park record with the controller and the workspace
+// values an agent step carries across substeps.  Resuming it in a later launch reproduces the synchronous step bit for bit.
+enum AsyncState { A_RETURNED = 0, A_PENDING = 1, A_PARKED = 2, A_READY = 3 };
+// park record [N][PK_STRIDE] floats (every integer in it is < 2^24, so a float holds it exactly)
+enum { PK_STAGE = 0, PK_I, PK_STEP_LIMIT, PK_OPEN_CLOSE, PK_DELTAS, PK_INIT_OBJ /*3*/, PK_NSA = 8, PK_NSB, PK_NSC, PK_ITERS, PK_NCONMAX,
+       PK_FLAGS, PK_FAIL, PK_GRASPED, PK_REACHED_TARGET, PK_REACHED_INITIAL, PK_TQ_REC = 18 /*5*/, PK_TGT = 24 /*5*/, PK_INIT_Q = 32 /*5*/,
+       PK_QPOS = 40 /*NQ: qpos as it entered the last position stage, before kinematics renormalised the free joint's quaternion*/,
+       PK_STRIDE = 56 };
+// control words [AC_WORDS] ints: the ready ring (slot of its oldest entry, number of entries), sticky error bits, this launch's
+// goal, the queue of this launch and its class sizes / cursors (class 0 = parked, 1 + order_class = pending)
+enum { AC_HEAD = 0, AC_READY, AC_ERR, AC_NEED, AC_NQUEUE, AC_SIZES = 32, AC_CURSORS = 64, AC_WORDS = 96 };
+enum { AERR_SEND = 1, AERR_SEND_RANGE = 2, AERR_RECV_SHORT = 4 };
+constexpr int ASYNC_CLASSES = 2 + 3 * ORDER_BUCKETS;
+constexpr int S_RESUME = S_FINISH + 1;  // a parked environment whose state was loaded this round (its position stage runs now)
+struct AsyncArgs {
+  int* astate;  // [N] AsyncState
+  int* ctl;     // [AC_WORDS]
+  float* park;  // [N][PK_STRIDE]
+  int* waited;  // [N] 1: pending and already queued by an earlier launch that stopped before fetching it
+};
+
 // FUSED = true: a block whose physics work is exhausted goes on to build observations (render_phase) instead of exiting, so
 // the rasteriser fills the SMs that idle while the longest substep chains finish.  Needs blockDim.x == RTHREADS.
-template <bool TIMING, bool FUSED>
-__global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_ls(SimBuffers s, EnvCfg c, const float* __restrict__ actions, int adim, RenderScene sc, ObsArgs oa) {
+// ASYNC = true: the asynchronous step above (not FUSED: the observation phase would wait for environments that get parked).
+template <bool TIMING, bool FUSED, bool ASYNC = false>
+__global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_ls(SimBuffers s, EnvCfg c, const float* __restrict__ actions, int adim, RenderScene sc, ObsArgs oa,
+                                                                                  AsyncArgs aa) {
+  static_assert(!(ASYNC && (FUSED || TIMING)), "the asynchronous step has its own instantiation");
   unsigned smid = 0;
   if (FUSED && threadIdx.x == 0) {
     atomicMin(s.tstamp, global_ns());
@@ -348,6 +375,77 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
     // ---- controller round: finish / fetch / decide (per warp, no block-wide dependency)
     LS_T0();
     bool dyn = false, pos = false;
+    if constexpr (ASYNC) {
+      // stop rule: once `need` environments have finished in this launch (s.queue[3] counts them), nothing new is fetched and
+      // every environment still mid-step is parked at its next substep boundary
+      const bool stop = *reinterpret_cast<volatile int*>(s.queue + 3) >= __ldg(aa.ctl + AC_NEED);
+      if (t.stage == S_RESUME) {
+        if (stop) {
+          t.stage = S_IDLE;  // dropped before it moved: its state row and park record still describe it, it stays parked
+        } else {
+          // restore the controller and run the substep it was parked before, without ticking again
+          const float* pk = aa.park + (size_t)t.env * PK_STRIDE;
+          t.stage = (int)pk[PK_STAGE]; t.i = (int)pk[PK_I]; t.step_limit = (int)pk[PK_STEP_LIMIT];
+          t.open_close = pk[PK_OPEN_CLOSE]; t.deltas = pk[PK_DELTAS];
+          for (int k = 0; k < 3; k++) t.init_obj[k] = pk[PK_INIT_OBJ + k];
+          t.k.nsa = (int)pk[PK_NSA]; t.k.nsb = (int)pk[PK_NSB]; t.k.nsc = (int)pk[PK_NSC]; t.k.iters = (int)pk[PK_ITERS];
+          t.k.nconmax = (int)pk[PK_NCONMAX]; t.k.flags = (int)pk[PK_FLAGS]; t.k.fail = (int)pk[PK_FAIL]; t.k.object_grasped = (int)pk[PK_GRASPED];
+          t.k.reached_target = pk[PK_REACHED_TARGET] != 0.0f; t.k.reached_initial = pk[PK_REACHED_INITIAL] != 0.0f;
+          t.k.tq_rec = lane < 5 ? pk[PK_TQ_REC + lane] : 0.0f;
+          if (lane < 5) { w.tgt[lane] = pk[PK_TGT + lane]; w.init_q[lane] = pk[PK_INIT_Q + lane]; }
+          __syncwarp();
+          dyn = true;
+        }
+      } else if (t.stage == S_LOADED && stop) {
+        t.stage = S_IDLE;  // loaded but not begun: it stays pending
+      }
+      if (t.stage == S_LOADED) t.stage = S_BEGIN;
+      if (t.stage != S_IDLE && !dyn) {
+        dyn = env_tick(m, c, w, t, actions + (size_t)t.env * adim, iters, lane);
+        if (!dyn) {
+          env_writeback(m, c, s, w, t, lane);
+        } else if (stop) {
+          // park: the controls of the next substep are set; store the state and the controller instead of integrating it
+          const int env = t.env;
+          store_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
+          float* pk = aa.park + (size_t)env * PK_STRIDE;
+          if (lane < 5) { pk[PK_TQ_REC + lane] = t.k.tq_rec; pk[PK_TGT + lane] = w.tgt[lane]; pk[PK_INIT_Q + lane] = w.init_q[lane]; }
+          if (lane == 0) {
+            pk[PK_STAGE] = (float)t.stage; pk[PK_I] = (float)t.i; pk[PK_STEP_LIMIT] = (float)t.step_limit;
+            pk[PK_OPEN_CLOSE] = t.open_close; pk[PK_DELTAS] = t.deltas;
+            for (int k = 0; k < 3; k++) pk[PK_INIT_OBJ + k] = t.init_obj[k];
+            pk[PK_NSA] = (float)t.k.nsa; pk[PK_NSB] = (float)t.k.nsb; pk[PK_NSC] = (float)t.k.nsc; pk[PK_ITERS] = (float)t.k.iters;
+            pk[PK_NCONMAX] = (float)t.k.nconmax; pk[PK_FLAGS] = (float)t.k.flags; pk[PK_FAIL] = (float)t.k.fail; pk[PK_GRASPED] = (float)t.k.object_grasped;
+            pk[PK_REACHED_TARGET] = t.k.reached_target ? 1.0f : 0.0f; pk[PK_REACHED_INITIAL] = t.k.reached_initial ? 1.0f : 0.0f;
+            aa.astate[env] = A_PARKED;
+          }
+          __syncwarp();
+          t.stage = S_IDLE;
+          dyn = false;
+        }
+      }
+      if (t.stage == S_IDLE && !exhausted && !stop) {
+        const int nstatic = gridDim.x * (blockDim.x >> 5);
+        int slot = first ? static_slot(s, nstatic) : nstatic + next_env(s.queue, lane);
+        first = false;
+        if (slot < __ldg(aa.ctl + AC_NQUEUE)) {
+          const int env = __ldg(s.order + slot);
+          t.env = env;
+          load_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
+          t.stage = S_LOADED;
+          if (__ldg(aa.astate + env) == A_PARKED) {
+            // the position stage below has to see the qpos the synchronous step's position stage saw (kinematics
+            // renormalises the free joint's quaternion in place, and renormalising twice can move its last bit)
+            if (lane < NQ) w.qpos[lane] = aa.park[(size_t)env * PK_STRIDE + PK_QPOS + lane];
+            __syncwarp();
+            t.stage = S_RESUME;
+          }
+          pos = true;
+        } else {
+          exhausted = true;
+        }
+      }
+    } else {
     if (t.stage == S_LOADED) t.stage = S_BEGIN;
     if (t.stage != S_IDLE) {
       dyn = env_tick(m, c, w, t, actions + (size_t)t.env * adim, iters, lane);
@@ -368,6 +466,7 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
       } else {
         exhausted = true;
       }
+    }
     }
     pos = pos || dyn;
     LS_T1(0);
@@ -399,6 +498,13 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
     if (s.ls_mask & 4) __syncthreads();
     LS_T0();
     if (dyn) euler_integrate(m, w, lane);
+    if constexpr (ASYNC) {
+      if (pos) {  // PK_QPOS: what this position stage starts from, for a resume after a park in the next round
+        __syncwarp();
+        if (lane < NQ) aa.park[(size_t)t.env * PK_STRIDE + PK_QPOS + lane] = w.qpos[lane];
+        __syncwarp();
+      }
+    }
     if (pos) kinematics(m, w, lane);
     LS_T1(4);
     if (s.ls_mask & 8) __syncthreads();
@@ -441,6 +547,82 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
   }
 #undef LS_T0
 #undef LS_T1
+}
+
+// ---- the small kernels around the asynchronous step (grs_async_* in gripper_sim.cu)
+
+// every environment ready with its current outputs, in id order
+__global__ void k_async_begin(AsyncArgs aa, int* __restrict__ ring, int n) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env < n) { aa.astate[env] = A_READY; aa.waited[env] = 0; ring[env] = env; }
+  if (env < AC_WORDS) aa.ctl[env] = env == AC_READY ? n : 0;
+}
+
+// send: each listed environment must be returned; its action row is written and it becomes pending
+__global__ void k_async_send(AsyncArgs aa, float* __restrict__ actions, int adim, const float* __restrict__ src, const int* __restrict__ ids, int cnt, int n) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= cnt) return;
+  const int env = ids[i];
+  if (env < 0 || env >= n) { atomicOr(aa.ctl + AC_ERR, AERR_SEND_RANGE); return; }
+  if (atomicCAS(aa.astate + env, A_RETURNED, A_PENDING) != A_RETURNED) { atomicOr(aa.ctl + AC_ERR, AERR_SEND); return; }
+  aa.waited[env] = 0;
+  for (int k = 0; k < adim; k++) actions[(size_t)env * adim + k] = src[(size_t)i * adim + k];
+}
+
+// queue of one launch: parked environments first (they carry the long chains), then the pending ones that an earlier launch
+// queued but stopped before fetching, then the other pending ones by order_class; nothing when `batch` environments are ready
+// already.  The second class keeps a pending environment from starving: when the pool holds more environments than the grid
+// has warps, a launch fetches only the head of the queue, and fresh sends of an earlier order_class would otherwise overtake
+// the same tail of the queue launch after launch.  Two passes as k_order_count / k_order_envs; AC_SIZES.. / AC_CURSORS.. are zero.
+__device__ __forceinline__ int async_class(const SimBuffers& s, const AsyncArgs& aa, const float* __restrict__ actions, int adim, int env, int batch) {
+  const int st = aa.astate[env];
+  if (aa.ctl[AC_READY] >= batch || (st != A_PARKED && st != A_PENDING)) return -1;
+  return st == A_PARKED ? 0 : aa.waited[env] ? 1 : 2 + order_class(s, actions, adim, env);
+}
+__global__ void k_async_order_count(SimBuffers s, AsyncArgs aa, const float* __restrict__ actions, int adim, int batch) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= s.n) return;
+  const int c = async_class(s, aa, actions, adim, env, batch);
+  if (c >= 0) atomicAdd(aa.ctl + AC_SIZES + c, 1);
+}
+__global__ void k_async_order_envs(SimBuffers s, AsyncArgs aa, const float* __restrict__ actions, int adim, int batch) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env == 0) {
+    int q = 0;
+    for (int k = 0; k < ASYNC_CLASSES; k++) q += aa.ctl[AC_SIZES + k];
+    aa.ctl[AC_NQUEUE] = q;
+    aa.ctl[AC_NEED] = batch - aa.ctl[AC_READY];
+  }
+  if (env >= s.n) return;
+  const int c = async_class(s, aa, actions, adim, env, batch);
+  if (c < 0) return;
+  int base = 0;
+  for (int k = 0; k < c; k++) base += aa.ctl[AC_SIZES + k];
+  s.order[base + atomicAdd(aa.ctl + AC_CURSORS + c, 1)] = env;
+  if (c > 0) aa.waited[env] = 1;  // read again only by the next launch's queue (a fetched one is parked or ready by then)
+}
+
+// after the step kernel and the observations: the environments this launch finished (s.done_list[0 .. s.queue[3]), in the
+// order they finished) join the ready ring; the first `batch` of the ring are returned.  One block.
+__global__ void k_async_recv(SimBuffers s, AsyncArgs aa, int* __restrict__ ring, int* __restrict__ out_ids, int batch) {
+  const int n = s.n, fin = s.queue[3], head = aa.ctl[AC_HEAD], ready = aa.ctl[AC_READY];  // head < n, ready + fin <= n
+  for (int i = threadIdx.x; i < fin; i += blockDim.x) {
+    const int env = s.done_list[i];
+    ring[(head + ready + i) % n] = env;
+    aa.astate[env] = A_READY;
+  }
+  __syncthreads();
+  const int take = min(batch, ready + fin);
+  for (int j = threadIdx.x; j < batch; j += blockDim.x) {
+    int env = -1;
+    if (j < take) { env = ring[(head + j) % n]; aa.astate[env] = A_RETURNED; }
+    out_ids[j] = env;
+  }
+  if (threadIdx.x == 0) {
+    aa.ctl[AC_HEAD] = (head + take) % n;
+    aa.ctl[AC_READY] = ready + fin - take;
+    if (take < batch) aa.ctl[AC_ERR] |= AERR_RECV_SHORT;
+  }
 }
 
 }  // namespace grs

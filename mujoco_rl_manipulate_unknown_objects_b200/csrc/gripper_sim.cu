@@ -83,6 +83,11 @@ struct grs_sim {
   bool fused_render = false;  // observation phase inside the step kernel (env_lockstep.cuh : render_phase)
   size_t ls_smem = 0;
   ObsArgs obs_args{};
+  // asynchronous step (grs_async_*): per-environment states, control words, park records, ready ring
+  bool async_on = false;
+  int async_batch = 0;
+  AsyncArgs aa{};
+  int* d_ring = nullptr;
 };
 
 template <class T>
@@ -186,6 +191,11 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     s->d_reset_obs = dalloc<unsigned char>(s.get(), obs_bytes);
     s->d_actions = dalloc<float>(s.get(), N * 6);
     s->d_hist = dalloc<float>(s.get(), N * 512 + 512);
+    s->aa.astate = dalloc<int>(s.get(), N);
+    s->aa.ctl = dalloc<int>(s.get(), AC_WORDS);
+    s->aa.park = dalloc<float>(s.get(), N * PK_STRIDE);
+    s->aa.waited = dalloc<int>(s.get(), N);
+    s->d_ring = dalloc<int>(s.get(), N);
     EnvCfg& e = s->ecfg;
     e.max_steps = cfg.max_steps; e.time_horizon = cfg.time_horizon; e.include_roll = cfg.include_roll; e.her_buffer = cfg.her_buffer;
     e.im_reward = cfg.im_reward; e.auto_reset = cfg.auto_reset; e.full_observation = cfg.full_observation;
@@ -229,6 +239,7 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
       raise_dyn_smem((const void*)k_env_step_ls<false, false>, s->ls_smem, device);
       raise_dyn_smem((const void*)k_env_step_ls<false, true>, s->ls_smem, device);
       raise_dyn_smem((const void*)k_env_step_ls<true, false>, s->ls_smem, device);
+      raise_dyn_smem((const void*)k_env_step_ls<false, false, true>, s->ls_smem, device);
       int ls_per_sm = 0;
       if (s->fused_render) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, true>, s->ls_warps * 32, s->ls_smem));
       else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, false>, s->ls_warps * 32, s->ls_smem));
@@ -300,9 +311,13 @@ extern "C" void* grs_stream(const grs_sim* s) { return s ? (void*)s->stream : nu
 #define GUARD(s)                                                          \
   if (!(s)) return fail("null simulator handle");                         \
   if ((s)->compile_only) return fail("handle was created by grs_compile_only: no device state");
+// calls that step, reset or overwrite the state rows would corrupt parked environments: refused in asynchronous mode
+#define GUARD_SYNC(s)                                                                                                        \
+  GUARD(s);                                                                                                                 \
+  if ((s)->async_on) return fail("asynchronous mode is on: drain the pool and call grs_async_end before stepping, resetting or setting state");
 
 extern "C" int32_t grs_reset(grs_sim* s, const uint8_t* mask_dev, void* stream) {
-  GUARD(s);
+  GUARD_SYNC(s);
   try {
     CU(cudaSetDevice(s->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
@@ -328,7 +343,7 @@ static void join_device_path(grs_sim* s) {
 }
 
 extern "C" int32_t grs_step(grs_sim* s, const float* actions_dev, void* stream) {
-  GUARD(s);
+  GUARD_SYNC(s);
   if (!actions_dev) return fail("actions pointer is null");
   try {
     CU(cudaSetDevice(s->device));
@@ -343,9 +358,9 @@ extern "C" int32_t grs_step(grs_sim* s, const float* actions_dev, void* stream) 
       s->launches += 2;
     }
     const bool fused = s->ls_warps > 0 && s->fused_render;
-    if (fused) k_env_step_ls<false, true><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args);
-    else if (s->ls_warps > 0 && s->ls_timing) k_env_step_ls<true, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args);
-    else if (s->ls_warps > 0) k_env_step_ls<false, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args);
+    if (fused) k_env_step_ls<false, true><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
+    else if (s->ls_warps > 0 && s->ls_timing) k_env_step_ls<true, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
+    else if (s->ls_warps > 0) k_env_step_ls<false, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
     else k_env_step<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, st>>>(s->b, s->ecfg, actions_dev, s->adim);
     CU(cudaGetLastError());
     CU(cudaEventRecord(s->ev1[s->ev_n], st));
@@ -368,7 +383,7 @@ static unsigned char* mapped_host_ptr(void* host) {
 
 extern "C" int32_t grs_step_host(grs_sim* s, const float* actions_host, uint8_t* obs_host, float* achieved_host, float* desired_host,
                                  float* reward_host, uint8_t* done_host, float* info_host, uint8_t* terminal_obs_host) {
-  GUARD(s);
+  GUARD_SYNC(s);
   if (!actions_host) return fail("actions pointer is null");
   try {
     CU(cudaSetDevice(s->device));
@@ -411,7 +426,7 @@ extern "C" int32_t grs_step_host(grs_sim* s, const float* actions_host, uint8_t*
 }
 
 extern "C" int32_t grs_reset_host(grs_sim* s, uint8_t* obs_host, float* achieved_host, float* desired_host) {
-  GUARD(s);
+  GUARD_SYNC(s);
   try {
     CU(cudaSetDevice(s->device));
     join_device_path(s);
@@ -426,7 +441,7 @@ extern "C" int32_t grs_reset_host(grs_sim* s, uint8_t* obs_host, float* achieved
 }
 
 extern "C" int32_t grs_substep(grs_sim* s, int32_t n, void* stream) {
-  GUARD(s);
+  GUARD_SYNC(s);
   if (n < 0) return fail("negative substep count");
   try {
     CU(cudaSetDevice(s->device));
@@ -459,6 +474,7 @@ extern "C" int32_t grs_buffer(grs_sim* s, const char* name, void** ptr, uint64_t
   else if (k == "render_state") { p = s->b.render_state; sz = N * RS_STRIDE * 4; }
   else if (k == "debug") { p = s->b.debug; sz = N * DEBUG_STRIDE * 4; }
   else if (k == "actions") { p = s->d_actions; sz = N * 6 * 4; }
+  else if (k == "async_state") { p = s->aa.astate; sz = N * 4; }
   else return fail("unknown buffer name '" + k + "'");
   *ptr = p;
   if (bytes) *bytes = sz;
@@ -487,7 +503,7 @@ extern "C" int32_t grs_get_state(grs_sim* s, float* qpos, float* qvel, float* ct
 
 extern "C" int32_t grs_set_state(grs_sim* s, const float* qpos, const float* qvel, const float* ctrl, const float* warm, const int32_t* flags,
                                  const float* xfrc_z) {
-  GUARD(s);
+  GUARD_SYNC(s);
   try {
     CU(cudaSetDevice(s->device));
     std::vector<float> h((size_t)s->n * ST_STRIDE);
@@ -539,7 +555,7 @@ extern "C" int32_t grs_get_contacts(grs_sim* s, int32_t* ncon, int32_t* geom, fl
 }
 
 extern "C" int32_t grs_debug_step(grs_sim* s) {
-  GUARD(s);
+  GUARD_SYNC(s);
   try {
     CU(cudaSetDevice(s->device));
     launch_queue_kernel_prep(s, s->stream);
@@ -696,4 +712,118 @@ extern "C" float grs_step_kernel_ms(grs_sim* s, int32_t reset_counters) {
   }
   if (reset_counters) { s->ms_sum = 0; s->ms_cnt = 0; }
   return avg;
+}
+
+// ------------------------------------------------------------------------------------------ asynchronous step
+static const char* async_err_text(int bits) {
+  if (bits & AERR_SEND_RANGE) return "grs_async_send: an environment id was out of range";
+  if (bits & AERR_SEND) return "grs_async_send: an environment id was not in the returned state (sent twice, duplicated, or not received yet)";
+  return "grs_async_recv: fewer than `batch` environments were in flight or ready (send actions for the returned ones first)";
+}
+
+extern "C" int32_t grs_async_begin(grs_sim* s, int32_t batch, void* stream) {
+  GUARD(s);
+  if (s->async_on) return fail("grs_async_begin: asynchronous mode is already on (grs_async_end first)");
+  if (batch <= 0 || batch > s->n) return fail("grs_async_begin: batch must be within 1..num_envs");
+  if (!s->cfg.auto_reset) return fail("grs_async_begin: the asynchronous step needs auto_reset=1");
+  if (s->ls_warps <= 0) return fail("grs_async_begin: the asynchronous step needs the lock-step step kernel (GRS_STEP_WARPS > 0)");
+  try {
+    CU(cudaSetDevice(s->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if (st != s->stream) s->last_dev_stream = st;
+    k_async_begin<<<(std::max(s->n, (int)AC_WORDS) + 255) / 256, 256, 0, st>>>(s->aa, s->d_ring, s->n);
+    CU(cudaGetLastError());
+    s->launches++;
+    s->async_on = true;
+    s->async_batch = batch;
+    return 0;
+  } catch (const std::exception& e) { return fail(e.what()); }
+}
+
+extern "C" int32_t grs_async_send(grs_sim* s, const float* actions_dev, const int32_t* env_ids_dev, int32_t n, void* stream) {
+  GUARD(s);
+  if (!s->async_on) return fail("grs_async_send: asynchronous mode is off (grs_async_begin first)");
+  if (n < 0 || n > s->n) return fail("grs_async_send: n must be within 0..num_envs");
+  if (n == 0) return 0;
+  if (!actions_dev || !env_ids_dev) return fail("grs_async_send: null pointer");
+  try {
+    CU(cudaSetDevice(s->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if (st != s->stream) s->last_dev_stream = st;
+    k_async_send<<<(n + 255) / 256, 256, 0, st>>>(s->aa, s->d_actions, s->adim, actions_dev, env_ids_dev, n, s->n);
+    CU(cudaGetLastError());
+    s->launches++;
+    return 0;
+  } catch (const std::exception& e) { return fail(e.what()); }
+}
+
+extern "C" int32_t grs_async_recv(grs_sim* s, int32_t* out_ids_dev, void* stream) {
+  GUARD(s);
+  if (!s->async_on) return fail("grs_async_recv: asynchronous mode is off (grs_async_begin first)");
+  if (!out_ids_dev) return fail("grs_async_recv: null pointer");
+  try {
+    CU(cudaSetDevice(s->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if (st != s->stream) s->last_dev_stream = st;
+    const int B = s->async_batch, g = (s->n + 255) / 256;
+    launch_queue_kernel_prep(s, st);
+    CU(cudaMemsetAsync(s->aa.ctl + AC_SIZES, 0, (AC_WORDS - AC_SIZES) * sizeof(int), st));
+    k_async_order_count<<<g, 256, 0, st>>>(s->b, s->aa, s->d_actions, s->adim, B);
+    k_async_order_envs<<<g, 256, 0, st>>>(s->b, s->aa, s->d_actions, s->adim, B);
+    if (s->ev_n == grs_sim::NEV) harvest_events(s);
+    CU(cudaEventRecord(s->ev0[s->ev_n], st));
+    k_env_step_ls<false, false, true><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, s->d_actions, s->adim, s->scene, s->obs_args, s->aa);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(s->ev1[s->ev_n], st));
+    s->ev_n++;
+    k_render_obs_indexed<<<s->n, RTHREADS, render_phase_smem_bytes(), st>>>(s->scene, s->obs_args, s->b.render_state, s->b.info, IN_STRIDE, s->b.done, s->b.reward,
+                                                                            s->b.done_list, s->b.queue + 3);
+    CU(cudaGetLastError());
+    k_async_recv<<<1, 1024, 0, st>>>(s->b, s->aa, s->d_ring, out_ids_dev, B);
+    CU(cudaGetLastError());
+    s->launches += 5;
+    return 0;
+  } catch (const std::exception& e) { return fail(e.what()); }
+}
+
+// counts[0..3]: environments returned / pending / parked / ready; counts[4]: the sticky error bits (reported and cleared here)
+static int async_counts(grs_sim* s, int64_t counts[5]) {
+  join_device_path(s);
+  CU(cudaStreamSynchronize(s->stream));
+  std::vector<int> st(s->n);
+  int ctl[AC_WORDS];
+  CU(cudaMemcpy(st.data(), s->aa.astate, st.size() * sizeof(int), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(ctl, s->aa.ctl, sizeof ctl, cudaMemcpyDeviceToHost));
+  for (int k = 0; k < 5; k++) counts[k] = 0;
+  for (int v : st) counts[std::min(std::max(v, 0), 3)]++;
+  counts[4] = ctl[AC_ERR];
+  if (ctl[AC_ERR]) CU(cudaMemset(s->aa.ctl + AC_ERR, 0, sizeof(int)));
+  return ctl[AC_ERR];
+}
+
+extern "C" int32_t grs_async_status(grs_sim* s, int64_t counts[5]) {
+  GUARD(s);
+  if (!counts) return fail("grs_async_status: null pointer");
+  try {
+    CU(cudaSetDevice(s->device));
+    if (!s->async_on) { for (int k = 0; k < 5; k++) counts[k] = 0; counts[0] = s->n; return 0; }
+    const int err = async_counts(s, counts);
+    return err ? fail(async_err_text(err)) : 0;
+  } catch (const std::exception& e) { return fail(e.what()); }
+}
+
+extern "C" int32_t grs_async_end(grs_sim* s) {
+  GUARD(s);
+  if (!s->async_on) return 0;
+  try {
+    CU(cudaSetDevice(s->device));
+    int64_t c[5];
+    const int err = async_counts(s, c);
+    if (err) return fail(async_err_text(err));
+    if (c[1] || c[2] || c[3])
+      return fail("grs_async_end: " + std::to_string(c[1]) + " environments pending, " + std::to_string(c[2]) + " parked, " + std::to_string(c[3]) +
+                  " ready but not received: receive them all first");
+    s->async_on = false;
+    return 0;
+  } catch (const std::exception& e) { return fail(e.what()); }
 }

@@ -551,6 +551,21 @@ __global__ void __launch_bounds__(RTHREADS) k_render_obs(RenderScene sc, ObsArgs
   render_obs_env(sc, o, render_state + (size_t)env * RS_STRIDE, env, (unsigned char)inf[IN_GRASP], (unsigned char)inf[IN_PHEROMONE], done ? done[env] != 0 : false, reward, sh, rgb8, rs2);
 }
 
+// The same over a list: block b builds the observation of environment list[b] for b < *count (the asynchronous step renders
+// the environments its launch finished; the grid is sized for the largest possible count).
+__global__ void __launch_bounds__(RTHREADS) k_render_obs_indexed(RenderScene sc, ObsArgs o, const float* __restrict__ render_state, const float* __restrict__ info,
+                                                                int info_stride, const unsigned char* __restrict__ done, float* __restrict__ reward,
+                                                                const int* __restrict__ list, const int* __restrict__ count) {
+  if ((int)blockIdx.x >= *count) return;
+  extern __shared__ __align__(16) unsigned char rsm[];
+  TileShared& sh = *reinterpret_cast<TileShared*>(rsm);
+  unsigned* rgb8 = reinterpret_cast<unsigned*>(rsm + sizeof(TileShared));
+  float* rs2 = reinterpret_cast<float*>(rsm + sizeof(TileShared) + TILE * TILE * sizeof(unsigned));
+  const int env = list[blockIdx.x];
+  const float* inf = info + (size_t)env * info_stride;
+  render_obs_env(sc, o, render_state + (size_t)env * RS_STRIDE, env, (unsigned char)inf[IN_GRASP], (unsigned char)inf[IN_PHEROMONE], done[env] != 0, reward, sh, rgb8, rs2);
+}
+
 // Explicit reset with reset randomisation: observation (and histograms) of the masked environments' new episodes
 __global__ void __launch_bounds__(RTHREADS) k_render_reset(RenderScene sc, ObsArgs o, const unsigned char* __restrict__ mask) {
   extern __shared__ __align__(16) unsigned char rsm[];
@@ -629,6 +644,7 @@ inline void launch_render_obs(const RenderScene& sc, const ObsArgs& o, const flo
   if (!attr) {
     if (cudaFuncSetAttribute(k_render_obs, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)render_phase_smem_bytes()) != cudaSuccess) throw std::runtime_error("cudaFuncSetAttribute(k_render_obs)");
     if (cudaFuncSetAttribute(k_render_reset, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)render_phase_smem_bytes()) != cudaSuccess) throw std::runtime_error("cudaFuncSetAttribute(k_render_reset)");
+    if (cudaFuncSetAttribute(k_render_obs_indexed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)render_phase_smem_bytes()) != cudaSuccess) throw std::runtime_error("cudaFuncSetAttribute(k_render_obs_indexed)");
     attr = true;
   }
   k_render_obs<<<n, RTHREADS, render_phase_smem_bytes(), st>>>(sc, o, render_state, info, IN_STRIDE, done, reward);
