@@ -1,9 +1,10 @@
 // Environment layer on the device: RobotEnv.step / reset (reference simulation/environment/robot_env.py:56-241),
-// Actuator (simulation/controller/actuator.py) and Reward (simulation/environment/reward.py:18-41), fused around
-// the physics substep loop of sim_kernels.cuh.  One warp owns one environment for a whole agent step: state is
-// loaded from HBM once, the data-dependent phase A / B / C loops (up to 3 x max_steps substeps) run on the
-// warp's shared-memory workspace, and one record per environment goes back to HBM.  Warps pull environments
-// from an atomic queue, so ragged trip counts (SURVEY.md F5) do not idle the rest of the grid.
+// Actuator (simulation/controller/actuator.py) and Reward (simulation/environment/reward.py:18-41) around the physics
+// substep of sim_kernels.cuh.  One warp owns one environment: its state is loaded from HBM into the warp's
+// shared-memory workspace, and one record per environment goes back to HBM.  This file holds the state and info
+// records, the IK target, the end-of-step bookkeeping (env_finalize), reset, and the per-environment kernels of the
+// parity tests and the renderer (k_substep, k_contacts, k_debug_step), whose warps pull environments from an atomic
+// queue.  The agent-step kernel, which runs the controller between lock-step substep rounds, is in env_lockstep.cuh.
 #pragma once
 #include "sim_kernels.cuh"
 
@@ -203,7 +204,7 @@ __device__ __forceinline__ float warp_max(float v) {
 }
 
 // robot_env.py:170-241 — everything after the substep loops: failure checks, goals, observation scalars, reward, done,
-// info record (into w.out).  Shared by the sequential and the lock-step step kernels.
+// info record (into w.out).  Called by the step kernel's controller (env_lockstep.cuh : env_tick) when an agent step ends.
 struct StepCounters { int nsa, nsb, nsc, iters, nconmax, flags, fail, object_grasped; bool reached_target, reached_initial; float tq_rec; };
 
 __device__ __noinline__ void env_finalize(const DevModel& m, const EnvCfg& c, WS& w, EnvFlags& f, const float* init_obj, StepCounters& k, int lane) {
@@ -257,103 +258,6 @@ __device__ __noinline__ void env_finalize(const DevModel& m, const EnvCfg& c, WS
   __syncwarp();
 }
 
-// robot_env.py:77-241 — one agent step of one environment, executed by one warp.  `act` is the raw action row.
-// Writes the info record into w.out (IN_* layout) and updates f.
-__device__ __noinline__ void env_step(const DevModel& m, const EnvCfg& c, WS& w, EnvFlags& f, const float4* hv, const int* adj, const float* __restrict__ act, int lane) {
-  float a6[6];
-  if (c.include_roll) { for (int k = 0; k < 6; k++) a6[k] = act[k]; }
-  else { a6[0] = act[0]; a6[1] = act[1]; a6[2] = act[2]; a6[3] = 0; a6[4] = act[3]; a6[5] = act[4]; }
-  const float open_close = a6[5];
-  float init_obj[3];
-  for (int k = 0; k < 3; k++) init_obj[k] = w.xpos[m.body_object][k];
-  if (lane < 5) w.init_q[lane] = w.qpos[lane];
-  if (lane == 0) get_target_pose(m, c, w, a6);
-  __syncwarp();
-  float tq_rec = lane < 5 ? w.tgt[lane] : 0.0f;
-  const float scale = lane < 3 ? 1.0f / c.max_trans : 1.0f / c.max_rot;
-  int nsa = 0, nsb = 0, nsc = 0, iters = 0, nconmax = w.ncon, flags = w.overflow;  // the contact set the step starts from counts (its position stage ran at load time)
-  bool reached_target = false, reached_initial = false;
-  int step_limit = c.max_steps;
-  // phase A: P-control towards the IK target (robot_env.py:97-110)
-  for (int i = 0; i < c.max_steps; i++) {
-    if (lane < 5) w.ctrl[lane] = (w.tgt[lane] - w.qpos[lane]) * scale;
-    __syncwarp();
-    iters += physics_step(m, w, hv, adj, lane, f.xfrc_z, true);
-    nsa++; step_limit--;
-    nconmax = max(nconmax, w.ncon); flags |= w.overflow;
-    float d = lane < 5 ? fabsf(w.qpos[lane] - w.tgt[lane]) : 0.0f;
-    d = warp_max(d);
-    if (d < c.pos_tol) {
-      reached_target = true;
-      if (lane < 5) w.ctrl[lane] = 0;
-      __syncwarp();
-      break;
-    }
-    if (!(d == d)) break;  // non-finite state: bail out, handled below
-  }
-  // phase B: fall back to the pose at the start of the step (robot_env.py:112-128)
-  if (step_limit == 0) {
-    if (lane < 5) w.tgt[lane] = w.init_q[lane];
-    __syncwarp();
-    for (int i = 0; i < c.max_steps; i++) {
-      if (lane < 5) w.ctrl[lane] = (w.tgt[lane] - w.qpos[lane]) * scale;
-      __syncwarp();
-      iters += physics_step(m, w, hv, adj, lane, f.xfrc_z, true);
-      nsb++;
-      nconmax = max(nconmax, w.ncon); flags |= w.overflow;
-      float d = lane < 5 ? fabsf(w.qpos[lane] - w.tgt[lane]) : 0.0f;
-      d = warp_max(d);
-      if (d < c.pos_tol) {
-        reached_initial = true;
-        if (lane < 5) w.ctrl[lane] = 0;
-        __syncwarp();
-        break;
-      }
-      if (!(d == d)) break;
-    }
-  }
-  int fail = 0;
-  if (!reached_target && !reached_initial) { fail = 1; f.status = 1; }
-  // phase C: gripper (robot_env.py:134-168)
-  int object_grasped = 0;
-  if (reached_target) {
-    if (open_close > 0.f && !f.gripper_open) {
-      if (lane == 0) { w.ctrl[5] = 0.5f; w.ctrl[6] = 0.5f; }
-      __syncwarp();
-      for (int i = 0; i < c.max_steps; i++) {
-        float deltas = fmaxf(fabsf(0.4f - w.qpos[5]), fabsf(0.4f - w.qpos[6]));
-        iters += physics_step(m, w, hv, adj, lane, f.xfrc_z, true);
-        nsc++;
-        nconmax = max(nconmax, w.ncon); flags |= w.overflow;
-        if (deltas < c.grasp_tol || (w.qpos[5] > 0.4f && w.qpos[6] > 0.4f)) { f.gripper_open = 1; break; }
-        if (!(deltas == deltas)) break;
-      }
-      __syncwarp();
-      if (lane == 0) { w.ctrl[5] = 0; w.ctrl[6] = 0; }
-    } else if (open_close < 0.f && f.gripper_open) {
-      if (lane == 0) { w.ctrl[5] = -1.0f; w.ctrl[6] = -1.0f; }
-      __syncwarp();
-      for (int i = 0; i < c.max_steps; i++) {
-        float deltas = fmaxf(fabsf(-0.4f - w.qpos[5]), fabsf(-0.4f - w.qpos[6]));
-        object_grasped = check_grasp(m, w);
-        iters += physics_step(m, w, hv, adj, lane, f.xfrc_z, true);
-        nsc++;
-        nconmax = max(nconmax, w.ncon); flags |= w.overflow;
-        if (deltas < c.grasp_tol) { f.gripper_open = 0; break; }
-        if (object_grasped == 3) { f.gripper_open = 0; break; }
-        if (!(deltas == deltas)) break;
-      }
-      __syncwarp();
-      if (lane == 0) { w.ctrl[5] = 0; w.ctrl[6] = 0; }
-    }
-    __syncwarp();
-  }
-  StepCounters k;
-  k.nsa = nsa; k.nsb = nsb; k.nsc = nsc; k.iters = iters; k.nconmax = nconmax; k.flags = flags; k.fail = fail; k.object_grasped = object_grasped;
-  k.reached_target = reached_target; k.reached_initial = reached_initial; k.tq_rec = tq_rec;
-  env_finalize(m, c, w, f, init_obj, k, lane);
-}
-
 // ----------------------------------------------------------------------------------------------- kernels
 struct SimBuffers {
   float* state;         // [N][ST_STRIDE]
@@ -380,11 +284,6 @@ struct SimBuffers {
   const int* adj;
   const DevModel* model;
   int n;
-  int order_ncon;  // longest-first order: previous-step contact count from which an environment counts as contact-heavy
-  int order_spt;   // queue order behind the gripper-closing class: 1 = shortest predicted chain first (arm only, then opening), 0 = longest first
-  int long_per_block;  // slot_order 3: gripper-closing environments per block
-  int slot_order;  // lock-step kernel, first environment of a warp: 0 = consecutive queue entries per block, 1 = consecutive entries to consecutive blocks, 2 = balanced (static_slot, env_lockstep.cuh)
-  int ls_mask;  // lock-step kernel: which stage boundaries carry a block barrier (bit 0 smooth | 1 constraint | 2 solve | 3 euler+kin | 4 crb)
 };
 constexpr int DEBUG_STRIDE = 2048;
 constexpr int WARPS_PER_BLOCK = 4;
@@ -446,42 +345,6 @@ __device__ __forceinline__ int next_env(int* queue, int lane) {
   int e = 0;
   if (lane == 0) e = atomicAdd(queue, 1);
   return __shfl_sync(FULL, e, 0);
-}
-
-// RobotEnv.step for every environment (+ SB3 VecEnv auto-reset when cfg.auto_reset)
-__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 5) k_env_step(SimBuffers s, EnvCfg c, const float* __restrict__ actions, int adim) {
-  const DevModel& m = stage_model(s.model);
-  WS& w = my_ws();
-  const int lane = threadIdx.x & 31;
-  for (int env = next_env(s.queue, lane); env < s.n; env = next_env(s.queue, lane)) {
-    EnvFlags f;
-    float* st = s.state + (size_t)env * ST_STRIDE;
-    load_state(w, f, st, lane);
-    forward_position(m, w, s.hull, s.adj, lane);
-    env_step(m, c, w, f, s.hull, s.adj, actions + (size_t)env * adim, lane);
-    for (int k = lane; k < IN_STRIDE; k += 32) s.info[(size_t)env * IN_STRIDE + k] = w.out[k];
-    write_render_state(m, w, c.obs_cam, s.render_state + (size_t)env * RS_STRIDE, lane);
-    const int done = (int)w.out[IN_DONE];
-    if (lane == 0) {
-      s.reward[env] = w.out[IN_REWARD];
-      s.done[env] = (unsigned char)done;
-      s.achieved[2 * env] = w.out[IN_ACHIEVED]; s.achieved[2 * env + 1] = w.out[IN_ACHIEVED + 1];
-      s.desired[2 * env] = w.out[IN_DESIRED]; s.desired[2 * env + 1] = w.out[IN_DESIRED + 1];
-    }
-    if (done && c.auto_reset) {
-      // VecEnv semantics: the returned goals belong to the NEW episode (robot_env.py:71-72); the terminal ones stay in info
-      for (int k = lane; k < ST_STRIDE; k += 32) st[k] = s.reset_record[k];
-      __syncwarp();
-      if (lane == 0) {
-        s.achieved[2 * env] = s.reset_record[ST_STRIDE + IN_ACHIEVED]; s.achieved[2 * env + 1] = s.reset_record[ST_STRIDE + IN_ACHIEVED + 1];
-        s.desired[2 * env] = s.reset_record[ST_STRIDE + IN_DESIRED]; s.desired[2 * env + 1] = s.reset_record[ST_STRIDE + IN_DESIRED + 1];
-        if (c.reset_noise_xy != 0.f || c.reset_noise_yaw != 0.f) apply_reset_noise(s, m, c, env, st);
-      }
-    } else {
-      store_state(w, f, st, lane);
-    }
-    __syncwarp();
-  }
 }
 
 // RobotEnv.reset executed once (every environment starts from qpos0 — the reference has no reset randomisation):

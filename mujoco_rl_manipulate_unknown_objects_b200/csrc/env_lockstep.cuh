@@ -1,14 +1,13 @@
-// Lock-step variant of the fused agent-step kernel.
+// The fused agent-step kernel, in lock-step rounds.
 //
-// The sequential kernel (k_env_step in env_kernels.cuh) lets every warp run its own environment's state machine
-// freely.  Profiling showed it to be INSTRUCTION-FETCH bound: ~120 KB of hot code per substep, 20 warps per SM at
-// unrelated program counters, 58 % hit rate in the 32 KB SM instruction cache and half of all issue slots lost to
-// "no instruction" stalls (DESIGN.md §3.1).  Here all warps of a block walk the substep pipeline
-// TOGETHER — smooth forces | constraint rows | Newton solve | integrate + kinematics | CRB | collision — with a block
-// barrier between the stages, so the SM's instruction cache only ever holds one stage's code.  The per-environment
-// controller state machine (reference robot_env.py:77-241) becomes an explicit `tick` that runs between rounds and
-// decides, per warp, whether this round carries a physics substep; environments still come from the atomic queue, so
-// ragged trip counts only cost idle warps inside a round, never idle rounds.
+// One warp integrates one environment's substeps.  Warps that each run their own environment's controller freely are
+// INSTRUCTION-FETCH bound: ~120 KB of hot code per substep, 20 warps per SM at unrelated program counters, 58 % hit rate
+// in the 32 KB SM instruction cache and half of all issue slots lost to "no instruction" stalls (DESIGN.md §3.1).  Here
+// all warps of a block walk the substep pipeline TOGETHER — smooth forces | constraint rows | Newton solve | integrate +
+// kinematics | CRB | collision — with block barriers between the stages, so the SM's instruction cache holds one stage's
+// code at a time.  The per-environment controller state machine (reference robot_env.py:77-241) is an explicit `tick`
+// that runs between rounds and decides, per warp, whether this round carries a physics substep; environments come from
+// an atomic queue, so ragged trip counts only cost idle warps inside a round, never idle rounds.
 //
 // Around that core: k_order_count / k_order_envs queue the environments longest chain first and group them by contact count;
 // a block whose physics work is exhausted becomes an observation builder (render_phase) for the environments that have
@@ -164,7 +163,7 @@ __device__ __noinline__ bool env_tick(const DevModel& m, const EnvCfg& c, WS& w,
   }
 }
 
-// results of a finished agent step -> HBM (+ SB3 auto-reset); same record layout as the sequential kernel
+// results of a finished agent step -> HBM (+ SB3 auto-reset)
 __device__ __noinline__ void env_writeback(const DevModel& m, const EnvCfg& c, const SimBuffers& s, WS& w, EnvCtl& t, int lane) {
   const int env = t.env;
   float* st = s.state + (size_t)env * ST_STRIDE;
@@ -202,20 +201,18 @@ __device__ __noinline__ void env_writeback(const DevModel& m, const EnvCfg& c, c
 // A second key groups environments of similar cost per substep: a lock-step round lasts as long as its slowest warp in each
 // stage, and the expensive stage (narrowphase: full MPR runs) is expensive exactly for environments whose gripper touches
 // something.  The contact count of the previous agent step is the predictor.  Classes are queued chain-length class first
-// (close the gripper | open it | arm only), most contacts first inside each; k_order_count sizes them, k_order_envs places.
+// (close the gripper | arm only | open it), most contacts first inside each; k_order_count sizes them, k_order_envs places.
 constexpr int ORDER_BUCKETS = 8;  // contact-count buckets per chain-length class; 3 x 8 classes; counters live in SimBuffers::queue[16..39] (sizes) and [40..63] (cursors)
 __device__ __forceinline__ int order_class(const SimBuffers& s, const float* __restrict__ actions, int adim, int env) {
   const float oc = actions[(size_t)env * adim + adim - 1];
   const bool open = s.state[(size_t)env * ST_STRIDE + ST_GRIPPER_OPEN] != 0.0f;
-  // chain-length class: closing the gripper (~175 extra substeps) | opening it (~75) | arm only
-  // order_spt: behind the closing class, shortest first (arm only, then opening): every environment has then STARTED by round
-  // ~150 instead of ~300, which bounds the damage of the chains nobody can predict (0.1 % of the environments run into the
-  // 400-substep arm time-out, tools/chain_predict.py: a 500-800-substep chain that starts late ends late)
+  // chain-length class: closing the gripper (~175 extra substeps) first, then the rest shortest first (arm only, then opening
+  // it, ~75): every environment has then STARTED by round ~150 instead of ~300, which bounds the damage of the chains nobody
+  // can predict (0.1 % of the environments run into the 400-substep arm time-out, tools/chain_predict.py: a 500-800-substep
+  // chain that starts late ends late)
   const bool arm_only = !((oc < 0.f && open) || (oc > 0.f && !open));
-  const int len = (oc < 0.f && open) ? 0 : (arm_only ? (s.order_spt ? 1 : 2) : (s.order_spt ? 2 : 1));
+  const int len = (oc < 0.f && open) ? 0 : (arm_only ? 1 : 2);
   const int ncon = (int)s.info[(size_t)env * IN_STRIDE + IN_NCON_MAX];
-  if (s.order_ncon > 0) return (arm_only ? ORDER_BUCKETS : 0) + (ncon >= s.order_ncon ? 0 : 1);  // two-level variant (sweeps)
-  if (s.order_ncon < 0) return (arm_only ? ORDER_BUCKETS : 0) + (ORDER_BUCKETS - 1 - min(max(ncon, 0), ORDER_BUCKETS - 1));  // long | short only
   return len * ORDER_BUCKETS + (ORDER_BUCKETS - 1 - min(max(ncon, 0), ORDER_BUCKETS - 1));  // most contacts first
 }
 __global__ void k_order_count(SimBuffers s, const float* __restrict__ actions, int adim) {
@@ -233,52 +230,10 @@ __global__ void k_order_envs(SimBuffers s, const float* __restrict__ actions, in
   s.done_list[env] = -1;
 }
 
-// First environment of a warp (static slot in the longest-first queue).
-//   slot_order 0: a block's warps take consecutive queue entries.  The first blocks then hold eight gripper-closing environments each
-//                 (three quarters of which run into the 400-substep timeout): ~485 full rounds, while the average block has ~330
-//                 rounds of work and finishes a third earlier (profiles/r2h_stage_timing_step150.log).
-//   slot_order 1: consecutive entries go to consecutive blocks (long chains spread thin, but every block mixes contact-heavy and
-//                 contact-free environments, and a lock-step round costs what its slowest warp costs).
-//   slot_order 2: balanced.  The gripper-closing class (chain-length class 0) is dealt out in equal runs, n0 / grid per block, the
-//                 rest of the static entries fill the block's other warps, also as one run: every block carries the same share of
-//                 long chains and both of its runs are contiguous in the contact-count order (homogeneous rounds).  Once the short
-//                 environments and the shared queue are exhausted, a block is left with its few long chains, which then run at
-//                 the latency of a nearly empty SM instead of that of a full one.
-//   slot_order 3: the closing class `long_per_block` per block from block 0 on; those blocks' remaining warps and all other
-//                 blocks take the short environments.
-__device__ __forceinline__ int static_slot(const SimBuffers& s, int nstatic) {
-  const int W = blockDim.x >> 5, G = gridDim.x, b = blockIdx.x, w = threadIdx.x >> 5;
-  if (s.slot_order == 1) return w * G + b;
-  if (s.slot_order >= 2 && s.order_ncon == 0) {
-    int n0 = 0;
-    for (int k = 0; k < ORDER_BUCKETS; k++) n0 += s.queue[16 + k];
-    if (n0 < min(nstatic, s.n)) {
-      if (s.slot_order == 2) {
-        const int Lb = n0 / G, r = n0 - Lb * G;       // blocks < r carry Lb + 1 long chains, the others Lb
-        const int myL = Lb + (b < r ? 1 : 0), long_start = b * Lb + min(b, r);
-        return w < myL ? long_start + w : n0 + (b * W - long_start) + (w - myL);
-      }
-      // slot_order = 3: the closing class L per block (s.long_per_block), the block's other warps take the short environments
-      const int L = min(max(s.long_per_block, 1), W);
-      if ((n0 + L - 1) / L <= G) {
-        const int long_start = min(b * L, n0), myL = min(L, n0 - long_start);
-        return w < myL ? long_start + w : n0 + (b * W - long_start) + (w - myL);
-      }
-    }
-  }
-  return b * W + w;
-}
-
 // Launch bounds (320 threads, 2 blocks per SM) cap the kernel at 96 registers.  Measured in the steady state of the bench
 // workload (profiles/r2e_warps_regs_ab.log, r2f_regs.log): 113-120 registers (bounds 512, 1) 18.2 M substeps/s, 96 registers
 // 19.1 M, 80 registers 18.4 M, 72 registers 17.4 M, 64 registers 17.2 M; the stack frame grows by only 40 bytes at 96.
-#ifndef GRS_LS_THREADS
-#define GRS_LS_THREADS 320
-#endif
-#ifndef GRS_LS_MINBLOCKS
-#define GRS_LS_MINBLOCKS 2
-#endif
-constexpr int LS_MAX_THREADS = GRS_LS_THREADS;
+constexpr int LS_MAX_THREADS = 320, LS_MIN_BLOCKS = 2;
 
 // TIMING = true: per-stage clock64 bookkeeping (sum over warps vs. per-round block maximum) into s.debug — a development
 // aid behind GRS_STEP_TIMING=1 that quantifies what the block barriers cost; the production instantiation carries none of it.
@@ -312,11 +267,43 @@ struct AsyncArgs {
   int* waited;  // [N] 1: pending and already queued by an earlier launch that stopped before fetching it
 };
 
+// park: the controls of the next substep are set; store the state and the controller instead of integrating it
+__device__ __forceinline__ void park_env(const SimBuffers& s, const AsyncArgs& aa, const WS& w, const EnvCtl& t, int lane) {
+  const int env = t.env;
+  store_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
+  float* pk = aa.park + (size_t)env * PK_STRIDE;
+  if (lane < 5) { pk[PK_TQ_REC + lane] = t.k.tq_rec; pk[PK_TGT + lane] = w.tgt[lane]; pk[PK_INIT_Q + lane] = w.init_q[lane]; }
+  if (lane == 0) {
+    pk[PK_STAGE] = (float)t.stage; pk[PK_I] = (float)t.i; pk[PK_STEP_LIMIT] = (float)t.step_limit;
+    pk[PK_OPEN_CLOSE] = t.open_close; pk[PK_DELTAS] = t.deltas;
+    for (int k = 0; k < 3; k++) pk[PK_INIT_OBJ + k] = t.init_obj[k];
+    pk[PK_NSA] = (float)t.k.nsa; pk[PK_NSB] = (float)t.k.nsb; pk[PK_NSC] = (float)t.k.nsc; pk[PK_ITERS] = (float)t.k.iters;
+    pk[PK_NCONMAX] = (float)t.k.nconmax; pk[PK_FLAGS] = (float)t.k.flags; pk[PK_FAIL] = (float)t.k.fail; pk[PK_GRASPED] = (float)t.k.object_grasped;
+    pk[PK_REACHED_TARGET] = t.k.reached_target ? 1.0f : 0.0f; pk[PK_REACHED_INITIAL] = t.k.reached_initial ? 1.0f : 0.0f;
+    aa.astate[env] = A_PARKED;
+  }
+  __syncwarp();
+}
+// resume: restore the controller of a parked environment whose state row is loaded, so that it runs the substep it was
+// parked before without ticking again
+__device__ __forceinline__ void resume_env(const AsyncArgs& aa, WS& w, EnvCtl& t, int lane) {
+  const float* pk = aa.park + (size_t)t.env * PK_STRIDE;
+  t.stage = (int)pk[PK_STAGE]; t.i = (int)pk[PK_I]; t.step_limit = (int)pk[PK_STEP_LIMIT];
+  t.open_close = pk[PK_OPEN_CLOSE]; t.deltas = pk[PK_DELTAS];
+  for (int k = 0; k < 3; k++) t.init_obj[k] = pk[PK_INIT_OBJ + k];
+  t.k.nsa = (int)pk[PK_NSA]; t.k.nsb = (int)pk[PK_NSB]; t.k.nsc = (int)pk[PK_NSC]; t.k.iters = (int)pk[PK_ITERS];
+  t.k.nconmax = (int)pk[PK_NCONMAX]; t.k.flags = (int)pk[PK_FLAGS]; t.k.fail = (int)pk[PK_FAIL]; t.k.object_grasped = (int)pk[PK_GRASPED];
+  t.k.reached_target = pk[PK_REACHED_TARGET] != 0.0f; t.k.reached_initial = pk[PK_REACHED_INITIAL] != 0.0f;
+  t.k.tq_rec = lane < 5 ? pk[PK_TQ_REC + lane] : 0.0f;
+  if (lane < 5) { w.tgt[lane] = pk[PK_TGT + lane]; w.init_q[lane] = pk[PK_INIT_Q + lane]; }
+  __syncwarp();
+}
+
 // FUSED = true: a block whose physics work is exhausted goes on to build observations (render_phase) instead of exiting, so
 // the rasteriser fills the SMs that idle while the longest substep chains finish.  Needs blockDim.x == RTHREADS.
 // ASYNC = true: the asynchronous step above (not FUSED: the observation phase would wait for environments that get parked).
 template <bool TIMING, bool FUSED, bool ASYNC = false>
-__global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_ls(SimBuffers s, EnvCfg c, const float* __restrict__ actions, int adim, RenderScene sc, ObsArgs oa,
+__global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(SimBuffers s, EnvCfg c, const float* __restrict__ actions, int adim, RenderScene sc, ObsArgs oa,
                                                                                   AsyncArgs aa) {
   static_assert(!(ASYNC && (FUSED || TIMING)), "the asynchronous step has its own instantiation");
   unsigned smid = 0;
@@ -374,65 +361,45 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
   for (;;) {
     // ---- controller round: finish / fetch / decide (per warp, no block-wide dependency)
     LS_T0();
-    bool dyn = false, pos = false;
+    bool dyn = false, pos = false, stop = false;
     if constexpr (ASYNC) {
       // stop rule: once `need` environments have finished in this launch (s.queue[3] counts them), nothing new is fetched and
       // every environment still mid-step is parked at its next substep boundary
-      const bool stop = *reinterpret_cast<volatile int*>(s.queue + 3) >= __ldg(aa.ctl + AC_NEED);
+      stop = *reinterpret_cast<volatile int*>(s.queue + 3) >= __ldg(aa.ctl + AC_NEED);
       if (t.stage == S_RESUME) {
         if (stop) {
           t.stage = S_IDLE;  // dropped before it moved: its state row and park record still describe it, it stays parked
         } else {
-          // restore the controller and run the substep it was parked before, without ticking again
-          const float* pk = aa.park + (size_t)t.env * PK_STRIDE;
-          t.stage = (int)pk[PK_STAGE]; t.i = (int)pk[PK_I]; t.step_limit = (int)pk[PK_STEP_LIMIT];
-          t.open_close = pk[PK_OPEN_CLOSE]; t.deltas = pk[PK_DELTAS];
-          for (int k = 0; k < 3; k++) t.init_obj[k] = pk[PK_INIT_OBJ + k];
-          t.k.nsa = (int)pk[PK_NSA]; t.k.nsb = (int)pk[PK_NSB]; t.k.nsc = (int)pk[PK_NSC]; t.k.iters = (int)pk[PK_ITERS];
-          t.k.nconmax = (int)pk[PK_NCONMAX]; t.k.flags = (int)pk[PK_FLAGS]; t.k.fail = (int)pk[PK_FAIL]; t.k.object_grasped = (int)pk[PK_GRASPED];
-          t.k.reached_target = pk[PK_REACHED_TARGET] != 0.0f; t.k.reached_initial = pk[PK_REACHED_INITIAL] != 0.0f;
-          t.k.tq_rec = lane < 5 ? pk[PK_TQ_REC + lane] : 0.0f;
-          if (lane < 5) { w.tgt[lane] = pk[PK_TGT + lane]; w.init_q[lane] = pk[PK_INIT_Q + lane]; }
-          __syncwarp();
+          resume_env(aa, w, t, lane);
           dyn = true;
         }
       } else if (t.stage == S_LOADED && stop) {
         t.stage = S_IDLE;  // loaded but not begun: it stays pending
       }
-      if (t.stage == S_LOADED) t.stage = S_BEGIN;
-      if (t.stage != S_IDLE && !dyn) {
-        dyn = env_tick(m, c, w, t, actions + (size_t)t.env * adim, iters, lane);
-        if (!dyn) {
-          env_writeback(m, c, s, w, t, lane);
-        } else if (stop) {
-          // park: the controls of the next substep are set; store the state and the controller instead of integrating it
-          const int env = t.env;
-          store_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
-          float* pk = aa.park + (size_t)env * PK_STRIDE;
-          if (lane < 5) { pk[PK_TQ_REC + lane] = t.k.tq_rec; pk[PK_TGT + lane] = w.tgt[lane]; pk[PK_INIT_Q + lane] = w.init_q[lane]; }
-          if (lane == 0) {
-            pk[PK_STAGE] = (float)t.stage; pk[PK_I] = (float)t.i; pk[PK_STEP_LIMIT] = (float)t.step_limit;
-            pk[PK_OPEN_CLOSE] = t.open_close; pk[PK_DELTAS] = t.deltas;
-            for (int k = 0; k < 3; k++) pk[PK_INIT_OBJ + k] = t.init_obj[k];
-            pk[PK_NSA] = (float)t.k.nsa; pk[PK_NSB] = (float)t.k.nsb; pk[PK_NSC] = (float)t.k.nsc; pk[PK_ITERS] = (float)t.k.iters;
-            pk[PK_NCONMAX] = (float)t.k.nconmax; pk[PK_FLAGS] = (float)t.k.flags; pk[PK_FAIL] = (float)t.k.fail; pk[PK_GRASPED] = (float)t.k.object_grasped;
-            pk[PK_REACHED_TARGET] = t.k.reached_target ? 1.0f : 0.0f; pk[PK_REACHED_INITIAL] = t.k.reached_initial ? 1.0f : 0.0f;
-            aa.astate[env] = A_PARKED;
-          }
-          __syncwarp();
-          t.stage = S_IDLE;
-          dyn = false;
-        }
+    }
+    if (t.stage == S_LOADED) t.stage = S_BEGIN;
+    if (t.stage != S_IDLE && !dyn) {
+      dyn = env_tick(m, c, w, t, actions + (size_t)t.env * adim, iters, lane);
+      if (!dyn) {
+        env_writeback(m, c, s, w, t, lane);
+      } else if (stop) {
+        park_env(s, aa, w, t, lane);
+        t.stage = S_IDLE;
+        dyn = false;
       }
-      if (t.stage == S_IDLE && !exhausted && !stop) {
-        const int nstatic = gridDim.x * (blockDim.x >> 5);
-        int slot = first ? static_slot(s, nstatic) : nstatic + next_env(s.queue, lane);
-        first = false;
-        if (slot < __ldg(aa.ctl + AC_NQUEUE)) {
-          const int env = __ldg(s.order + slot);
-          t.env = env;
-          load_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
-          t.stage = S_LOADED;
+    }
+    if (t.stage == S_IDLE && !exhausted && !stop) {
+      // first environment of a warp: static slot, so that a block starts with consecutive queue entries (environments of the
+      // same class, see k_order_envs); later ones come from the shared counter, which starts behind the static slots
+      const int nstatic = gridDim.x * (blockDim.x >> 5);
+      const int slot = first ? blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5) : nstatic + next_env(s.queue, lane);
+      first = false;
+      if (slot < (ASYNC ? __ldg(aa.ctl + AC_NQUEUE) : s.n)) {
+        const int env = __ldg(s.order + slot);
+        t.env = env;
+        load_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
+        t.stage = S_LOADED;
+        if constexpr (ASYNC) {
           if (__ldg(aa.astate + env) == A_PARKED) {
             // the position stage below has to see the qpos the synchronous step's position stage saw (kinematics
             // renormalises the free joint's quaternion in place, and renormalising twice can move its last bit)
@@ -440,33 +407,11 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
             __syncwarp();
             t.stage = S_RESUME;
           }
-          pos = true;
-        } else {
-          exhausted = true;
         }
-      }
-    } else {
-    if (t.stage == S_LOADED) t.stage = S_BEGIN;
-    if (t.stage != S_IDLE) {
-      dyn = env_tick(m, c, w, t, actions + (size_t)t.env * adim, iters, lane);
-      if (!dyn) env_writeback(m, c, s, w, t, lane);
-    }
-    if (t.stage == S_IDLE && !exhausted) {
-      // first environment of a warp: static slot, so that a block starts with consecutive queue entries (environments of the
-      // same class, see k_order_envs); later ones come from the shared counter, which starts behind the static slots
-      const int nstatic = gridDim.x * (blockDim.x >> 5);
-      int slot = first ? static_slot(s, nstatic) : nstatic + next_env(s.queue, lane);
-      first = false;
-      if (slot < s.n) {
-        const int env = __ldg(s.order + slot);
-        t.env = env;
-        load_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
-        t.stage = S_LOADED;
         pos = true;  // position stage of the loaded state (no dynamics this round)
       } else {
         exhausted = true;
       }
-    }
     }
     pos = pos || dyn;
     LS_T1(0);
@@ -486,16 +431,16 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
     LS_T0();
     if (dyn) smooth_forces(m, w, lane, true, t.f.xfrc_z);
     LS_T1(1);
-    if (s.ls_mask & 1) __syncthreads();
+    // block barriers after the constraint rows, the Newton solve and CRB only (profiles/r2m_sweep.log: none 5 % slower)
     LS_T0();
     if (dyn) make_constraint(m, w, lane);
     LS_T1(2);
-    if (s.ls_mask & 2) __syncthreads();
+    __syncthreads();
     iters = 0;
     LS_T0();
     if (dyn) iters = solve_newton(m, w, lane, m.iterations);
     LS_T1(3);
-    if (s.ls_mask & 4) __syncthreads();
+    __syncthreads();
     LS_T0();
     if (dyn) euler_integrate(m, w, lane);
     if constexpr (ASYNC) {
@@ -507,11 +452,10 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, GRS_LS_MINBLOCKS) k_env_step_l
     }
     if (pos) kinematics(m, w, lane);
     LS_T1(4);
-    if (s.ls_mask & 8) __syncthreads();
     LS_T0();
     if (pos) com_pos_crb(m, w, lane);
     LS_T1(5);
-    if (s.ls_mask & 16) __syncthreads();
+    __syncthreads();
     LS_T0();
     if (pos) collision(m, w, hull, s.adj, lane);
     LS_T1(6);

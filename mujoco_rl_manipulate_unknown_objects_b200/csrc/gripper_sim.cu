@@ -77,7 +77,7 @@ struct grs_sim {
   long ms_cnt = 0;
   int grid = 0;
   size_t smem = 0;
-  // lock-step step kernel geometry (GRS_STEP_WARPS warps per block; 0 selects the sequential kernel)
+  // step kernel geometry (GRS_STEP_WARPS warps per block)
   int ls_warps = 8, ls_grid = 0;
   bool ls_timing = false;
   bool fused_render = false;  // observation phase inside the step kernel (env_lockstep.cuh : render_phase)
@@ -178,12 +178,6 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     b.reset_obj = dalloc<float>(s.get(), N * 12);
     b.tstamp = dalloc<unsigned long long>(s.get(), 4);
     { const unsigned long long init[4] = {~0ull, 0, 0, 0}; CU(cudaMemcpy(b.tstamp, init, sizeof init, cudaMemcpyHostToDevice)); }
-    b.ls_mask = 22;
-    b.order_ncon = getenv("GRS_ORDER_NCON") ? atoi(getenv("GRS_ORDER_NCON")) : 0;
-    if (const char* e = getenv("GRS_LS_MASK")) b.ls_mask = atoi(e);
-    b.slot_order = getenv("GRS_SLOT_ORDER") ? atoi(getenv("GRS_SLOT_ORDER")) : 0;
-    b.long_per_block = getenv("GRS_LONG_PER_BLOCK") ? atoi(getenv("GRS_LONG_PER_BLOCK")) : 6;
-    b.order_spt = getenv("GRS_ORDER_SPT") ? atoi(getenv("GRS_ORDER_SPT")) : 1;
     b.order = dalloc<int>(s.get(), N);
     const size_t obs_bytes = (size_t)s->C * s->H * s->W;
     s->d_obs = dalloc<unsigned char>(s.get(), N * obs_bytes);
@@ -210,42 +204,41 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     if (!(cfg.reset_noise_xy >= 0.f) || !(cfg.reset_noise_yaw >= 0.f)) throw std::runtime_error("reset_noise_xy / reset_noise_yaw must be >= 0");
     e.reset_noise_xy = cfg.reset_noise_xy; e.reset_noise_yaw = cfg.reset_noise_yaw; e.seed = cfg.seed;
     e.pos_tol = cfg.pos_tolerance; e.grasp_tol = cfg.grasp_tolerance; e.max_trans = cfg.max_translation; e.max_rot = cfg.max_rotation;
-    // launch geometry: persistent blocks, as many as fit (one WS per warp in shared memory)
+    // launch geometry of the per-environment kernels (k_substep, k_contacts, k_debug_step, k_camera_state): persistent blocks,
+    // as many as fit (one WS per warp in shared memory)
     s->smem = smem_bytes();
-    raise_dyn_smem((const void*)k_env_step, s->smem, device);
     raise_dyn_smem((const void*)k_substep, s->smem, device);
     raise_dyn_smem((const void*)k_contacts, s->smem, device);
     raise_dyn_smem((const void*)k_debug_step, s->smem, device);
     raise_dyn_smem((const void*)k_make_reset_record, s->smem, device);
     int per_sm = 0, nsm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_env_step, WARPS_PER_BLOCK * 32, s->smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_substep, WARPS_PER_BLOCK * 32, s->smem));
     CU(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    if (per_sm < 1) throw std::runtime_error("step kernel does not fit on this device");
+    if (per_sm < 1) throw std::runtime_error("substep kernel does not fit on this device");
     int want = (num_envs + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
     s->grid = std::min(want, per_sm * nsm);
-    if (const char* e = getenv("GRS_STEP_WARPS")) s->ls_warps = std::max(0, std::min(LS_MAX_THREADS / 32, atoi(e)));
-    if (s->ls_warps > 0) {
-      s->ls_smem = (sizeof(DevModel) + 15) / 16 * 16 + (size_t)s->ls_warps * sizeof(WS);
-      {
-        // hull vertices in shared memory when two blocks per SM still fit (227 KB per block, 228 KB per SM, 1 KB reserved each)
-        const size_t with_hull = s->ls_smem + (size_t)s->b.hull_count * sizeof(float4);
-        const bool want = getenv("GRS_HULL_SMEM") ? atoi(getenv("GRS_HULL_SMEM")) != 0 : true;
-        if (want && 2 * (with_hull + 1024) <= 228 * 1024) { s->ls_smem = with_hull; s->b.hull_smem = 1; }
-      }
-      s->ls_timing = getenv("GRS_STEP_TIMING") != nullptr;
-      // the observation phase needs RTHREADS-wide blocks and the observation tile in the block's shared memory
-      s->fused_render = !s->ls_timing && s->ls_warps * 32 == RTHREADS && s->ls_smem >= render_phase_smem_bytes() && cfg.width <= TILE && cfg.height <= TILE;
-      if (const char* e = getenv("GRS_FUSED_RENDER")) s->fused_render = s->fused_render && atoi(e) != 0;
-      raise_dyn_smem((const void*)k_env_step_ls<false, false>, s->ls_smem, device);
-      raise_dyn_smem((const void*)k_env_step_ls<false, true>, s->ls_smem, device);
-      raise_dyn_smem((const void*)k_env_step_ls<true, false>, s->ls_smem, device);
-      raise_dyn_smem((const void*)k_env_step_ls<false, false, true>, s->ls_smem, device);
-      int ls_per_sm = 0;
-      if (s->fused_render) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, true>, s->ls_warps * 32, s->ls_smem));
-      else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, false>, s->ls_warps * 32, s->ls_smem));
-      if (ls_per_sm < 1) throw std::runtime_error("lock-step step kernel does not fit on this device");
-      s->ls_grid = std::min((num_envs + s->ls_warps - 1) / s->ls_warps, ls_per_sm * nsm);
+    // step kernel geometry
+    if (const char* e = getenv("GRS_STEP_WARPS")) s->ls_warps = std::max(1, std::min(LS_MAX_THREADS / 32, atoi(e)));
+    s->ls_smem = (sizeof(DevModel) + 15) / 16 * 16 + (size_t)s->ls_warps * sizeof(WS);
+    {
+      // hull vertices in shared memory when two blocks per SM still fit (227 KB per block, 228 KB per SM, 1 KB reserved each)
+      const size_t with_hull = s->ls_smem + (size_t)s->b.hull_count * sizeof(float4);
+      const bool want = getenv("GRS_HULL_SMEM") ? atoi(getenv("GRS_HULL_SMEM")) != 0 : true;
+      if (want && 2 * (with_hull + 1024) <= 228 * 1024) { s->ls_smem = with_hull; s->b.hull_smem = 1; }
     }
+    s->ls_timing = getenv("GRS_STEP_TIMING") != nullptr;
+    // the observation phase needs RTHREADS-wide blocks and the observation tile in the block's shared memory
+    s->fused_render = !s->ls_timing && s->ls_warps * 32 == RTHREADS && s->ls_smem >= render_phase_smem_bytes() && cfg.width <= TILE && cfg.height <= TILE;
+    if (const char* e = getenv("GRS_FUSED_RENDER")) s->fused_render = s->fused_render && atoi(e) != 0;
+    raise_dyn_smem((const void*)k_env_step_ls<false, false>, s->ls_smem, device);
+    raise_dyn_smem((const void*)k_env_step_ls<false, true>, s->ls_smem, device);
+    raise_dyn_smem((const void*)k_env_step_ls<true, false>, s->ls_smem, device);
+    raise_dyn_smem((const void*)k_env_step_ls<false, false, true>, s->ls_smem, device);
+    int ls_per_sm = 0;
+    if (s->fused_render) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, true>, s->ls_warps * 32, s->ls_smem));
+    else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, false>, s->ls_warps * 32, s->ls_smem));
+    if (ls_per_sm < 1) throw std::runtime_error("step kernel does not fit on this device");
+    s->ls_grid = std::min((num_envs + s->ls_warps - 1) / s->ls_warps, ls_per_sm * nsm);
     for (int i = 0; i < grs_sim::NEV; i++) { CU(cudaEventCreate(&s->ev0[i])); CU(cudaEventCreate(&s->ev1[i])); }
     render_scene_upload(s->hm, s->scene, s->owned);
     // the reset record and the observation of a freshly reset environment (identical for every env and every episode)
@@ -352,20 +345,16 @@ extern "C" int32_t grs_step(grs_sim* s, const float* actions_dev, void* stream) 
     launch_queue_kernel_prep(s, st);
     if (s->ev_n == grs_sim::NEV) harvest_events(s);
     CU(cudaEventRecord(s->ev0[s->ev_n], st));
-    if (s->ls_warps > 0) {
-      k_order_count<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
-      k_order_envs<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
-      s->launches += 2;
-    }
-    const bool fused = s->ls_warps > 0 && s->fused_render;
-    if (fused) k_env_step_ls<false, true><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
-    else if (s->ls_warps > 0 && s->ls_timing) k_env_step_ls<true, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
-    else if (s->ls_warps > 0) k_env_step_ls<false, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
-    else k_env_step<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, st>>>(s->b, s->ecfg, actions_dev, s->adim);
+    k_order_count<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
+    k_order_envs<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
+    s->launches += 2;
+    if (s->fused_render) k_env_step_ls<false, true><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
+    else if (s->ls_timing) k_env_step_ls<true, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
+    else k_env_step_ls<false, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
     CU(cudaGetLastError());
     CU(cudaEventRecord(s->ev1[s->ev_n], st));
     s->ev_n++;
-    if (!fused) { launch_render_obs(s->scene, s->obs_args, s->b.render_state, s->b.info, s->b.done, s->b.reward, s->n, st); s->launches++; }
+    if (!s->fused_render) { launch_render_obs(s->scene, s->obs_args, s->b.render_state, s->b.info, s->b.done, s->b.reward, s->n, st); s->launches++; }
     s->launches += 1;
     return 0;
   } catch (const std::exception& e) { return fail(e.what()); }
@@ -702,7 +691,7 @@ extern "C" float grs_step_kernel_ms(grs_sim* s, int32_t reset_counters) {
   cudaSetDevice(s->device);
   harvest_events(s);
   float avg = s->ms_cnt ? (float)(s->ms_sum / s->ms_cnt) : 0.0f;
-  if (s->fused_render && s->ls_warps > 0) {
+  if (s->fused_render) {
     // fused kernel: the physics phase is timed on the device (globaltimer: first block start -> last block leaving the
     // substep loop, accumulated by the last block of every launch); the events above cover physics + observation phases
     unsigned long long t[4] = {0, 0, 0, 0};
@@ -726,7 +715,6 @@ extern "C" int32_t grs_async_begin(grs_sim* s, int32_t batch, void* stream) {
   if (s->async_on) return fail("grs_async_begin: asynchronous mode is already on (grs_async_end first)");
   if (batch <= 0 || batch > s->n) return fail("grs_async_begin: batch must be within 1..num_envs");
   if (!s->cfg.auto_reset) return fail("grs_async_begin: the asynchronous step needs auto_reset=1");
-  if (s->ls_warps <= 0) return fail("grs_async_begin: the asynchronous step needs the lock-step step kernel (GRS_STEP_WARPS > 0)");
   try {
     CU(cudaSetDevice(s->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;

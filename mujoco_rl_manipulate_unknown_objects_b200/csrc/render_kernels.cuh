@@ -539,7 +539,8 @@ __device__ __forceinline__ void render_obs_env(const RenderScene& sc, const ObsA
 }
 
 // Standalone observation kernel: one block per environment.  info: per-env info rows; done: per-env done flags (NULL for
-// the reset image).  Used for the reset image, the sequential step kernel and GRS_FUSED_RENDER=0.
+// the reset image).  Used for the reset image and whenever the step kernel runs without its observation phase
+// (GRS_FUSED_RENDER=0, GRS_STEP_TIMING, other block widths than RTHREADS).
 __global__ void __launch_bounds__(RTHREADS) k_render_obs(RenderScene sc, ObsArgs o, const float* __restrict__ render_state, const float* __restrict__ info, int info_stride,
                                                         const unsigned char* __restrict__ done, float* __restrict__ reward) {
   extern __shared__ __align__(16) unsigned char rsm[];

@@ -45,12 +45,11 @@ def test_results_do_not_depend_on_scheduling(n, scene):
     import torch
     steps = 4 if n <= 8192 else 3
     base = _run(n, scene, steps)
-    # 0 = sequential kernel; GRS_GAP_SKIP=0 evaluates every cached separating axis instead of skipping those whose separation
-    # budget is still positive (sim_kernels.cuh : collision) — the skip is exact, so not a bit may change; GRS_SLOT_ORDER=1
-    # hands the first queue entries to different blocks
-    variants = (dict(GRS_FUSED_RENDER="0"), dict(GRS_STEP_WARPS="10", GRS_HULL_SMEM="0"), dict(GRS_STEP_WARPS="0"), dict(GRS_GAP_SKIP="0"),
-                dict(GRS_SLOT_ORDER="1", GRS_NO_HOST_MIRROR="1"))
-    for env in (variants if n <= 8192 else variants[2:4]):
+    # 10 warps per block hands the queue entries to other warps and blocks; GRS_GAP_SKIP=0 evaluates every cached separating
+    # axis instead of skipping those whose separation budget is still positive (sim_kernels.cuh : collision) — the skip is
+    # exact, so not a bit may change
+    variants = (dict(GRS_FUSED_RENDER="0"), dict(GRS_STEP_WARPS="10", GRS_HULL_SMEM="0"), dict(GRS_GAP_SKIP="0", GRS_NO_HOST_MIRROR="1"))
+    for env in (variants if n <= 8192 else variants[1:]):
         other = _run(n, scene, steps, env)
         for t in range(steps):
             for k in base[t]:

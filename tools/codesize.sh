@@ -1,7 +1,7 @@
 #!/bin/bash
 # per-device-function SASS size of the fused step kernel (instruction-cache budget, see DESIGN.md)
 cd "$(dirname "$0")/.."
-cuobjdump -elf mujoco_rl_manipulate_unknown_objects_b200/libgripper_sim_b200.so | grep -E "^\s+0x[0-9a-f]+\s+0x[0-9a-f]+\s+0x[0-9a-f]+.*${1:-k_env_step}" \
+cuobjdump -elf mujoco_rl_manipulate_unknown_objects_b200/libgripper_sim_b200.so | grep -E "^\s+0x[0-9a-f]+\s+0x[0-9a-f]+\s+0x[0-9a-f]+.*${1:-k_env_step_ls}" \
  | python3 -c "
 import sys,re
 tot=0
