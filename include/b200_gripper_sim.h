@@ -224,7 +224,13 @@ GRS_API int32_t grl_adam_step(float* params_dev, const float* grads_dev, float* 
  * compute_reward call per relabelled row) under SAC.train (train_agent.py:61-88).  Errors are reported through grl_last_error().
  *
  * One ring of capacity + 1 slots per environment, slot-major [S][N]; a slot holds obs u8[C][H][W], next_obs u8[C][H][W],
- * action f32[A], reward f32, done u8 and the step's info row f32[GRS_INFO_STRIDE].  All environments add in lock-step.
+ * action f32[A], reward f32, done u8 and the step's info row f32[GRS_INFO_STRIDE].  Transition t of environment n lives in slot t % S.
+ *
+ * A buffer has one of two write modes, fixed by its first begin call; the calls of the other mode then fail.
+ *   lock-step (grl_replay_begin / grl_replay_add): all environments add in every call and share one host-side count.
+ *   indexed (grl_replay_begin_indexed / grl_replay_add_indexed): for an asynchronous pool (grs_async_*), where environments
+ *     advance at different rates.  Each environment has its own count on the device ("added"); the calls never synchronise.
+ *     Bad ids and an empty sample set a sticky device error that grl_replay_status reports and clears.
  *
  * grl_replay_create: C*H*W must be a multiple of 16.  her_reward: the simulator's her_buffer (the reward carries
  *   exp(-|dg - ag|), recomputed for relabelled goals).  seed feeds the sampling hash.  NULL on bad sizes or no CUDA device.
@@ -232,9 +238,19 @@ GRS_API int32_t grl_adam_step(float* params_dev, const float* grads_dev, float* 
  *   before the first add); closes every open episode at its newest stored transition without marking it done.
  * grl_replay_add: one vectorised step, read from the simulator's buffers after grs_step: next_obs = terminal_obs where done,
  *   else obs; then obs (the reset observation where done) becomes the pending observation of the next slot.
- * grl_replay_size: complete transitions per environment, min(added, capacity).
+ * grl_replay_begin_indexed: closes every environment's open episode at its newest stored transition without marking it done, and
+ *   disarms every environment.  Writes no observation: an environment's next listing in grl_replay_add_indexed records it.
+ * grl_replay_add_indexed: env_ids_dev int32[count] (a grs_async_recv batch); the other arrays are the simulator's full
+ *   per-environment buffers ([N][...], read at row id; actions_dev = grs_buffer "actions", which grs_async_send fills).  A
+ *   disarmed environment gets obs[id] as its pending observation and is armed; an armed one completes its pending transition
+ *   as grl_replay_add does, then obs[id] becomes the next pending observation.  Ids < 0 are skipped; ids >= N are skipped and
+ *   reported; an id listed twice in one call is written once and reported.
+ * grl_replay_size: lock-step mode: complete transitions per environment, min(added, capacity).  Fails in indexed mode.
+ * grl_replay_status: synchronises the device; *transitions = the complete transitions stored over all environments (sum of
+ *   min(added[n], capacity)).  Reports the sticky error bits of indexed mode as a failure with their description, and clears them.
  * grl_replay_sample: `batch` transitions, a pure function of the buffer, seed, `draw`, batch and her_ratio.  Environment and
- *   transition uniform among the complete ones; with probability her_ratio the desired goal is replaced by the achieved goal
+ *   transition uniform among the complete ones (in indexed mode each environment is drawn in proportion to its complete
+ *   transitions, which with equal counts is the lock-step draw, bit for bit); with probability her_ratio the desired goal is replaced by the achieved goal
  *   (info[GRS_INFO_ACHIEVED]) of a transition drawn uniformly from the same episode at or after the sampled one (the episode ends
  *   at its done transition, or at the newest stored one while it runs), and with her_reward the reward becomes
  *   reward - h(ag, dg_old) + h(ag, dg_new), h(a, d) = 1 / exp(|d - a|) (0 for transitions with FLAGS bit 1).  A step
@@ -242,8 +258,11 @@ GRS_API int32_t grl_adam_step(float* params_dev, const float* grads_dev, float* 
  *   device arrays obs, next_obs u8[B][C][H][W] (16-byte aligned), actions f32[B][A], reward f32[B], done u8[B], desired_goal,
  *   achieved_goal f32[B][2]; info f32[B][GRS_INFO_STRIDE], index i64[B] (flat slot * N + env) and goal_index i64[B] (flat index
  *   of the goal's transition, -1 when not relabelled) may be NULL.  Fails on an empty buffer, batch <= 0 or her_ratio outside
- *   [0, 1].
- * grl_replay_buffer: named storage views "obs", "next_obs", "actions", "reward", "done", "info" ([S][N][...], S = capacity + 1). */
+ *   [0, 1]; in indexed mode an empty buffer is found on the device instead: every row gets index = goal_index = -1 (the other
+ *   outputs are not written) and grl_replay_status reports it.  Indexed sampling uses one scratch array of the buffer: do not
+ *   sample one buffer on two streams at once.
+ * grl_replay_buffer: named storage views "obs", "next_obs", "actions", "reward", "done", "info" ([S][N][...], S = capacity + 1)
+ *   and "added" (int64[N], indexed mode's per-environment counts of complete transitions). */
 typedef struct grl_replay grl_replay;
 GRS_API grl_replay* grl_replay_create(int32_t capacity, int32_t num_envs, int32_t channels, int32_t height, int32_t width, int32_t action_dim,
                                       int32_t her_reward, uint32_t seed, int32_t device);
@@ -251,7 +270,12 @@ GRS_API void grl_replay_destroy(grl_replay* rb);
 GRS_API int32_t grl_replay_begin(grl_replay* rb, const uint8_t* obs_dev, void* stream);
 GRS_API int32_t grl_replay_add(grl_replay* rb, const float* actions_dev, const float* reward_dev, const uint8_t* done_dev, const float* info_dev,
                                const uint8_t* obs_dev, const uint8_t* terminal_obs_dev, void* stream);
+GRS_API int32_t grl_replay_begin_indexed(grl_replay* rb, void* stream);
+GRS_API int32_t grl_replay_add_indexed(grl_replay* rb, const int32_t* env_ids_dev, int32_t count, const float* actions_dev, const float* reward_dev,
+                                       const uint8_t* done_dev, const float* info_dev, const uint8_t* obs_dev, const uint8_t* terminal_obs_dev,
+                                       void* stream);
 GRS_API int64_t grl_replay_size(const grl_replay* rb);
+GRS_API int32_t grl_replay_status(grl_replay* rb, int64_t* transitions);
 GRS_API int32_t grl_replay_sample(grl_replay* rb, int32_t batch, float her_ratio, uint64_t draw, uint8_t* obs_dev, uint8_t* next_obs_dev,
                                   float* actions_dev, float* reward_dev, uint8_t* done_dev, float* desired_goal_dev, float* achieved_goal_dev,
                                   float* info_dev, int64_t* index_dev, int64_t* goal_index_dev, void* stream);

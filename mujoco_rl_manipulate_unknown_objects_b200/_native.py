@@ -39,7 +39,7 @@ SYMBOLS += ["grp_last_error", "grp_create", "grp_destroy", "grp_num_params", "gr
 
 SYMBOLS += ["grl_last_error", "grl_gae", "grl_adam_step"]
 SYMBOLS += ["grl_replay_create", "grl_replay_destroy", "grl_replay_begin", "grl_replay_add", "grl_replay_size", "grl_replay_sample",
-            "grl_replay_buffer"]
+            "grl_replay_buffer", "grl_replay_begin_indexed", "grl_replay_add_indexed", "grl_replay_status"]
 
 _lib = None
 
@@ -126,6 +126,9 @@ def load():
     L.grl_replay_size.argtypes = [vp]
     L.grl_replay_sample.argtypes = [vp, i32, C.c_float, u64] + [vp] * 10 + [vp]
     L.grl_replay_buffer.argtypes = [vp, C.c_char_p, C.POINTER(vp), C.POINTER(u64)]
+    L.grl_replay_begin_indexed.argtypes = [vp, vp]
+    L.grl_replay_add_indexed.argtypes = [vp, vp, i32] + [vp] * 6 + [vp]
+    L.grl_replay_status.argtypes = [vp, C.POINTER(i64)]
     _lib = L
     return L
 

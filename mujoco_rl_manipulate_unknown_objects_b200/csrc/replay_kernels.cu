@@ -14,30 +14,50 @@
 //                     numbers come from a counter-based hash of (seed, draw, sample, k): a batch is a pure function of the
 //                     buffer contents and these arguments, with no generator state on the device.
 //
-// Layout: `capacity + 1` slots per environment, slot-major [S][N] like the PPO rollout storage; transition t (counted from 0
-// in lock-step over the environments) lives in slot t % S.  The extra slot holds the pending observation, so `capacity`
-// complete transitions stay sampleable once the ring has wrapped.
+// Layout: `capacity + 1` slots per environment, slot-major [S][N] like the PPO rollout storage; transition t of environment n
+// lives in slot t % S.  The extra slot holds the pending observation, so `capacity` complete transitions stay sampleable once
+// the ring has wrapped.
+//
+// Write modes, fixed by a buffer's first begin call:
+//   lock-step (k_replay_begin / k_replay_add): every environment adds in every call; t is one host-side counter.
+//   indexed (k_replay_begin_indexed / k_replay_add_indexed): the environments of an asynchronous pool advance at their own
+//     rates, so each has its own device-side cursor added[n].  An add call lists the environments it writes; the first listing
+//     after begin_indexed only records the observation (arms the environment), every later one completes a transition.
+//     Sampling first scans min(added[n], capacity) into csum (k_replay_scan) and then draws a transition uniformly over all
+//     complete ones: g < total, env = upper bound of g in csum.  With equal counts that is below(u0, N), the lock-step draw.
+//     Bad ids and an empty buffer set bits of a sticky device error word (ERR_*), read and cleared by grl_replay_status.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include <cmath>
 #include <cstring>
 #include <string>
+#include <vector>
 
 #include "../../include/b200_gripper_sim.h"
 
 int grl_set_error(const std::string& m);  // train_kernels.cu: grl_last_error()'s message
 
+enum { MODE_NONE = 0, MODE_LOCKSTEP, MODE_INDEXED };
+enum { ERR_RANGE = 1, ERR_DUPLICATE = 2, ERR_EMPTY = 4 };  // bits of the sticky device error word
+
 struct grl_replay {
   int K, S, N, C, H, W, A, her_reward, device;
   unsigned seed;
   long long img;     // bytes of one observation, a multiple of 16
-  long long added;   // complete transitions per environment ever added
-  bool begun;
+  long long added;   // lock-step mode: complete transitions per environment ever added
+  int mode;          // MODE_*: fixed by the first begin call
+  unsigned long long calls;  // indexed mode: add calls so far (the stamp of the next one is calls + 1)
   uint8_t *obs, *next_obs, *done;
   float *actions, *reward, *info;
   long long *ep_end;    // [S][N] transition index of the episode's last transition, -1 while the episode is open
   long long *ep_start;  // [N]    first transition of each environment's open episode
+  // indexed mode
+  long long* env_added;     // [N] complete transitions of each environment ever added
+  int* armed;               // [N] the environment's pending observation is recorded
+  unsigned long long* stamp;  // [N] the last add call that wrote the environment (duplicate ids in one call)
+  long long* csum;          // [N] inclusive prefix sum of min(env_added, K), written before every indexed sample
+  int* err;                 // sticky ERR_* bits
 };
 
 namespace {
@@ -50,10 +70,14 @@ struct Ring {
   long long *ep_end, *ep_start;
   long long img, S;
   int N, A;
+  long long *env_added, *csum;
+  int *armed, *err;
+  unsigned long long* stamp;
 };
 
 Ring ring_of(const grl_replay* r) {
-  return Ring{r->obs, r->next_obs, r->done, r->actions, r->reward, r->info, r->ep_end, r->ep_start, r->img, r->S, r->N, r->A};
+  return Ring{r->obs, r->next_obs, r->done, r->actions, r->reward, r->info, r->ep_end, r->ep_start, r->img, r->S, r->N, r->A,
+              r->env_added, r->csum, r->armed, r->err, r->stamp};
 }
 
 __host__ __device__ inline unsigned fmix(unsigned h) {
@@ -83,22 +107,39 @@ __device__ inline void close_episode(const Ring& r, int n, long long start, long
   for (long long u = lo + threadIdx.x; u <= t_end; u += blockDim.x) r.ep_end[(u % r.S) * r.N + n] = t_end;
 }
 
-__global__ void __launch_bounds__(THREADS) k_replay_begin(Ring r, const uint8_t* __restrict__ obs, long long added, long long K) {
-  const int n = blockIdx.x;
+// copies environment n's observation obs[n] into slot `slot` (the pending observation)
+__device__ inline void put_pending(const Ring& r, int n, long long slot, const uint8_t* __restrict__ obs) {
   const int4* src = reinterpret_cast<const int4*>(obs + (size_t)n * r.img);
-  int4* dst = reinterpret_cast<int4*>(r.obs + ((size_t)(added % r.S) * r.N + n) * r.img);
+  int4* dst = reinterpret_cast<int4*>(r.obs + ((size_t)slot * r.N + n) * r.img);
   for (long long i = threadIdx.x; i < r.img / 16; i += blockDim.x) dst[i] = __ldg(src + i);
+}
+
+// an explicit reset: closes environment n's open episode at its newest stored transition (added - 1), the next one starts at added
+__device__ inline void restart_episode(const Ring& r, int n, long long added, long long K) {
   const long long start = r.ep_start[n];
   __syncthreads();  // every thread has read ep_start before thread 0 moves it
   if (added > start) close_episode(r, n, start, added - 1, K);
   if (threadIdx.x == 0) r.ep_start[n] = added;
 }
 
-__global__ void __launch_bounds__(THREADS) k_replay_add(Ring r, const float* __restrict__ actions, const float* __restrict__ reward,
-                                                       const uint8_t* __restrict__ done, const float* __restrict__ info,
-                                                       const uint8_t* __restrict__ obs, const uint8_t* __restrict__ terminal_obs,
-                                                       long long t, long long K) {
+__global__ void __launch_bounds__(THREADS) k_replay_begin(Ring r, const uint8_t* __restrict__ obs, long long added, long long K) {
   const int n = blockIdx.x;
+  put_pending(r, n, added % r.S, obs);
+  restart_episode(r, n, added, K);
+}
+
+__global__ void __launch_bounds__(THREADS) k_replay_begin_indexed(Ring r, long long K) {
+  const int n = blockIdx.x;
+  restart_episode(r, n, r.env_added[n], K);
+  if (threadIdx.x == 0) r.armed[n] = 0;  // the environment's next listing in an add call records its observation
+}
+
+// Completes transition t of environment n from row n of the simulator's buffers (the whole block calls it): next_obs =
+// terminal_obs on done, else obs; action, reward, done and info row; the episode's bookkeeping; then obs (the reset observation
+// where done) becomes the pending observation of slot (t + 1) % S.
+__device__ inline void add_transition(const Ring& r, int n, long long t, long long K, const float* __restrict__ actions,
+                                      const float* __restrict__ reward, const uint8_t* __restrict__ done, const float* __restrict__ info,
+                                      const uint8_t* __restrict__ obs, const uint8_t* __restrict__ terminal_obs) {
   const size_t row = (size_t)(t % r.S) * r.N + n, nrow = (size_t)((t + 1) % r.S) * r.N + n;
   const int d = done[n] != 0;
   const int4* cur = reinterpret_cast<const int4*>(obs + (size_t)n * r.img);
@@ -123,34 +164,118 @@ __global__ void __launch_bounds__(THREADS) k_replay_add(Ring r, const float* __r
   }
 }
 
+__global__ void __launch_bounds__(THREADS) k_replay_add(Ring r, const float* __restrict__ actions, const float* __restrict__ reward,
+                                                       const uint8_t* __restrict__ done, const float* __restrict__ info,
+                                                       const uint8_t* __restrict__ obs, const uint8_t* __restrict__ terminal_obs,
+                                                       long long t, long long K) {
+  add_transition(r, blockIdx.x, t, K, actions, reward, done, info, obs, terminal_obs);
+}
+
+// one block per listed id; reads row id of the simulator's per-environment buffers
+__global__ void __launch_bounds__(THREADS) k_replay_add_indexed(Ring r, const int32_t* __restrict__ env_ids, const float* __restrict__ actions,
+                                                               const float* __restrict__ reward, const uint8_t* __restrict__ done,
+                                                               const float* __restrict__ info, const uint8_t* __restrict__ obs,
+                                                               const uint8_t* __restrict__ terminal_obs, unsigned long long call, long long K) {
+  __shared__ int s_go, s_armed;
+  __shared__ long long s_t;
+  const int id = env_ids[blockIdx.x];
+  if (id < 0) return;  // a short recv's missing entries
+  if (threadIdx.x == 0) {
+    s_go = 0;
+    if (id >= r.N) atomicOr(r.err, ERR_RANGE);
+    else if (atomicExch(r.stamp + id, call) == call) atomicOr(r.err, ERR_DUPLICATE);  // an earlier block of this call has it
+    else { s_go = 1; s_armed = r.armed[id]; s_t = r.env_added[id]; }
+  }
+  __syncthreads();
+  if (!s_go) return;
+  const long long t = s_t;
+  if (!s_armed) {
+    put_pending(r, id, t % r.S, obs);
+    if (threadIdx.x == 0) r.armed[id] = 1;
+    return;
+  }
+  add_transition(r, id, t, K, actions, reward, done, info, obs, terminal_obs);
+  if (threadIdx.x == 0) r.env_added[id] = t + 1;
+}
+
+// csum[n] = sum of min(env_added[m], K) over m <= n: one block, each thread scans a contiguous run of environments
+__global__ void __launch_bounds__(1024) k_replay_scan(Ring r, long long K) {
+  __shared__ long long part[1024];
+  const int per = (r.N + blockDim.x - 1) / blockDim.x, lo = threadIdx.x * per, hi = min(lo + per, r.N);
+  long long s = 0;
+  for (int n = lo; n < hi; n++) s += min(r.env_added[n], K);
+  part[threadIdx.x] = s;
+  __syncthreads();
+  for (int d = 1; d < blockDim.x; d <<= 1) {  // Hillis-Steele inclusive scan of the per-thread sums
+    const long long v = threadIdx.x >= d ? part[threadIdx.x - d] : 0;
+    __syncthreads();
+    part[threadIdx.x] += v;
+    __syncthreads();
+  }
+  s = threadIdx.x ? part[threadIdx.x - 1] : 0;
+  for (int n = lo; n < hi; n++) r.csum[n] = s += min(r.env_added[n], K);
+}
+
 struct SampleOut {
   uint8_t *obs, *next_obs, *done;
   float *actions, *reward, *desired, *achieved, *info;
   long long *index, *goal_index;
 };
 
+// INDEXED: `added` and `size` are ignored; the environment is drawn in proportion to its complete transitions (csum, written by
+// k_replay_scan on the same stream), then the transition uniformly among them.  An empty buffer gives index = goal_index = -1.
+template <bool INDEXED>
 __global__ void __launch_bounds__(THREADS) k_replay_sample(Ring r, SampleOut o, long long added, long long size, unsigned seed,
                                                           unsigned long long draw, float her_ratio, int her_reward) {
   __shared__ long long s_row, s_grow;
   const int b = blockIdx.x;
   if (threadIdx.x == 0) {
     const unsigned base = sample_base(seed, draw, (unsigned)b);
-    const long long env = below(sample_u32(base, 0), r.N);
-    const long long t = added - size + below(sample_u32(base, 1), size);
-    const long long row = (t % r.S) * r.N + env;
-    long long grow = -1;
-    if ((float)(sample_u32(base, 2) >> 8) * (1.0f / 16777216.0f) < her_ratio) {
-      const long long e = r.ep_end[row];
-      long long end = e >= 0 ? e : added - 1;
-      // a step whose state went non-finite (FLAGS bit 1, always the done step of its episode) records a non-finite achieved
-      // goal: it is never a goal source, and a sample that is such a step itself is not relabelled
-      if (e >= 0 && ((int)r.info[((e % r.S) * r.N + env) * GRS_INFO_STRIDE + GRS_INFO_FLAGS] & 2)) end = e - 1;
-      if (end >= t) grow = ((t + below(sample_u32(base, 3), end - t + 1)) % r.S) * r.N + env;
+    long long env = 0;
+    if constexpr (INDEXED) {
+      const long long total = r.csum[r.N - 1];
+      if (total > 0) {
+        const long long g = below(sample_u32(base, 0), total);
+        int lo = 0, hi = r.N - 1;  // the first environment whose csum exceeds g
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (r.csum[mid] > g) hi = mid;
+          else lo = mid + 1;
+        }
+        env = lo;
+        added = r.env_added[env];
+        size = r.csum[env] - (env ? r.csum[env - 1] : 0);
+      } else {
+        env = -1;
+      }
+    } else {
+      env = below(sample_u32(base, 0), r.N);
     }
-    s_row = row; s_grow = grow;
+    if (INDEXED && env < 0) {  // nothing to sample
+      atomicOr(r.err, ERR_EMPTY);
+      s_row = -1;
+    } else {
+      const long long t = added - size + below(sample_u32(base, 1), size);
+      const long long row = (t % r.S) * r.N + env;
+      long long grow = -1;
+      if ((float)(sample_u32(base, 2) >> 8) * (1.0f / 16777216.0f) < her_ratio) {
+        const long long e = r.ep_end[row];
+        long long end = e >= 0 ? e : added - 1;
+        // a step whose state went non-finite (FLAGS bit 1, always the done step of its episode) records a non-finite achieved
+        // goal: it is never a goal source, and a sample that is such a step itself is not relabelled
+        if (e >= 0 && ((int)r.info[((e % r.S) * r.N + env) * GRS_INFO_STRIDE + GRS_INFO_FLAGS] & 2)) end = e - 1;
+        if (end >= t) grow = ((t + below(sample_u32(base, 3), end - t + 1)) % r.S) * r.N + env;
+      }
+      s_row = row; s_grow = grow;
+    }
   }
   __syncthreads();
   const long long row = s_row, grow = s_grow;
+  if (INDEXED && row < 0) {
+    if (threadIdx.x == 0 && o.index) o.index[b] = -1;
+    if (threadIdx.x == 0 && o.goal_index) o.goal_index[b] = -1;
+    return;
+  }
   const long long nv = r.img / 16;
   const int4* so = reinterpret_cast<const int4*>(r.obs + row * r.img);
   const int4* sn = reinterpret_cast<const int4*>(r.next_obs + row * r.img);
@@ -201,10 +326,19 @@ void release(grl_replay* r) {
   cudaGetDevice(&prev);
   cudaSetDevice(r->device);
   for (void* p : {(void*)r->obs, (void*)r->next_obs, (void*)r->done, (void*)r->actions, (void*)r->reward, (void*)r->info, (void*)r->ep_end,
-                  (void*)r->ep_start})
+                  (void*)r->ep_start, (void*)r->env_added, (void*)r->armed, (void*)r->stamp, (void*)r->csum, (void*)r->err})
     if (p) cudaFree(p);
   cudaSetDevice(prev);
   delete r;
+}
+
+// refuses a call of the other write mode; otherwise fixes the buffer's mode to `mode`
+int claim_mode(grl_replay* rb, int mode, const char* who) {
+  if (rb->mode != MODE_NONE && rb->mode != mode)
+    return grl_set_error(std::string(who) + ": the buffer is in " + (rb->mode == MODE_INDEXED ? "indexed" : "lock-step") +
+                         " write mode; the two modes cannot be mixed on one buffer");
+  rb->mode = mode;
+  return 0;
 }
 
 }  // namespace
@@ -234,12 +368,17 @@ extern "C" grl_replay* grl_replay_create(int32_t capacity, int32_t num_envs, int
                     cudaMalloc(&r->done, rows) == cudaSuccess && cudaMalloc(&r->actions, rows * r->A * sizeof(float)) == cudaSuccess &&
                     cudaMalloc(&r->reward, rows * sizeof(float)) == cudaSuccess &&
                     cudaMalloc(&r->info, rows * GRS_INFO_STRIDE * sizeof(float)) == cudaSuccess &&
-                    cudaMalloc(&r->ep_end, rows * sizeof(long long)) == cudaSuccess && cudaMalloc(&r->ep_start, r->N * sizeof(long long)) == cudaSuccess;
+                    cudaMalloc(&r->ep_end, rows * sizeof(long long)) == cudaSuccess && cudaMalloc(&r->ep_start, r->N * sizeof(long long)) == cudaSuccess &&
+                    cudaMalloc(&r->env_added, r->N * sizeof(long long)) == cudaSuccess && cudaMalloc(&r->armed, r->N * sizeof(int)) == cudaSuccess &&
+                    cudaMalloc(&r->stamp, r->N * sizeof(unsigned long long)) == cudaSuccess &&
+                    cudaMalloc(&r->csum, r->N * sizeof(long long)) == cudaSuccess && cudaMalloc(&r->err, sizeof(int)) == cudaSuccess;
     if (!ok) {
       cudaGetLastError();
       return grl_set_error("grl_replay_create: cudaMalloc of " + std::to_string(rows) + " slots failed");
     }
-    if (cudaMemset(r->ep_end, 0xff, rows * sizeof(long long)) != cudaSuccess || cudaMemset(r->ep_start, 0, r->N * sizeof(long long)) != cudaSuccess)
+    if (cudaMemset(r->ep_end, 0xff, rows * sizeof(long long)) != cudaSuccess || cudaMemset(r->ep_start, 0, r->N * sizeof(long long)) != cudaSuccess ||
+        cudaMemset(r->env_added, 0, r->N * sizeof(long long)) != cudaSuccess || cudaMemset(r->armed, 0, r->N * sizeof(int)) != cudaSuccess ||
+        cudaMemset(r->stamp, 0, r->N * sizeof(unsigned long long)) != cudaSuccess || cudaMemset(r->err, 0, sizeof(int)) != cudaSuccess)
       return grl_set_error("grl_replay_create: cudaMemset failed");
     return 0;
   });
@@ -254,18 +393,27 @@ extern "C" void grl_replay_destroy(grl_replay* rb) {
 extern "C" int32_t grl_replay_begin(grl_replay* rb, const uint8_t* obs_dev, void* stream) {
   if (!rb || !obs_dev) return grl_set_error("grl_replay_begin: null pointer");
   if (misaligned(obs_dev)) return grl_set_error("grl_replay_begin: obs must be 16-byte aligned");
+  if (const int rc = claim_mode(rb, MODE_LOCKSTEP, "grl_replay_begin")) return rc;
   return on_device(rb->device, [&]() -> int {
     k_replay_begin<<<rb->N, THREADS, 0, (cudaStream_t)stream>>>(ring_of(rb), obs_dev, rb->added, rb->K);
-    const int rc = launched("grl_replay_begin");
-    if (rc == 0) rb->begun = true;
-    return rc;
+    return launched("grl_replay_begin");
+  });
+}
+
+extern "C" int32_t grl_replay_begin_indexed(grl_replay* rb, void* stream) {
+  if (!rb) return grl_set_error("grl_replay_begin_indexed: null pointer");
+  if (const int rc = claim_mode(rb, MODE_INDEXED, "grl_replay_begin_indexed")) return rc;
+  return on_device(rb->device, [&]() -> int {
+    k_replay_begin_indexed<<<rb->N, THREADS, 0, (cudaStream_t)stream>>>(ring_of(rb), rb->K);
+    return launched("grl_replay_begin_indexed");
   });
 }
 
 extern "C" int32_t grl_replay_add(grl_replay* rb, const float* actions_dev, const float* reward_dev, const uint8_t* done_dev, const float* info_dev,
                                   const uint8_t* obs_dev, const uint8_t* terminal_obs_dev, void* stream) {
   if (!rb || !actions_dev || !reward_dev || !done_dev || !info_dev || !obs_dev || !terminal_obs_dev) return grl_set_error("grl_replay_add: null pointer");
-  if (!rb->begun) return grl_set_error("grl_replay_add: call grl_replay_begin with the observations the actions were taken on first");
+  if (rb->mode == MODE_INDEXED) return grl_set_error("grl_replay_add: the buffer is in indexed write mode (grl_replay_add_indexed)");
+  if (rb->mode != MODE_LOCKSTEP) return grl_set_error("grl_replay_add: call grl_replay_begin with the observations the actions were taken on first");
   if (misaligned(obs_dev) || misaligned(terminal_obs_dev)) return grl_set_error("grl_replay_add: obs and terminal_obs must be 16-byte aligned");
   return on_device(rb->device, [&]() -> int {
     k_replay_add<<<rb->N, THREADS, 0, (cudaStream_t)stream>>>(ring_of(rb), actions_dev, reward_dev, done_dev, info_dev, obs_dev, terminal_obs_dev,
@@ -276,9 +424,59 @@ extern "C" int32_t grl_replay_add(grl_replay* rb, const float* actions_dev, cons
   });
 }
 
+extern "C" int32_t grl_replay_add_indexed(grl_replay* rb, const int32_t* env_ids_dev, int32_t count, const float* actions_dev, const float* reward_dev,
+                                          const uint8_t* done_dev, const float* info_dev, const uint8_t* obs_dev, const uint8_t* terminal_obs_dev,
+                                          void* stream) {
+  if (!rb || !env_ids_dev || !actions_dev || !reward_dev || !done_dev || !info_dev || !obs_dev || !terminal_obs_dev)
+    return grl_set_error("grl_replay_add_indexed: null pointer");
+  if (rb->mode == MODE_LOCKSTEP) return grl_set_error("grl_replay_add_indexed: the buffer is in lock-step write mode (grl_replay_add)");
+  if (rb->mode != MODE_INDEXED) return grl_set_error("grl_replay_add_indexed: call grl_replay_begin_indexed first");
+  if (count < 0) return grl_set_error("grl_replay_add_indexed: count must not be negative");
+  if (misaligned(obs_dev) || misaligned(terminal_obs_dev)) return grl_set_error("grl_replay_add_indexed: obs and terminal_obs must be 16-byte aligned");
+  if (count == 0) return 0;
+  return on_device(rb->device, [&]() -> int {
+    k_replay_add_indexed<<<count, THREADS, 0, (cudaStream_t)stream>>>(ring_of(rb), env_ids_dev, actions_dev, reward_dev, done_dev, info_dev, obs_dev,
+                                                                     terminal_obs_dev, rb->calls + 1, rb->K);
+    const int rc = launched("grl_replay_add_indexed");
+    if (rc == 0) rb->calls++;
+    return rc;
+  });
+}
+
 extern "C" int64_t grl_replay_size(const grl_replay* rb) {
   if (!rb) return -1;
+  if (rb->mode == MODE_INDEXED) {
+    grl_set_error("grl_replay_size: the environments of an indexed-mode buffer hold different counts; grl_replay_status gives the total");
+    return -1;
+  }
   return rb->added < rb->K ? rb->added : rb->K;
+}
+
+extern "C" int32_t grl_replay_status(grl_replay* rb, int64_t* transitions) {
+  if (!rb || !transitions) return grl_set_error("grl_replay_status: null pointer");
+  if (rb->mode != MODE_INDEXED) {
+    *transitions = (rb->added < rb->K ? rb->added : rb->K) * (int64_t)rb->N;
+    return 0;
+  }
+  return on_device(rb->device, [&]() -> int {
+    std::vector<long long> added(rb->N);
+    int err = 0;
+    if (cudaDeviceSynchronize() != cudaSuccess || cudaMemcpy(added.data(), rb->env_added, rb->N * sizeof(long long), cudaMemcpyDeviceToHost) != cudaSuccess ||
+        cudaMemcpy(&err, rb->err, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess || (err && cudaMemset(rb->err, 0, sizeof(int)) != cudaSuccess)) {
+      const cudaError_t e = cudaGetLastError();
+      return grl_set_error(std::string("grl_replay_status: ") + cudaGetErrorString(e));
+    }
+    long long total = 0;
+    for (long long a : added) total += a < rb->K ? a : rb->K;
+    *transitions = total;
+    if (!err) return 0;
+    std::string m = "grl_replay_status:";
+    if (err & ERR_RANGE) m += " an add_indexed call listed an environment id >= num_envs (skipped);";
+    if (err & ERR_DUPLICATE) m += " an add_indexed call listed an environment id twice (written once);";
+    if (err & ERR_EMPTY) m += " a sample found no complete transition (its rows have index -1);";
+    m.pop_back();
+    return grl_set_error(m);
+  });
 }
 
 extern "C" int32_t grl_replay_sample(grl_replay* rb, int32_t batch, float her_ratio, uint64_t draw, uint8_t* obs_dev, uint8_t* next_obs_dev,
@@ -286,16 +484,23 @@ extern "C" int32_t grl_replay_sample(grl_replay* rb, int32_t batch, float her_ra
                                      float* info_dev, int64_t* index_dev, int64_t* goal_index_dev, void* stream) {
   if (!rb || !obs_dev || !next_obs_dev || !actions_dev || !reward_dev || !done_dev || !desired_goal_dev || !achieved_goal_dev)
     return grl_set_error("grl_replay_sample: null pointer");
-  const long long size = grl_replay_size(rb);
-  if (size <= 0) return grl_set_error("grl_replay_sample: the buffer holds no complete transition");
+  const bool indexed = rb->mode == MODE_INDEXED;
+  const long long size = indexed ? 0 : grl_replay_size(rb);
+  if (!indexed && size <= 0) return grl_set_error("grl_replay_sample: the buffer holds no complete transition");
   if (batch <= 0) return grl_set_error("grl_replay_sample: batch size must be positive");
   if (!(her_ratio >= 0.0f && her_ratio <= 1.0f)) return grl_set_error("grl_replay_sample: her_ratio must lie in [0, 1]");
   if (misaligned(obs_dev) || misaligned(next_obs_dev)) return grl_set_error("grl_replay_sample: obs and next_obs must be 16-byte aligned");
   const SampleOut o{obs_dev, next_obs_dev, done_dev, actions_dev, reward_dev, desired_goal_dev, achieved_goal_dev, info_dev,
                     reinterpret_cast<long long*>(index_dev), reinterpret_cast<long long*>(goal_index_dev)};
   return on_device(rb->device, [&]() -> int {
-    k_replay_sample<<<batch, THREADS, 0, (cudaStream_t)stream>>>(ring_of(rb), o, rb->added, size, rb->seed, (unsigned long long)draw, her_ratio,
-                                                                rb->her_reward);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (indexed) {
+      k_replay_scan<<<1, 1024, 0, st>>>(ring_of(rb), rb->K);
+      if (const int rc = launched("grl_replay_sample")) return rc;
+      k_replay_sample<true><<<batch, THREADS, 0, st>>>(ring_of(rb), o, 0, 0, rb->seed, (unsigned long long)draw, her_ratio, rb->her_reward);
+    } else {
+      k_replay_sample<false><<<batch, THREADS, 0, st>>>(ring_of(rb), o, rb->added, size, rb->seed, (unsigned long long)draw, her_ratio, rb->her_reward);
+    }
     return launched("grl_replay_sample");
   });
 }
@@ -305,7 +510,8 @@ extern "C" int32_t grl_replay_buffer(grl_replay* rb, const char* name, void** pt
   const uint64_t rows = (uint64_t)rb->S * rb->N;
   struct { const char* n; void* p; uint64_t b; } views[] = {
       {"obs", rb->obs, rows * rb->img}, {"next_obs", rb->next_obs, rows * rb->img}, {"actions", rb->actions, rows * rb->A * sizeof(float)},
-      {"reward", rb->reward, rows * sizeof(float)}, {"done", rb->done, rows}, {"info", rb->info, rows * GRS_INFO_STRIDE * sizeof(float)}};
+      {"reward", rb->reward, rows * sizeof(float)}, {"done", rb->done, rows}, {"info", rb->info, rows * GRS_INFO_STRIDE * sizeof(float)},
+      {"added", rb->env_added, (uint64_t)rb->N * sizeof(long long)}};
   for (auto& v : views)
     if (std::strcmp(v.n, name) == 0) { *ptr = v.p; *bytes = v.b; return 0; }
   return grl_set_error(std::string("grl_replay_buffer: unknown buffer '") + name + "'");

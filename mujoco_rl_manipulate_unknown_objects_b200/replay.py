@@ -5,6 +5,9 @@ Replaces SB3's HerReplayBuffer (train_agent.py:61-88) for the batched environmen
 simulator's device buffers and sampled, with "future" goal relabelling and the reward recomputed on the device, into device
 tensors.  Differs from SB3 2.x in one respect: SB3 samples only from finished episodes, here every complete transition can be
 sampled (a 400-step episode does not fit a 128-slot ring); a goal drawn for a running episode comes from its stored part.
+
+Two write modes, fixed by the first begin call: lock-step (`begin` / `add`, every environment in every call) and indexed
+(`begin_indexed` / `add_indexed`, the environments an AsyncGripperEnv.recv returned, each with its own count on the device).
 """
 import ctypes as C
 
@@ -13,10 +16,11 @@ from ._native import INFO
 
 
 class DeviceReplayBuffer:
-    """`capacity` transitions per environment for `num_envs` environments that step in lock-step, on one GPU.
+    """`capacity` transitions per environment for `num_envs` environments, on one GPU.
 
     Storage views (torch tensors aliasing the library's memory, slot-major [capacity + 1, num_envs, ...]): obs, next_obs,
-    actions, reward, done, info.  Calls run on torch's current stream."""
+    actions, reward, done, info; `added` int64[num_envs] counts each environment's complete transitions in indexed mode.
+    Calls run on torch's current stream."""
 
     def __init__(self, capacity, num_envs, obs_shape=(5, 64, 64), action_dim=6, her_reward=False, seed=0, device=0):
         import torch
@@ -31,7 +35,8 @@ class DeviceReplayBuffer:
         self.capacity, self.num_envs, self.obs_shape, self.action_dim = int(capacity), int(num_envs), (c, h, w), int(action_dim)
         self.her_reward, self.seed = bool(her_reward), int(seed)
         self.device = torch.device("cuda", int(device))
-        self.begun = False  # begin() has recorded the observations the next actions are taken on
+        self.begun = False  # begin() or begin_indexed() was called
+        self.indexed = False  # the buffer is in indexed write mode
         self.draw = 0  # counter of sample() calls: the batch is a pure function of the buffer, seed, draw, size and her_ratio
         S, N = self.capacity + 1, self.num_envs
         self.obs = self._view("obs", (S, N, c, h, w), torch.uint8)
@@ -40,6 +45,7 @@ class DeviceReplayBuffer:
         self.reward = self._view("reward", (S, N), torch.float32)
         self.done = self._view("done", (S, N), torch.uint8)
         self.info = self._view("info", (S, N, INFO["STRIDE"]), torch.float32)
+        self.added = self._view("added", (N,), torch.int64)
         self.nbytes = sum(t.numel() * t.element_size() for t in (self.obs, self.next_obs, self.actions, self.reward, self.done, self.info))
 
     def _check(self, rc):
@@ -72,6 +78,12 @@ class DeviceReplayBuffer:
         self._check(self._lib.grl_replay_begin(self._h, self._ptr(obs, self._torch.uint8, (self.num_envs,) + self.obs_shape), self._stream()))
         self.begun = True
 
+    def begin_indexed(self):
+        """Enters indexed write mode, for an asynchronous pool, after every AsyncGripperEnv.async_reset: closes the open
+        episodes and disarms every environment, whose next listing in add_indexed() then records its observation."""
+        self._check(self._lib.grl_replay_begin_indexed(self._h, self._stream()))
+        self.begun = self.indexed = True
+
     def add(self, actions, reward, done, info, obs, terminal_obs):
         """One vectorised step, from the simulator's buffers after its step (GripperSim.actions / reward / done / info / obs /
         terminal_obs)."""
@@ -81,12 +93,38 @@ class DeviceReplayBuffer:
                                              self._ptr(done, t.uint8, (N,)), self._ptr(info, t.float32, (N, INFO["STRIDE"])),
                                              self._ptr(obs, t.uint8, img), self._ptr(terminal_obs, t.uint8, img), self._stream()))
 
+    def add_indexed(self, env_ids, actions, reward, done, info, obs, terminal_obs):
+        """The environments env_ids (int32 [n], an AsyncGripperEnv.recv batch; -1 entries are skipped) from the simulator's
+        full per-environment buffers [N, ...] (GripperSim.actions / reward / done / info / obs / terminal_obs, read at row id).
+        Out-of-range and duplicated ids are reported by status()."""
+        t, N = self._torch, self.num_envs
+        img = (N,) + self.obs_shape
+        if env_ids.device != self.device or env_ids.dtype != t.int32 or not env_ids.is_contiguous() or env_ids.dim() != 1:
+            raise ValueError("env_ids must be a contiguous 1-d int32 tensor on %s" % self.device)
+        self._check(self._lib.grl_replay_add_indexed(self._h, C.c_void_p(env_ids.data_ptr()), env_ids.numel(),
+                                                     self._ptr(actions, t.float32, (N, self.action_dim)), self._ptr(reward, t.float32, (N,)),
+                                                     self._ptr(done, t.uint8, (N,)), self._ptr(info, t.float32, (N, INFO["STRIDE"])),
+                                                     self._ptr(obs, t.uint8, img), self._ptr(terminal_obs, t.uint8, img), self._stream()))
+
+    def status(self):
+        """Synchronises and returns the complete transitions stored over all environments; raises NativeError if an indexed
+        add or sample met a bad id or an empty buffer since the last call (the error is cleared by reporting it)."""
+        n = C.c_int64()
+        self._check(self._lib.grl_replay_status(self._h, C.byref(n)))
+        return int(n.value)
+
     @property
     def transitions_per_env(self):
-        return int(self._lib.grl_replay_size(self._h))
+        """Lock-step mode only (raises in indexed mode, where the counts differ)."""
+        n = int(self._lib.grl_replay_size(self._h))
+        if n < 0:
+            self._check(n)
+        return n
 
     def __len__(self):
-        """Complete transitions stored over all environments."""
+        """Complete transitions stored over all environments (synchronises in indexed mode)."""
+        if self.indexed:
+            return int(self.added.clamp(max=self.capacity).sum())
         return self.transitions_per_env * self.num_envs
 
     # ------------------------------------------------------------------ sampling
@@ -94,6 +132,7 @@ class DeviceReplayBuffer:
         """`batch_size` transitions as a dict of device tensors: obs, next_obs u8[B, C, H, W], actions f32[B, A], reward f32[B],
         done u8[B], desired_goal, achieved_goal f32[B, 2], info f32[B, 40], index i64[B] (flat slot * N + env into the storage
         views) and goal_index i64[B] (flat index of the transition the relabelled goal comes from, -1 if not relabelled).
+        In indexed mode an empty buffer is not seen on the host: every row gets index -1 and status() raises.
         her_ratio: probability of "future" relabelling (SB3's n_sampled_goal=4 is 0.8).  draw: the sampling counter to use
         (default: the next one)."""
         t = self._torch

@@ -55,16 +55,26 @@ class RolloutStats:
         self._t = torch
         self.v = torch.zeros(len(STAT_NAMES), dtype=torch.float64, device=device)
 
-    def update(self, info, reward, done):
-        """info f32[N, 40] (GRS_INFO_* layout), reward f32[N], done u8/bool[N] of one vectorised step."""
+    def update(self, info, reward, done, weight=None):
+        """info f32[N, 40] (GRS_INFO_* layout), reward f32[N], done u8/bool[N] of one vectorised step.  weight (optional,
+        [N]): each row counts weight times (0 leaves a row out without boolean indexing, which would synchronise)."""
         t, I = self._t, INFO
-        d = done.to(t.float64)
-        nsub = info[:, I["NSUB_A"]:I["NSUB_A"] + 3].sum(dtype=t.float64)
+        if weight is not None:
+            w = weight.to(t.float64)
+            d = done.to(t.float64) * w
+            n = w.sum()
+            total = lambda x: (x.to(t.float64) * w).sum()  # noqa: E731
+            nsub = total(info[:, I["NSUB_A"]:I["NSUB_A"] + 3].sum(1, dtype=t.float64))
+        else:
+            d = done.to(t.float64)
+            n = t.tensor(float(info.shape[0]), dtype=t.float64, device=info.device)
+            total = lambda x: x.sum(dtype=t.float64)  # noqa: E731
+            nsub = info[:, I["NSUB_A"]:I["NSUB_A"] + 3].sum(dtype=t.float64)
         row = t.stack([
-            t.tensor(float(info.shape[0]), dtype=t.float64, device=info.device), nsub, reward.sum(dtype=t.float64), d.sum(),
+            n, nsub, total(reward), d.sum(),
             (info[:, I["EPISODE_RETURN"]].to(t.float64) * d).sum(), (info[:, I["EPISODE_STEP"]].to(t.float64) * d).sum(),
-            ((info[:, I["STATUS"]] == 1).to(t.float64) * d).sum(), info[:, I["LINE_DISTANCE"]].sum(dtype=t.float64),
-            info[:, I["TOTAL_DISTANCE"]].sum(dtype=t.float64), (info[:, I["GRASP"]] == 3).sum().to(t.float64)])
+            ((info[:, I["STATUS"]] == 1).to(t.float64) * d).sum(), total(info[:, I["LINE_DISTANCE"]]),
+            total(info[:, I["TOTAL_DISTANCE"]]), total(info[:, I["GRASP"]] == 3)])
         self.v += row
 
     def all_reduce(self):
@@ -154,6 +164,44 @@ class RolloutWorker:
                     storage["mu"][k].copy_(self.policy.mu[:n])
                     storage["log_std"][k].copy_(self.policy.log_std[:n])
                     storage["noise"][k].copy_(self.noise)
+        return stats
+
+    def start_async(self, batch_size, replay=None):
+        """Switches the worker to an asynchronous pool over its simulator (AsyncGripperEnv, batch `batch_size`): resets every
+        environment and, with a replay buffer, enters its indexed write mode (DeviceReplayBuffer.begin_indexed)."""
+        from .async_env import AsyncGripperEnv
+        t = self.sim._torch
+        if getattr(self, "pool", None) is not None:
+            self.pool.async_end()  # a restart needs every environment received first
+        self.pool = AsyncGripperEnv(self.sim, batch_size)
+        self.pool.async_reset()
+        if replay is not None:
+            replay.begin_indexed()
+        # stepped[n]: environment n has completed an agent step since async_reset (its first return is the reset observation);
+        # entry N takes the -1 ids of a short recv
+        self._stepped = t.zeros(self.sim.num_envs + 1, dtype=t.bool, device=self.device)
+
+    def collect_async(self, n_recv, deterministic=False, replay=None):
+        """n_recv rounds of the pool started by start_async: recv the next batch, add it to `replay` (optional, indexed mode)
+        straight from the simulator's per-environment buffers, count it, run the policy on its observations and send the
+        actions.  No host synchronisation.  The statistics cover the returned rows that end an agent step, not the first
+        return of each environment after start_async.  Returns RolloutStats (local; call .all_reduce())."""
+        t, s = self.sim._torch, self.sim
+        stats = RolloutStats(self.device)
+        B = self.pool.batch_size
+        for _ in range(n_recv):
+            r = self.pool.recv()
+            ids = r["env_id"]
+            if replay is not None:
+                replay.add_indexed(ids, s.actions, s.reward, s.done, s.info, s.obs, s.terminal_obs)
+            slot = t.where(ids >= 0, ids.long(), s.num_envs)
+            stats.update(r["info"], r["reward"], r["done"], weight=self._stepped[slot] & (ids >= 0))
+            self._stepped[slot] = True
+            act, noise = self.actions[:B], self.noise[:B]
+            if not deterministic:
+                noise.normal_(generator=self.gen)
+            self.policy.forward(r["obs"], deterministic=deterministic, noise=None if deterministic else noise, out=act)
+            self.pool.send(act, ids)
         return stats
 
     def make_storage(self, n_steps):

@@ -255,6 +255,13 @@ class GripperSim(CompiledModel):
         return rgb, depth
 
     @property
+    def actions(self):
+        """float32 [N, action_dim] view of the library's action buffer: the actions AsyncGripperEnv.send stored for each
+        environment (row id), unchanged until the environment is sent again.  The synchronous step() need not write it."""
+        N, a = self.num_envs, self.action_dim
+        return self._tensor("actions", (N * 6,), "<f4")[:N * a].view(N, a)  # allocated N x 6, written with stride action_dim
+
+    @property
     def launch_count(self):
         return int(self._lib.grs_launch_count(self._h))
 

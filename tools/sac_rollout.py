@@ -4,12 +4,20 @@ from it (k_replay_sample + torch autograd + one flat-bucket Adam per optimiser, 
 
   python tools/sac_rollout.py [--envs 4096] [--capacity 128] [--steps 16] [--iters 3] [--gradient-steps 16]   # one GPU
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P tools/sac_rollout.py
+  python tools/sac_rollout.py --pool-batch B [...]   # the asynchronous pool: N = --envs environments, batch B
 
 Per iteration, rank 0 prints one JSON line: rollout substeps/s over all ranks with and without replay= (two workers built with the
 same seeds and weights, so both step the same trajectories), the gradient-step time, the replay ratio (gradient steps per
 collected transition), the buffer's bytes, and every rank's parameter checksum.  A last line gives the k_replay_add /
 k_replay_sample times (CUDA events over many launches) with the bytes they move, computed from the shapes, and the card's name
-and power limit."""
+and power limit.
+
+With --pool-batch B the workers run an AsyncGripperEnv pool (RolloutWorker.start_async / collect_async) and the buffer is in
+indexed write mode.  An iteration is steps x N / B recvs, the same number of transitions per environment as the synchronous
+mode; the "plain" worker runs the same pool without the buffer (its completion order is scheduling-dependent, so
+same_trajectories is not expected).  The kernel line times k_replay_add_indexed at B ids and the indexed sample (k_replay_scan +
+k_replay_sample<true>) at batch 256 and 4 096, each next to the lock-step kernel at the same size (k_replay_add over B
+environments, k_replay_sample<false> on a filled lock-step buffer of the training buffer's shape)."""
 import argparse, json, os, subprocess, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -24,7 +32,9 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--scene", default="sugar_cube"); ap.add_argument("--envs", type=int, default=4096); ap.add_argument("--capacity", type=int, default=128)
 ap.add_argument("--steps", type=int, default=16); ap.add_argument("--iters", type=int, default=3); ap.add_argument("--gradient-steps", type=int, default=16)
 ap.add_argument("--batch", type=int, default=256); ap.add_argument("--her-ratio", type=float, default=0.8); ap.add_argument("--launches", type=int, default=50)
+ap.add_argument("--pool-batch", type=int, default=0, help="run the asynchronous pool with this batch size (0: the synchronous step)")
 a = ap.parse_args()
+pool = a.pool_batch > 0
 rank, world, local = dist_info()
 local %= torch.cuda.device_count()  # more ranks than GPUs (a functional check on one card) share them over gloo instead of NCCL
 torch.cuda.set_device(local)
@@ -40,6 +50,15 @@ N, obs_shape, A = a.envs, w.sim.obs_shape, w.sim.action_dim
 rb = DeviceReplayBuffer(a.capacity, N, obs_shape, A, her_reward=True, seed=rank_seed(0, rank), device=local)
 learner = SACLearner(w, rb, batch_size=a.batch, her_ratio=a.her_ratio, seed=1)
 plain.policy.load_state_dict(learner.actor.state_dict())
+if pool:
+    recvs = a.steps * N // a.pool_batch
+    plain.start_async(a.pool_batch)
+    w.start_async(a.pool_batch, replay=rb)
+    collect_plain = lambda: plain.collect_async(recvs)  # noqa: E731
+    collect_replay = lambda: w.collect_async(recvs, replay=rb)  # noqa: E731
+else:
+    collect_plain = lambda: plain.collect(a.steps)  # noqa: E731
+    collect_replay = lambda: w.collect(a.steps, replay=rb)  # noqa: E731
 
 
 def timed(fn):
@@ -69,9 +88,9 @@ def gather(x):
 
 collected = 0
 for it in range(a.iters):
-    t_plain, s_plain = timed(lambda: plain.collect(a.steps).all_reduce())
-    t_replay, s_replay = timed(lambda: w.collect(a.steps, replay=rb).all_reduce())
-    collected += a.steps * N * world
+    t_plain, s_plain = timed(lambda: collect_plain().all_reduce())
+    t_replay, s_replay = timed(lambda: collect_replay().all_reduce())
+    collected += s_replay.as_dict()["transitions"]
     t_update, losses = timed(lambda: learner.update(a.gradient_steps))
     plain.policy.load_state_dict(learner.actor.state_dict())  # both workers keep stepping the same trajectories
     t_plain, t_replay, t_update = max_over_ranks(t_plain, t_replay, t_update)
@@ -79,11 +98,14 @@ for it in range(a.iters):
     dp, dr = s_plain.as_dict(), s_replay.as_dict()
     if rank == 0:
         print(json.dumps({"iter": it, "n_gpus": world, "envs_per_gpu": N, "rollout_steps": a.steps, "capacity": a.capacity,
+                          "mode": "pool" if pool else "sync", "pool_batch": a.pool_batch if pool else None,
                           "substeps_per_s_plain": dp["substeps"] / t_plain, "substeps_per_s_replay": dr["substeps"] / t_replay,
-                          "same_trajectories": dp["substeps"] == dr["substeps"] and dp["reward_sum"] == dr["reward_sum"],
+                          "transitions_per_s_plain": dp["transitions"] / t_plain, "transitions_per_s_replay": dr["transitions"] / t_replay,
+                          "same_trajectories": None if pool else dp["substeps"] == dr["substeps"] and dp["reward_sum"] == dr["reward_sum"],
                           "replay_overhead": t_replay / t_plain - 1.0, "gradient_steps": a.gradient_steps, "batch": a.batch,
                           "gradient_step_ms": 1e3 * t_update / a.gradient_steps, "replay_ratio": learner.actor_opt.step_count * world / collected,
                           "buffer_bytes_per_gpu": rb.nbytes, "stored_transitions_per_gpu": len(rb), "losses": losses,
+                          "added_min_max": [int(rb.added.min()), int(rb.added.max())] if pool else None,
                           "param_checksum_per_rank": sums, "checksums_equal": len(set(sums)) == 1}), flush=True)
 
 # kernel times: CUDA events over many launches.  The add kernel runs on a second, small buffer (its cost does not depend on the
@@ -91,8 +113,6 @@ for it in range(a.iters):
 img = int(torch.tensor(obs_shape).prod())
 small = 4 * (A + 1 + INFO["STRIDE"]) + 1
 add_bytes = {"read": N * (img + small), "written": N * (2 * img + small + 8)}
-bench = DeviceReplayBuffer(16, N, obs_shape, A, device=local)
-bench.begin(w.sim.obs)
 s = w.sim
 args = (w.actions, s.reward, s.done, s.info, s.obs, s.terminal_obs)
 
@@ -110,15 +130,55 @@ def events(fn, n):
     return e0.elapsed_time(e1) / n * 1e3  # us
 
 
-res = {"k_replay_add": {"envs": N, "us": events(lambda: bench.add(*args), a.launches), **add_bytes}}
-res["k_replay_add"]["GB_per_s"] = (add_bytes["read"] + add_bytes["written"]) / res["k_replay_add"]["us"] / 1e3
-res["k_replay_sample"] = []
-for B in (256, 4096, 16384):
-    by = {"read": B * (2 * img + small + 16), "written": B * (2 * img + small + 16 + 16)}
-    draws = iter(range(10 ** 6, 2 * 10 ** 6))
-    us = events(lambda: rb.sample(B, a.her_ratio, draw=next(draws)), a.launches)
-    res["k_replay_sample"].append({"batch": B, "us": us, **by, "GB_per_s": (by["read"] + by["written"]) / us / 1e3})
-bench.close()
+def sample_bytes(B):
+    return {"read": B * (2 * img + small + 16), "written": B * (2 * img + small + 16 + 16)}
+
+
+def rate(d):
+    d["GB_per_s"] = (d["read"] + d["written"]) / d["us"] / 1e3
+    return d
+
+
+if not pool:
+    bench = DeviceReplayBuffer(16, N, obs_shape, A, device=local)
+    bench.begin(w.sim.obs)
+    res = {"k_replay_add": rate({"envs": N, "us": events(lambda: bench.add(*args), a.launches), **add_bytes})}
+    res["k_replay_sample"] = []
+    for B in (256, 4096, 16384):
+        draws = iter(range(10 ** 6, 2 * 10 ** 6))
+        us = events(lambda: rb.sample(B, a.her_ratio, draw=next(draws)), a.launches)
+        res["k_replay_sample"].append(rate({"batch": B, "us": us, **sample_bytes(B)}))
+    bench.close()
+else:
+    # k_replay_add_indexed at B ids (an indexed buffer over all N environments, armed once) next to k_replay_add over B environments
+    Bp = a.pool_batch
+    ix = DeviceReplayBuffer(16, N, obs_shape, A, device=local)
+    ix.begin_indexed()
+    ids = torch.randperm(N, device=w.device, generator=torch.Generator(device=w.device).manual_seed(0)).int()
+    ix.add_indexed(ids, *args)
+    ids = ids[:Bp].contiguous()
+    ls = DeviceReplayBuffer(16, Bp, obs_shape, A, device=local)
+    ls.begin(s.obs[:Bp])
+    ls_args = tuple(x[:Bp] for x in args)
+    rows = {"read": Bp * (img + small) + 4 * Bp, "written": Bp * (2 * img + small + 8)}
+    res = {"k_replay_add_indexed": rate({"ids": Bp, "us": events(lambda: ix.add_indexed(ids, *args), a.launches), **rows}),
+           "k_replay_add": rate({"envs": Bp, "us": events(lambda: ls.add(*ls_args), a.launches), **dict(rows, read=Bp * (img + small))})}
+    ix.close()
+    ls.close()
+    # the indexed sample (scan + gather) on the training buffer, the lock-step sample on a filled buffer of the same shape
+    ref = DeviceReplayBuffer(a.capacity, N, obs_shape, A, her_reward=True, device=local)
+    ref.begin(s.obs)
+    for _ in range(a.capacity + 1):
+        ref.add(*args)
+    res["sample"] = []
+    for B in (256, 4096):
+        draws = iter(range(10 ** 6, 2 * 10 ** 6))
+        us_ix = events(lambda: rb.sample(B, a.her_ratio, draw=next(draws)), a.launches)
+        us_ls = events(lambda: ref.sample(B, a.her_ratio, draw=next(draws)), a.launches)
+        res["sample"].append({"batch": B, "indexed": rate({"us": us_ix, **sample_bytes(B), "scan_read": 8 * N, "scan_written": 8 * N}),
+                              "lock_step": rate({"us": us_ls, **sample_bytes(B)})})
+    ref.close()
+    rb.status()  # raises on a bad id or an empty sample recorded on the device
 if rank == 0:
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i", str(local)],
                        stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True).stdout.strip()
