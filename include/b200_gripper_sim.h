@@ -62,7 +62,9 @@ enum {
   GRS_INFO_FINAL_OBJ_POS = 18 /*3*/, GRS_INFO_GRIPPER_POS = 21 /*3*/, GRS_INFO_ACHIEVED = 24 /*2*/, GRS_INFO_DESIRED = 26 /*2*/,
   GRS_INFO_SOLVER_ITERS = 28 /* Newton iterations summed over the substeps */, GRS_INFO_NCON_MAX,
   GRS_INFO_FLAGS /* bit 0: contact buffer overflowed, bit 1: non-finite state was reset */, GRS_INFO_EPISODE_STEP,
-  GRS_INFO_EPISODE_RETURN = 32 /* Monitor `r` */, GRS_INFO_EPISODE_SUBSTEPS, GRS_INFO_TARGET_QPOS = 34 /*5*/, GRS_INFO_STRIDE = 40
+  GRS_INFO_EPISODE_RETURN = 32 /* Monitor `r` */, GRS_INFO_EPISODE_SUBSTEPS, GRS_INFO_TARGET_QPOS = 34 /*5*/,
+  GRS_INFO_OBJECT = 39 /* variant (scene index) of the episode the step belongs to; a step that ends an episode reports the ended one */,
+  GRS_INFO_STRIDE = 40
 };
 /* packed per-environment state record ("state" buffer), floats */
 enum {
@@ -78,6 +80,15 @@ GRS_API void grs_default_config(grs_config* cfg);
 
 /* replaces mujoco.Physics.from_xml_path(...) + RobotEnv.__init__ (robot_env.py:24-44) for num_envs instances */
 GRS_API grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs_config* cfg, int32_t device);
+/* Mixed simulator: `count` scenes (variants 0..count-1, 1 <= count <= 8) that differ only in the object (its mesh, body and geom
+ * pose, and the world cameras' poses).  Every environment runs one variant per episode: buffer "object" int32[N] holds the
+ * variant of its current episode (read only), "next_object" int32[N] the variant its next reset starts (the caller may write it
+ * between calls; a value outside 0..count-1 keeps the current variant).  Both start as n % count.  The create call fails, naming
+ * the field and both files, when a scene differs from the first in anything the variants share (counts, body tree, joint / dof /
+ * actuator layout, named bodies, geoms and pairs, the gripper's hulls and render data, options, camera fovy, lights).
+ * grs_create(path, ...) is grs_create_scenes(&path, 1, ...).  grs_model_get* and grs_model_names answer for variant 0. */
+GRS_API grs_sim* grs_create_scenes(const char* const* xml_paths, int32_t count, int32_t num_envs, const grs_config* cfg, int32_t device);
+GRS_API int32_t grs_num_scenes(const grs_sim* sim);
 GRS_API void grs_destroy(grs_sim* sim);
 
 GRS_API int32_t grs_num_envs(const grs_sim* sim);
@@ -104,7 +115,9 @@ GRS_API int32_t grs_substep(grs_sim* sim, int32_t n, void* stream);
 
 /* named device buffers: "state" f32[N][64], "info" f32[N][40], "obs" u8[N][C][H][W], "terminal_obs" (same),
  * "reward" f32[N], "done" u8[N], "achieved" f32[N][2], "desired" f32[N][2], "render_state" f32[N][96],
- * "debug" f32[N][GRS_DEBUG_STRIDE].  Returns 0 and fills ptr/bytes, or non-zero for an unknown name. */
+ * "debug" f32[N][GRS_DEBUG_STRIDE], "reset_obs" u8[K][C][H][W] (the first observation of an episode of each variant,
+ * K = grs_num_scenes), "object" and "next_object" int32[N] (grs_create_scenes).  Returns 0 and fills ptr/bytes, or non-zero
+ * for an unknown name. */
 GRS_API int32_t grs_buffer(grs_sim* sim, const char* name, void** ptr, uint64_t* bytes);
 
 /* physics.data.qpos/qvel/ctrl/qacc_warmstart + the env flags, as host arrays [N][14],[N][13],[N][7],[N][13],[N][3]
@@ -126,7 +139,9 @@ GRS_API int32_t grs_debug_step(grs_sim* sim);
 /* compiled-model constants for compiler parity (mjModel fields). Returns the number of doubles written,
  * or the required count when out == NULL, or -1 for an unknown name.  Names: body_mass, body_ipos, body_iquat,
  * body_inertia, body_invweight0, dof_invweight0, dof_armature, dof_damping, geom_pos, geom_quat, geom_rbound,
- * geom_friction, qpos0, meaninertia, extent, hull_verts:<mesh>, body_pos, body_quat, jnt_axis, jnt_range ... */
+ * geom_friction, qpos0, meaninertia, extent, hull_verts:<mesh>, body_pos, body_quat, jnt_axis, jnt_range ...
+ * grs_model_get_int "step_smem" (not for grs_compile_only handles): the step kernel's shared memory per block in bytes,
+ * whether the hull vertices of all variants are staged there (1) or read from global memory (0), their count, warps per block. */
 GRS_API int64_t grs_model_get(const grs_sim* sim, const char* name, double* out, int64_t cap);
 GRS_API int64_t grs_model_get_int(const grs_sim* sim, const char* name, int32_t* out, int64_t cap);
 /* names of the model's bodies / geoms / joints / cameras / meshes (kind = "body" ...), '\n'-separated, NUL-terminated;

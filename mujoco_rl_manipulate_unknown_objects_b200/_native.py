@@ -23,13 +23,13 @@ class GrsConfig(C.Structure):
 INFO = dict(REWARD=0, DONE=1, STATUS=2, GRASP=3, PHEROMONE=4, OBJECT_GRASPED=5, GRIPPER_OPEN=6, REACHED_TARGET=7,
             REACHED_INITIAL=8, FAIL=9, NSUB_A=10, NSUB_B=11, NSUB_C=12, TOTAL_DISTANCE=13, LINE_DISTANCE=14,
             INIT_OBJ_POS=15, FINAL_OBJ_POS=18, GRIPPER_POS=21, ACHIEVED=24, DESIRED=26, SOLVER_ITERS=28, NCON_MAX=29,
-            FLAGS=30, EPISODE_STEP=31, EPISODE_RETURN=32, EPISODE_SUBSTEPS=33, TARGET_QPOS=34, STRIDE=40)
+            FLAGS=30, EPISODE_STEP=31, EPISODE_RETURN=32, EPISODE_SUBSTEPS=33, TARGET_QPOS=34, OBJECT=39, STRIDE=40)
 STATE_STRIDE, RENDER_STATE_STRIDE, DEBUG_STRIDE = 64, 96, 2048
 # debug-step dump layout (csrc/env_kernels.cuh DBG_*)
 DBG = dict(M=0, BIAS=169, FSMOOTH=182, ASMOOTH=195, NCON=208, NEFC=209, NLIM=210, ITERS=211, QACC=212, FCON=225, D=238,
            AREF=293, FORCE=348, J=403, CONTACT=1118, MU=1298)
 
-SYMBOLS = ["grs_last_error", "grs_default_config", "grs_create", "grs_destroy", "grs_num_envs", "grs_action_dim",
+SYMBOLS = ["grs_last_error", "grs_default_config", "grs_create", "grs_create_scenes", "grs_num_scenes", "grs_destroy", "grs_num_envs", "grs_action_dim",
            "grs_obs_shape", "grs_stream", "grs_reset", "grs_step", "grs_step_host", "grs_reset_host", "grs_substep",
            "grs_buffer", "grs_get_state", "grs_set_state", "grs_max_contacts", "grs_get_contacts", "grs_debug_step",
            "grs_model_get", "grs_model_get_int", "grs_model_names", "grs_compile_only", "grs_render", "grs_launch_count",
@@ -63,6 +63,10 @@ def load():
     L.grs_default_config.argtypes = [C.POINTER(GrsConfig)]
     L.grs_create.restype = vp
     L.grs_create.argtypes = [C.c_char_p, i32, C.POINTER(GrsConfig), i32]
+    L.grs_create_scenes.restype = vp
+    L.grs_create_scenes.argtypes = [C.POINTER(C.c_char_p), i32, i32, C.POINTER(GrsConfig), i32]
+    L.grs_num_scenes.restype = i32
+    L.grs_num_scenes.argtypes = [vp]
     L.grs_compile_only.restype = vp
     L.grs_compile_only.argtypes = [C.c_char_p]
     L.grs_destroy.argtypes = [vp]

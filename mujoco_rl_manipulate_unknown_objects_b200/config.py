@@ -14,7 +14,8 @@ DEFAULTS = dict(sim_env="/xmls/acorn_env.xml", width_capture=64, height_capture=
 
 
 def make_config(**overrides):
-    """Namespace with the reference defaults; keyword arguments override (unknown names are rejected)."""
+    """Namespace with the reference defaults; keyword arguments override (unknown names are rejected).  `sim_env` may be a list or
+    tuple of scenes: a mixed simulator whose environments each run one of them per episode (GripperSim.next_object_ids)."""
     unknown = set(overrides) - set(DEFAULTS)
     if unknown:
         raise TypeError("unknown config field(s): %s" % ", ".join(sorted(unknown)))
@@ -32,3 +33,10 @@ def scene_path(sim_env):
     if not os.path.exists(p):
         raise FileNotFoundError("scene file %r not found (looked in %s)" % (sim_env, ASSETS))
     return p
+
+
+def scene_paths(sim_env):
+    """`config.sim_env` as a list of resolved scene files: one for a string, one per entry for a list or tuple."""
+    if isinstance(sim_env, (list, tuple)):
+        return [scene_path(e) for e in sim_env]
+    return [scene_path(sim_env)]

@@ -126,4 +126,51 @@ void build_dev_model(const HostModel& h, DevModel& d, std::vector<float>& hv4, s
   }
 }
 
+std::string scene_mismatch(const HostModel& a, const HostModel& b) {
+#define SAME(f) if (!(a.f == b.f)) return #f;
+#define SAME_N(f, n) for (int i_ = 0; i_ < (n); i_++) if (!(a.f[i_] == b.f[i_])) return #f;
+  SAME(nq) SAME(nv) SAME(nu) SAME(nbody) SAME(njnt) SAME(ngeom) SAME(nmesh) SAME(npair) SAME(ncam) SAME(nlight)
+  SAME(body_parentid) SAME(body_jntadr) SAME(body_jntnum) SAME(body_dofadr) SAME(body_dofnum) SAME(body_rootid)
+  SAME(jnt_type) SAME(jnt_bodyid) SAME(jnt_qposadr) SAME(jnt_dofadr) SAME(jnt_limited)
+  SAME(dof_bodyid) SAME(dof_jntid) SAME(dof_parentid) SAME(act_dofid) SAME(act_gear) SAME(act_ctrlrange)
+  SAME(body_ee) SAME(body_object) SAME_N(finger1, 2) SAME_N(finger2, 2)
+  SAME(geom_type) SAME(geom_bodyid) SAME(geom_meshid) SAME(pair_geom1) SAME(pair_geom2)
+  SAME(geom_rgba) SAME(geom_matprop)
+  SAME(timestep) SAME(iterations) SAME(impratio) SAME(cone_elliptic) SAME_N(gravity, 3)
+  SAME(cam_names) SAME(cam_fovy)
+  SAME(light_bodyid) SAME(light_directional) SAME(light_pos) SAME(light_dir) SAME(light_diffuse) SAME(light_ambient) SAME(light_specular)
+  SAME_N(tex_rgb1, 3) SAME_N(tex_rgb2, 3) SAME_N(texrepeat, 2) SAME_N(sky_rgb1, 3) SAME_N(sky_rgb2, 3)
+#undef SAME
+#undef SAME_N
+  // the gripper's collision hulls, render triangles and plane sizes are stored once for all variants
+  for (int g = 0; g < a.ngeom; g++) {
+    if (a.geom_bodyid[g] == a.body_object) continue;
+    for (int k = 0; k < 3; k++) if (a.geom_size[3 * g + k] != b.geom_size[3 * g + k]) return "geom_size";
+    if (a.geom_meshid[g] < 0) continue;
+    const HostMesh &ma = a.meshes[a.geom_meshid[g]], &mb = b.meshes[b.geom_meshid[g]];
+    if (ma.hull_verts != mb.hull_verts) return "hull_verts:" + ma.name;
+    if (ma.adjadr != mb.adjadr || ma.adj != mb.adj) return "hull_adj:" + ma.name;
+    if (ma.tri != mb.tri) return "mesh_tri:" + ma.name;
+  }
+  return "";
+}
+
+void rebase_hull(const DevModel& d0, DevModel& d, const std::vector<float>& hv4, const std::vector<int>& adj, std::vector<float>& all_hv4,
+                 std::vector<int>& all_adj) {
+  for (int g = 0; g < d.ngeom; g++) {
+    if (d.geom_body[g] != d.body_object) {
+      d.geom_hvadr[g] = d0.geom_hvadr[g]; d.geom_adjadr[g] = d0.geom_adjadr[g];
+      continue;
+    }
+    if (d.geom_hvnum[g] == 0) continue;
+    int adj_end = (int)adj.size();  // this geom's hull-graph block ends where the next one starts
+    for (int o = 0; o < d.ngeom; o++)
+      if (d.geom_hvnum[o] > 0 && d.geom_adjadr[o] > d.geom_adjadr[g]) adj_end = std::min(adj_end, d.geom_adjadr[o]);
+    const int hv_at = (int)all_hv4.size() / 4, adj_at = (int)all_adj.size();
+    all_hv4.insert(all_hv4.end(), hv4.begin() + 4 * d.geom_hvadr[g], hv4.begin() + 4 * (d.geom_hvadr[g] + d.geom_hvnum[g]));
+    all_adj.insert(all_adj.end(), adj.begin() + d.geom_adjadr[g], adj.begin() + adj_end);
+    d.geom_hvadr[g] = hv_at; d.geom_adjadr[g] = adj_at;
+  }
+}
+
 }  // namespace grs

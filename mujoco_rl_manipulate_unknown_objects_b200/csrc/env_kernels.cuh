@@ -23,7 +23,7 @@ enum { ST_QPOS = 0, ST_QVEL = 14, ST_CTRL = 27, ST_WARM = 34, ST_GRIPPER_OPEN = 
 enum { IN_REWARD = 0, IN_DONE, IN_STATUS, IN_GRASP, IN_PHEROMONE, IN_OBJECT_GRASPED, IN_GRIPPER_OPEN, IN_REACHED_TARGET, IN_REACHED_INITIAL,
        IN_FAIL, IN_NSUB_A, IN_NSUB_B, IN_NSUB_C, IN_TOTAL_DISTANCE, IN_LINE_DISTANCE, IN_INIT_OBJ_POS, IN_FINAL_OBJ_POS = 18,
        IN_GRIPPER_POS = 21, IN_ACHIEVED = 24, IN_DESIRED = 26, IN_SOLVER_ITERS = 28, IN_NCON_MAX, IN_FLAGS, IN_EPISODE_STEP,
-       IN_EPISODE_RETURN = 32, IN_EPISODE_SUBSTEPS, IN_TARGET_QPOS = 34, IN_STRIDE = 40 };
+       IN_EPISODE_RETURN = 32, IN_EPISODE_SUBSTEPS, IN_TARGET_QPOS = 34, IN_OBJECT = 39, IN_STRIDE = 40 };
 constexpr int RS_STRIDE = 96;
 
 struct EnvFlags { int gripper_open, episode_step, status; float xfrc_z, ep_return, ep_substeps; };
@@ -102,7 +102,7 @@ __device__ __forceinline__ void euler_matrix_sxyz(float ai, float aj, float ak, 
 
 // actuator.py:21-44 (_normalise_action), :58-102 (get_target_pose), :249-293 (clip / constraints).
 // Executed by lane 0; the five target joint positions land in w.tgt.
-__device__ __noinline__ void get_target_pose(const DevModel& m, const EnvCfg& c, WS& w, const float* a6) {
+static __device__ __noinline__ void get_target_pose(const DevModel& m, const EnvCfg& c, WS& w, const float* a6) {
   float t[3] = {a6[0] * c.max_trans, a6[1] * c.max_trans, a6[2] * c.max_trans};
   float rot[2] = {a6[3] * c.max_rot, a6[4] * c.max_rot};
   float len = sqrtf(dot3(t, t));
@@ -207,7 +207,7 @@ __device__ __forceinline__ float warp_max(float v) {
 // info record (into w.out).  Called by the step kernel's controller (env_lockstep.cuh : env_tick) when an agent step ends.
 struct StepCounters { int nsa, nsb, nsc, iters, nconmax, flags, fail, object_grasped; bool reached_target, reached_initial; float tq_rec; };
 
-__device__ __noinline__ void env_finalize(const DevModel& m, const EnvCfg& c, WS& w, EnvFlags& f, const float* init_obj, StepCounters& k, int lane) {
+static __device__ __noinline__ void env_finalize(const DevModel& m, const EnvCfg& c, WS& w, EnvFlags& f, const float* init_obj, StepCounters& k, int lane) {
   int nsa = k.nsa, nsb = k.nsb, nsc = k.nsc, iters = k.iters, nconmax = k.nconmax, flags = k.flags, fail = k.fail, object_grasped = k.object_grasped;
   const bool reached_target = k.reached_target, reached_initial = k.reached_initial;
   const float tq_rec = k.tq_rec;
@@ -267,7 +267,7 @@ struct SimBuffers {
   float* achieved;      // [N][2]
   float* desired;       // [N][2]
   float* render_state;  // [N][RS_STRIDE]
-  float* reset_record;  // [ST_STRIDE] state + [IN_STRIDE] info + [RS_STRIDE] render state of a freshly reset environment
+  float* reset_record;  // [nobj][REC_STRIDE]: [ST_STRIDE] state + [IN_STRIDE] info + [RS_STRIDE] render state of a freshly reset environment
   float* debug;         // [N][DEBUG_STRIDE]
   int* queue;           // [0] work-queue counter, [1..2] bucket counters of the longest-first order, [3] finished environments,
                         // [4] observation tickets handed out, [5] blocks that left the fused kernel, [6] blocks that started,
@@ -282,9 +282,13 @@ struct SimBuffers {
   int hull_count;       // float4 entries behind `hull`; the lock-step kernel copies them to shared memory when hull_smem is set
   int hull_smem;
   const int* adj;
-  const DevModel* model;
+  const DevModel* model;  // [nobj] at MODEL_BYTES stride
   int n;
+  int nobj;
+  int* object;             // [N] variant of each environment's current episode
+  const int* next_object;  // [N] variant of its next episode (written by the caller)
 };
+constexpr int REC_STRIDE = ST_STRIDE + IN_STRIDE + RS_STRIDE;
 constexpr int DEBUG_STRIDE = 2048;
 constexpr int WARPS_PER_BLOCK = 4;
 
@@ -295,6 +299,13 @@ __host__ __device__ inline float reset_uniform(unsigned seed, unsigned env, unsi
   unsigned h = seed * 0x9E3779B1u ^ env * 0x85EBCA77u ^ episode * 0xC2B2AE3Du ^ k * 0x27D4EB2Fu;
   h ^= h >> 15; h *= 0x2C1B3C6Du; h ^= h >> 12; h *= 0x297A2D39u; h ^= h >> 15;
   return (float)(h >> 8) * (2.0f / 16777216.0f) - 1.0f;
+}
+// A reset starts the variant next_object[env] names (the current one when the value names none) and records it in object[env].
+__device__ __forceinline__ int take_next_object(const SimBuffers& s, int env) {
+  const int nv = s.next_object[env];
+  const int v = (unsigned)nv < (unsigned)s.nobj ? nv : s.object[env];
+  s.object[env] = v;
+  return v;
 }
 // `st` already holds the reset record.  Moves / turns the free object, records the pose of its geom for the observation of the
 // new episode and the achieved goal (object xy, robot_env.py:71).  One lane suffices (called by lane 0).
@@ -326,20 +337,23 @@ __device__ inline void apply_reset_noise(const SimBuffers& s, const DevModel& m,
 
 extern __shared__ __align__(16) unsigned char grs_smem[];
 
-__device__ __forceinline__ const DevModel& stage_model(const DevModel* gm) {
-  DevModel* sm = reinterpret_cast<DevModel*>(grs_smem);
-  const int nw = sizeof(DevModel) / 4;
-  const unsigned* src = reinterpret_cast<const unsigned*>(gm);
-  unsigned* dst = reinterpret_cast<unsigned*>(sm);
+// Shared-memory layout of the per-environment kernels: the models of all variants at MODEL_BYTES stride (the same layout as
+// in HBM), then one WS per warp.
+constexpr unsigned MODEL_BYTES = (sizeof(DevModel) + 15) / 16 * 16;
+__device__ __forceinline__ const DevModel& smem_model(int v) { return *reinterpret_cast<const DevModel*>(grs_smem + (unsigned)v * MODEL_BYTES); }
+__device__ __forceinline__ const DevModel& hbm_model(const SimBuffers& s, int v) {
+  return *reinterpret_cast<const DevModel*>(reinterpret_cast<const unsigned char*>(s.model) + (size_t)v * MODEL_BYTES);
+}
+template <bool MULTI>
+__device__ __forceinline__ void stage_models(const SimBuffers& s) {
+  const int nw = (MULTI ? s.nobj : 1) * (int)MODEL_BYTES / 4;
+  const unsigned* src = reinterpret_cast<const unsigned*>(s.model);
+  unsigned* dst = reinterpret_cast<unsigned*>(grs_smem);
   for (int i = threadIdx.x; i < nw; i += blockDim.x) dst[i] = src[i];
   __syncthreads();
-  return *sm;
 }
-__device__ __forceinline__ WS& my_ws() {
-  constexpr int off = (sizeof(DevModel) + 15) / 16 * 16;
-  return reinterpret_cast<WS*>(grs_smem + off)[threadIdx.x >> 5];
-}
-inline size_t smem_bytes() { return (sizeof(DevModel) + 15) / 16 * 16 + WARPS_PER_BLOCK * sizeof(WS); }
+__device__ __forceinline__ WS& my_ws(int nobj) { return reinterpret_cast<WS*>(grs_smem + (unsigned)nobj * MODEL_BYTES)[threadIdx.x >> 5]; }
+inline size_t smem_bytes(int nobj) { return (size_t)nobj * MODEL_BYTES + WARPS_PER_BLOCK * sizeof(WS); }
 
 __device__ __forceinline__ int next_env(int* queue, int lane) {
   int e = 0;
@@ -349,9 +363,12 @@ __device__ __forceinline__ int next_env(int* queue, int lane) {
 
 // RobotEnv.reset executed once (every environment starts from qpos0 — the reference has no reset randomisation):
 // mj_resetData + mj_forward with actuation disabled (dm_control Physics.reset), then the env bookkeeping of robot_env.py:62-73
+// One block per variant; block v writes the reset record of variant v.
+template <bool MULTI>
 __global__ void __launch_bounds__(32) k_make_reset_record(SimBuffers s, EnvCfg c) {
-  const DevModel& m = stage_model(s.model);
-  WS& w = my_ws();
+  stage_models<MULTI>(s);
+  const DevModel& m = smem_model(MULTI ? blockIdx.x : 0);
+  WS& w = my_ws(MULTI ? s.nobj : 1);
   const int lane = threadIdx.x & 31;
   if (lane < NQ) w.qpos[lane] = m.qpos0[lane];
   for (int k = lane; k < MAXPAIR * 3; k += 32) (&w.sep[0][0])[k] = 0.0f;
@@ -366,10 +383,11 @@ __global__ void __launch_bounds__(32) k_make_reset_record(SimBuffers s, EnvCfg c
   __syncwarp();
   EnvFlags f;
   f.gripper_open = 1; f.episode_step = 0; f.status = 0; f.xfrc_z = m.xfrc_ee_z; f.ep_return = 0; f.ep_substeps = 0;
-  for (int k = lane; k < ST_STRIDE; k += 32) s.reset_record[k] = 0;
+  float* rec = s.reset_record + (size_t)blockIdx.x * REC_STRIDE;
+  for (int k = lane; k < ST_STRIDE; k += 32) rec[k] = 0;
   __syncwarp();
-  store_state(w, f, s.reset_record, lane);
-  float* o = s.reset_record + ST_STRIDE;
+  store_state(w, f, rec, lane);
+  float* o = rec + ST_STRIDE;
   for (int k = lane; k < IN_STRIDE; k += 32) o[k] = 0;
   __syncwarp();
   if (lane == 0) {
@@ -380,33 +398,40 @@ __global__ void __launch_bounds__(32) k_make_reset_record(SimBuffers s, EnvCfg c
     o[IN_DESIRED] = c.dir[0]; o[IN_DESIRED + 1] = c.dir[1];  // robot_env.py:72 — the direction itself, not a projection
     for (int k = 0; k < 3; k++) { o[IN_FINAL_OBJ_POS + k] = w.xpos[m.body_object][k]; o[IN_GRIPPER_POS + k] = w.xpos[m.body_ee][k]; }
     o[IN_NCON_MAX] = (float)w.ncon;
+    o[IN_OBJECT] = (float)blockIdx.x;
   }
-  write_render_state(m, w, c.obs_cam, s.reset_record + ST_STRIDE + IN_STRIDE, lane);
+  write_render_state(m, w, c.obs_cam, rec + ST_STRIDE + IN_STRIDE, lane);
 }
 
-// RobotEnv.reset for the masked environments: copy the reset record
-__global__ void k_reset(SimBuffers s, EnvCfg c, const unsigned char* __restrict__ mask) {
+// RobotEnv.reset for the masked environments: take the next variant, copy its reset record
+static __global__ void k_reset(SimBuffers s, EnvCfg c, const unsigned char* __restrict__ mask) {
   const int env = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (env >= s.n) return;
   if (mask && !mask[env]) return;
-  for (int k = lane; k < ST_STRIDE; k += 32) s.state[(size_t)env * ST_STRIDE + k] = s.reset_record[k];
-  for (int k = lane; k < IN_STRIDE; k += 32) s.info[(size_t)env * IN_STRIDE + k] = s.reset_record[ST_STRIDE + k];
-  for (int k = lane; k < RS_STRIDE; k += 32) s.render_state[(size_t)env * RS_STRIDE + k] = s.reset_record[ST_STRIDE + IN_STRIDE + k];
+  int v = 0;
+  if (lane == 0) v = take_next_object(s, env);
+  v = __shfl_sync(FULL, v, 0);
+  const float* rec = s.reset_record + (size_t)v * REC_STRIDE;
+  for (int k = lane; k < ST_STRIDE; k += 32) s.state[(size_t)env * ST_STRIDE + k] = rec[k];
+  for (int k = lane; k < IN_STRIDE; k += 32) s.info[(size_t)env * IN_STRIDE + k] = rec[ST_STRIDE + k];
+  for (int k = lane; k < RS_STRIDE; k += 32) s.render_state[(size_t)env * RS_STRIDE + k] = rec[ST_STRIDE + IN_STRIDE + k];
   if (lane == 0) {
     s.reward[env] = 0; s.done[env] = 0;
-    s.achieved[2 * env] = s.reset_record[ST_STRIDE + IN_ACHIEVED]; s.achieved[2 * env + 1] = s.reset_record[ST_STRIDE + IN_ACHIEVED + 1];
-    s.desired[2 * env] = s.reset_record[ST_STRIDE + IN_DESIRED]; s.desired[2 * env + 1] = s.reset_record[ST_STRIDE + IN_DESIRED + 1];
+    s.achieved[2 * env] = rec[ST_STRIDE + IN_ACHIEVED]; s.achieved[2 * env + 1] = rec[ST_STRIDE + IN_ACHIEVED + 1];
+    s.desired[2 * env] = rec[ST_STRIDE + IN_DESIRED]; s.desired[2 * env + 1] = rec[ST_STRIDE + IN_DESIRED + 1];
   }
   __syncwarp();
-  if (lane == 0 && (c.reset_noise_xy != 0.f || c.reset_noise_yaw != 0.f)) apply_reset_noise(s, *s.model, c, env, s.state + (size_t)env * ST_STRIDE);
+  if (lane == 0 && (c.reset_noise_xy != 0.f || c.reset_noise_yaw != 0.f)) apply_reset_noise(s, hbm_model(s, v), c, env, s.state + (size_t)env * ST_STRIDE);
 }
 
 // n x physics.step() with the controls held in the state (parity tests; robot_env.py:100)
+template <bool MULTI>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 5) k_substep(SimBuffers s, int nsteps) {
-  const DevModel& m = stage_model(s.model);
-  WS& w = my_ws();
+  stage_models<MULTI>(s);
+  WS& w = my_ws(MULTI ? s.nobj : 1);
   const int lane = threadIdx.x & 31;
   for (int env = next_env(s.queue, lane); env < s.n; env = next_env(s.queue, lane)) {
+    const DevModel& m = smem_model(MULTI ? s.object[env] : 0);
     EnvFlags f;
     float* st = s.state + (size_t)env * ST_STRIDE;
     load_state(w, f, st, lane);
@@ -418,11 +443,13 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 5) k_substep(SimBuffers 
 }
 
 // contacts of the current state -> debug buffer: [0] ncon, then per contact K: g1, g2, dist, pos[3], frame[9]  (stride 15)
+template <bool MULTI>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32) k_contacts(SimBuffers s) {
-  const DevModel& m = stage_model(s.model);
-  WS& w = my_ws();
+  stage_models<MULTI>(s);
+  WS& w = my_ws(MULTI ? s.nobj : 1);
   const int lane = threadIdx.x & 31;
   for (int env = next_env(s.queue, lane); env < s.n; env = next_env(s.queue, lane)) {
+    const DevModel& m = smem_model(MULTI ? s.object[env] : 0);
     EnvFlags f;
     load_state(w, f, s.state + (size_t)env * ST_STRIDE, lane);
     forward_position(m, w, s.hull, s.adj, lane);
@@ -444,11 +471,13 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32) k_contacts(SimBuffers s)
 // one physics.step() with a dump of the intermediate quantities (layout documented in python/_debug_layout)
 enum { DBG_M = 0, DBG_BIAS = 169, DBG_FSMOOTH = 182, DBG_ASMOOTH = 195, DBG_NCON = 208, DBG_NEFC = 209, DBG_NLIM = 210, DBG_ITERS = 211,
        DBG_QACC = 212, DBG_FCON = 225, DBG_D = 238, DBG_AREF = 293, DBG_FORCE = 348, DBG_J = 403, DBG_CONTACT = 1118 /* 12 x 15 */, DBG_MU = 1298, DBG_END = 1310 };
+template <bool MULTI>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32) k_debug_step(SimBuffers s) {
-  const DevModel& m = stage_model(s.model);
-  WS& w = my_ws();
+  stage_models<MULTI>(s);
+  WS& w = my_ws(MULTI ? s.nobj : 1);
   const int lane = threadIdx.x & 31;
   for (int env = next_env(s.queue, lane); env < s.n; env = next_env(s.queue, lane)) {
+    const DevModel& m = smem_model(MULTI ? s.object[env] : 0);
     EnvFlags f;
     float* st = s.state + (size_t)env * ST_STRIDE;
     load_state(w, f, st, lane);

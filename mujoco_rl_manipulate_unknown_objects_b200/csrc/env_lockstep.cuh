@@ -36,7 +36,7 @@ __device__ __forceinline__ void ctl_stats(EnvCtl& t, const WS& w, int iters) {
 // Advances the controller state machine of one environment up to the next physics substep.
 // Returns true when a substep has to be integrated this round (controls are set), false when the agent step is complete
 // (w.out holds the info record, t.f the updated flags).  `solver_iters` = Newton iterations of the substep just taken.
-__device__ __noinline__ bool env_tick(const DevModel& m, const EnvCfg& c, WS& w, EnvCtl& t, const float* __restrict__ act, int solver_iters, int lane) {
+static __device__ __noinline__ bool env_tick(const DevModel& m, const EnvCfg& c, WS& w, EnvCtl& t, const float* __restrict__ act, int solver_iters, int lane) {
   const float scale = lane < 3 ? 1.0f / c.max_trans : 1.0f / c.max_rot;
 #pragma unroll 1
   for (;;) {
@@ -163,11 +163,14 @@ __device__ __noinline__ bool env_tick(const DevModel& m, const EnvCfg& c, WS& w,
   }
 }
 
-// results of a finished agent step -> HBM (+ SB3 auto-reset)
-__device__ __noinline__ void env_writeback(const DevModel& m, const EnvCfg& c, const SimBuffers& s, WS& w, EnvCtl& t, int lane) {
+// results of a finished agent step -> HBM (+ SB3 auto-reset, which starts the variant next_object names)
+static __device__ __noinline__ void env_writeback(const DevModel& m, const EnvCfg& c, const SimBuffers& s, WS& w, EnvCtl& t, int lane) {
   const int env = t.env;
   float* st = s.state + (size_t)env * ST_STRIDE;
-  for (int k = lane; k < IN_STRIDE; k += 32) s.info[(size_t)env * IN_STRIDE + k] = w.out[k];
+  int vo = 0;
+  if (lane == 0) vo = s.object[env];  // lane 0 alone reads and (below) writes object[env]
+  const float v_step = (float)__shfl_sync(FULL, vo, 0);  // IN_OBJECT: the variant of the episode this step belongs to
+  for (int k = lane; k < IN_STRIDE; k += 32) s.info[(size_t)env * IN_STRIDE + k] = k == IN_OBJECT ? v_step : w.out[k];
   write_render_state(m, w, c.obs_cam, s.render_state + (size_t)env * RS_STRIDE, lane);
   const int done = (int)w.out[IN_DONE];
   if (lane == 0) {
@@ -177,12 +180,16 @@ __device__ __noinline__ void env_writeback(const DevModel& m, const EnvCfg& c, c
     s.desired[2 * env] = w.out[IN_DESIRED]; s.desired[2 * env + 1] = w.out[IN_DESIRED + 1];
   }
   if (done && c.auto_reset) {
-    for (int k = lane; k < ST_STRIDE; k += 32) st[k] = s.reset_record[k];
+    int v = 0;
+    if (lane == 0) v = take_next_object(s, env);
+    v = __shfl_sync(FULL, v, 0);
+    const float* rec = s.reset_record + (size_t)v * REC_STRIDE;
+    for (int k = lane; k < ST_STRIDE; k += 32) st[k] = rec[k];
     __syncwarp();
     if (lane == 0) {
-      s.achieved[2 * env] = s.reset_record[ST_STRIDE + IN_ACHIEVED]; s.achieved[2 * env + 1] = s.reset_record[ST_STRIDE + IN_ACHIEVED + 1];
-      s.desired[2 * env] = s.reset_record[ST_STRIDE + IN_DESIRED]; s.desired[2 * env + 1] = s.reset_record[ST_STRIDE + IN_DESIRED + 1];
-      if (c.reset_noise_xy != 0.f || c.reset_noise_yaw != 0.f) apply_reset_noise(s, m, c, env, st);
+      s.achieved[2 * env] = rec[ST_STRIDE + IN_ACHIEVED]; s.achieved[2 * env + 1] = rec[ST_STRIDE + IN_ACHIEVED + 1];
+      s.desired[2 * env] = rec[ST_STRIDE + IN_DESIRED]; s.desired[2 * env + 1] = rec[ST_STRIDE + IN_DESIRED + 1];
+      if (c.reset_noise_xy != 0.f || c.reset_noise_yaw != 0.f) apply_reset_noise(s, smem_model(v), c, env, st);
     }
   } else {
     store_state(w, t.f, st, lane);
@@ -215,12 +222,12 @@ __device__ __forceinline__ int order_class(const SimBuffers& s, const float* __r
   const int ncon = (int)s.info[(size_t)env * IN_STRIDE + IN_NCON_MAX];
   return len * ORDER_BUCKETS + (ORDER_BUCKETS - 1 - min(max(ncon, 0), ORDER_BUCKETS - 1));  // most contacts first
 }
-__global__ void k_order_count(SimBuffers s, const float* __restrict__ actions, int adim) {
+static __global__ void k_order_count(SimBuffers s, const float* __restrict__ actions, int adim) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= s.n) return;
   atomicAdd(s.queue + 16 + order_class(s, actions, adim, env), 1);
 }
-__global__ void k_order_envs(SimBuffers s, const float* __restrict__ actions, int adim) {
+static __global__ void k_order_envs(SimBuffers s, const float* __restrict__ actions, int adim) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= s.n) return;
   const int c = order_class(s, actions, adim, env);
@@ -302,7 +309,10 @@ __device__ __forceinline__ void resume_env(const AsyncArgs& aa, WS& w, EnvCtl& t
 // FUSED = true: a block whose physics work is exhausted goes on to build observations (render_phase) instead of exiting, so
 // the rasteriser fills the SMs that idle while the longest substep chains finish.  Needs blockDim.x == RTHREADS.
 // ASYNC = true: the asynchronous step above (not FUSED: the observation phase would wait for environments that get parked).
-template <bool TIMING, bool FUSED, bool ASYNC = false>
+// MULTI = true: a mixed simulator (SimBuffers::nobj > 1); each warp runs the model of its environment's variant.  The
+// single-scene instantiation keeps the model at a constant shared-memory address; the MULTI ones are compiled in
+// multi_kernels.cu only (see SimKernels below).
+template <bool TIMING, bool FUSED, bool ASYNC = false, bool MULTI = false>
 __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(SimBuffers s, EnvCfg c, const float* __restrict__ actions, int adim, RenderScene sc, ObsArgs oa,
                                                                                   AsyncArgs aa) {
   static_assert(!(ASYNC && (FUSED || TIMING)), "the asynchronous step has its own instantiation");
@@ -313,15 +323,15 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
     asm("mov.u32 %0, %%smid;" : "=r"(smid));
     atomicAdd(s.sm_phys + (smid & 255), 1);
   }
-  // Block staging by the TMA engine: the compiled model (2.3 KB) and, when they fit beside two blocks' workspaces, the convex-hull
-  // vertices of every geom (<= 18.7 KB; the support scans of the collision stage then cost shared-memory latency instead of
-  // L1/L2 round trips, which were half of that stage's stall samples) arrive as two bulk asynchronous copies (cp.async.bulk,
-  // 1-D) that complete on one mbarrier; no thread touches the bytes on their way in.
+  // Block staging by the TMA engine: the compiled models of every variant (3.8 KB each) and, when they fit beside two blocks'
+  // workspaces, the convex-hull vertices of every geom (<= 18.7 KB for one scene; the support scans of the collision stage then
+  // cost shared-memory latency instead of L1/L2 round trips, which were half of that stage's stall samples) arrive as two bulk
+  // asynchronous copies (cp.async.bulk, 1-D) that complete on one mbarrier; no thread touches the bytes on their way in.
   __shared__ unsigned long long stage_bar;
   const float4* hull = s.hull;
   {
     const unsigned bar = (unsigned)__cvta_generic_to_shared(&stage_bar);
-    constexpr unsigned model_bytes = (sizeof(DevModel) + 15) / 16 * 16;
+    const unsigned model_bytes = (MULTI ? (unsigned)s.nobj : 1u) * MODEL_BYTES;
     const unsigned hull_off = model_bytes + (unsigned)(blockDim.x >> 5) * (unsigned)sizeof(WS), hull_bytes = s.hull_smem ? (unsigned)s.hull_count * 16u : 0u;
     if (threadIdx.x == 0) {
       asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar) : "memory");
@@ -339,8 +349,8 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
       asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(done) : "r"(bar) : "memory");
     if (s.hull_smem) hull = reinterpret_cast<const float4*>(grs_smem + hull_off);
   }
-  const DevModel& m = *reinterpret_cast<const DevModel*>(grs_smem);
-  WS& w = my_ws();
+  const DevModel* mp = &smem_model(0);  // the model of the warp's current environment (its variant, set when it is loaded)
+  WS& w = my_ws(MULTI ? s.nobj : 1);
   const int lane = threadIdx.x & 31;
   __shared__ unsigned long long t_sum[8], t_max[8], t_round[8];
   __shared__ unsigned long long t_rounds, t_lone[8], t_lone_rounds;  // rounds in which exactly one warp of the block was active
@@ -379,9 +389,9 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
     }
     if (t.stage == S_LOADED) t.stage = S_BEGIN;
     if (t.stage != S_IDLE && !dyn) {
-      dyn = env_tick(m, c, w, t, actions + (size_t)t.env * adim, iters, lane);
+      dyn = env_tick(*mp, c, w, t, actions + (size_t)t.env * adim, iters, lane);
       if (!dyn) {
-        env_writeback(m, c, s, w, t, lane);
+        env_writeback(*mp, c, s, w, t, lane);
       } else if (stop) {
         park_env(s, aa, w, t, lane);
         t.stage = S_IDLE;
@@ -397,6 +407,7 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
       if (slot < (ASYNC ? __ldg(aa.ctl + AC_NQUEUE) : s.n)) {
         const int env = __ldg(s.order + slot);
         t.env = env;
+        if constexpr (MULTI) mp = &smem_model(s.object[env]);
         load_state(w, t.f, s.state + (size_t)env * ST_STRIDE, lane);
         t.stage = S_LOADED;
         if constexpr (ASYNC) {
@@ -427,6 +438,7 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
       if (prev_active == 1) t_lone_rounds++;
     }
     prev_active = n_active;
+    const DevModel& m = *mp;
     // ---- the substep pipeline, stage by stage, whole block in step (dm_control legacy step: mj_step2 then mj_step1)
     LS_T0();
     if (dyn) smooth_forces(m, w, lane, true, t.f.xfrc_z);
@@ -496,14 +508,14 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
 // ---- the small kernels around the asynchronous step (grs_async_* in gripper_sim.cu)
 
 // every environment ready with its current outputs, in id order
-__global__ void k_async_begin(AsyncArgs aa, int* __restrict__ ring, int n) {
+static __global__ void k_async_begin(AsyncArgs aa, int* __restrict__ ring, int n) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env < n) { aa.astate[env] = A_READY; aa.waited[env] = 0; ring[env] = env; }
   if (env < AC_WORDS) aa.ctl[env] = env == AC_READY ? n : 0;
 }
 
 // send: each listed environment must be returned; its action row is written and it becomes pending
-__global__ void k_async_send(AsyncArgs aa, float* __restrict__ actions, int adim, const float* __restrict__ src, const int* __restrict__ ids, int cnt, int n) {
+static __global__ void k_async_send(AsyncArgs aa, float* __restrict__ actions, int adim, const float* __restrict__ src, const int* __restrict__ ids, int cnt, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= cnt) return;
   const int env = ids[i];
@@ -523,13 +535,13 @@ __device__ __forceinline__ int async_class(const SimBuffers& s, const AsyncArgs&
   if (aa.ctl[AC_READY] >= batch || (st != A_PARKED && st != A_PENDING)) return -1;
   return st == A_PARKED ? 0 : aa.waited[env] ? 1 : 2 + order_class(s, actions, adim, env);
 }
-__global__ void k_async_order_count(SimBuffers s, AsyncArgs aa, const float* __restrict__ actions, int adim, int batch) {
+static __global__ void k_async_order_count(SimBuffers s, AsyncArgs aa, const float* __restrict__ actions, int adim, int batch) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= s.n) return;
   const int c = async_class(s, aa, actions, adim, env, batch);
   if (c >= 0) atomicAdd(aa.ctl + AC_SIZES + c, 1);
 }
-__global__ void k_async_order_envs(SimBuffers s, AsyncArgs aa, const float* __restrict__ actions, int adim, int batch) {
+static __global__ void k_async_order_envs(SimBuffers s, AsyncArgs aa, const float* __restrict__ actions, int adim, int batch) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env == 0) {
     int q = 0;
@@ -548,7 +560,7 @@ __global__ void k_async_order_envs(SimBuffers s, AsyncArgs aa, const float* __re
 
 // after the step kernel and the observations: the environments this launch finished (s.done_list[0 .. s.queue[3]), in the
 // order they finished) join the ready ring; the first `batch` of the ring are returned.  One block.
-__global__ void k_async_recv(SimBuffers s, AsyncArgs aa, int* __restrict__ ring, int* __restrict__ out_ids, int batch) {
+static __global__ void k_async_recv(SimBuffers s, AsyncArgs aa, int* __restrict__ ring, int* __restrict__ out_ids, int batch) {
   const int n = s.n, fin = s.queue[3], head = aa.ctl[AC_HEAD], ready = aa.ctl[AC_READY];  // head < n, ready + fin <= n
   for (int i = threadIdx.x; i < fin; i += blockDim.x) {
     const int env = s.done_list[i];
@@ -568,5 +580,27 @@ __global__ void k_async_recv(SimBuffers s, AsyncArgs aa, int* __restrict__ ring,
     if (take < batch) aa.ctl[AC_ERR] |= AERR_RECV_SHORT;
   }
 }
+
+// ---- host: the kernels one simulator launches.  The mixed-simulator instantiations (MULTI = true) are compiled in their own
+// translation unit (multi_kernels.cu): there the stage functions (collision, kinematics, the solver, ...) receive a model address
+// that varies per warp.  In this one every caller passes the block's single model at its constant shared-memory address, so the
+// compiler specialises the noinline stage functions to it; a second, per-warp caller in the same module undoes that and the
+// single-scene step kernel's narrowphase callees spill (DESIGN.md §3.6).
+using StepKernel = void (*)(SimBuffers, EnvCfg, const float*, int, RenderScene, ObsArgs, AsyncArgs);
+struct SimKernels {
+  StepKernel step, step_fused, step_timing, step_async;
+  void (*make_reset_record)(SimBuffers, EnvCfg);
+  void (*substep)(SimBuffers, int);
+  void (*contacts)(SimBuffers);
+  void (*debug_step)(SimBuffers);
+  void (*camera_state)(SimBuffers, int);
+};
+template <bool MULTI>
+inline SimKernels sim_kernels() {
+  return SimKernels{k_env_step_ls<false, false, false, MULTI>, k_env_step_ls<false, true, false, MULTI>, k_env_step_ls<true, false, false, MULTI>,
+                    k_env_step_ls<false, false, true, MULTI>, k_make_reset_record<MULTI>, k_substep<MULTI>, k_contacts<MULTI>, k_debug_step<MULTI>,
+                    k_camera_state<MULTI>};
+}
+SimKernels multi_sim_kernels();  // sim_kernels<true>(), multi_kernels.cu
 
 }  // namespace grs

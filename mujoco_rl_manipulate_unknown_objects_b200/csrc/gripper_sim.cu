@@ -26,7 +26,8 @@ using namespace grs;
 
 static_assert(GRS_INFO_STRIDE == IN_STRIDE && GRS_STATE_STRIDE == ST_STRIDE && GRS_DEBUG_STRIDE == DEBUG_STRIDE && GRS_RENDER_STATE_STRIDE == RS_STRIDE,
               "header / kernel record layouts diverged");
-static_assert(GRS_ST_XFRC_Z == ST_XFRC_Z && GRS_INFO_TARGET_QPOS == IN_TARGET_QPOS && GRS_INFO_EPISODE_RETURN == IN_EPISODE_RETURN, "record layouts diverged");
+static_assert(GRS_ST_XFRC_Z == ST_XFRC_Z && GRS_INFO_TARGET_QPOS == IN_TARGET_QPOS && GRS_INFO_EPISODE_RETURN == IN_EPISODE_RETURN && GRS_INFO_OBJECT == IN_OBJECT,
+              "record layouts diverged");
 
 static thread_local std::string g_err;
 static int fail(const std::string& msg) { g_err = msg; return 1; }
@@ -52,7 +53,8 @@ static void raise_dyn_smem(const void* func, size_t bytes, int device) {
 }
 
 struct grs_sim {
-  HostModel hm;
+  HostModel hm;  // variant 0: what grs_model_get* answer for
+  std::vector<std::string> scenes;  // scene file of each variant
   bool compile_only = false;
   int n = 0, device = 0, C = 5, H = 64, W = 64, adim = 6;
   grs_config cfg{};
@@ -82,6 +84,7 @@ struct grs_sim {
   bool ls_timing = false;
   bool fused_render = false;  // observation phase inside the step kernel (env_lockstep.cuh : render_phase)
   size_t ls_smem = 0;
+  SimKernels kern{};  // single-scene or mixed-simulator instantiations (env_lockstep.cuh)
   ObsArgs obs_args{};
   // asynchronous step (grs_async_*): per-environment states, control words, park records, ready ring
   bool async_on = false;
@@ -128,9 +131,16 @@ static void harvest_events(grs_sim* s) {
 
 static void launch_queue_kernel_prep(grs_sim* s, cudaStream_t st) { CU(cudaMemsetAsync(s->b.queue, 0, 64 * sizeof(int), st)); }
 
+
 extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs_config* cfg_in, int32_t device) {
+  return grs_create_scenes(&xml_path, 1, num_envs, cfg_in, device);
+}
+
+extern "C" grs_sim* grs_create_scenes(const char* const* xml_paths, int32_t count, int32_t num_envs, const grs_config* cfg_in, int32_t device) {
   grs_sim* raw = nullptr;
   try {
+    if (count < 1 || count > MAXOBJ) throw std::runtime_error("a simulator holds 1.." + std::to_string(MAXOBJ) + " scenes (got " + std::to_string(count) + ")");
+    if (!xml_paths) throw std::runtime_error("xml_paths is null");
     if (num_envs <= 0) throw std::runtime_error("num_envs must be positive");
     grs_config cfg;
     if (cfg_in) cfg = *cfg_in; else grs_default_config(&cfg);
@@ -143,24 +153,42 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     if (device < 0 || device >= ndev) throw std::runtime_error("invalid CUDA device index");
     auto s = std::make_unique<grs_sim>();
     raw = s.get();
-    s->hm = compile_mjcf(xml_path ? xml_path : "");
+    // every variant is compiled on its own; they must agree on everything the simulator stores once (scene_mismatch)
+    std::vector<HostModel> hms;
+    for (int v = 0; v < count; v++) {
+      s->scenes.push_back(xml_paths[v] ? xml_paths[v] : "");
+      hms.push_back(compile_mjcf(s->scenes[v]));
+      const std::string f = v ? scene_mismatch(hms[0], hms[v]) : "";
+      if (!f.empty()) throw std::runtime_error("scene " + s->scenes[v] + " cannot share a simulator with " + s->scenes[0] + ": " + f + " differs");
+    }
+    s->hm = hms[0];
+    const int K = count;
     s->n = num_envs; s->device = device; s->cfg = cfg;
     s->C = cfg.full_observation ? 5 : 4; s->H = cfg.height; s->W = cfg.width; s->adim = cfg.include_roll ? 6 : 5;
     CU(cudaSetDevice(device));
     CU(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
-    DevModel dm;
+    // one DevModel per variant, MODEL_BYTES apart (the step kernel bulk-copies them in 16-byte units); variant 0's hulls first, then
+    // the object hull of every other variant
     std::vector<float> hv;
     std::vector<int> adj;
-    build_dev_model(s->hm, dm, hv, adj);
-    s->d_model = (DevModel*)dalloc<unsigned char>(s.get(), (sizeof(DevModel) + 15) / 16 * 16);  // the step kernel bulk-copies it in 16-byte units
-    CU(cudaMemcpy(s->d_model, &dm, sizeof dm, cudaMemcpyHostToDevice));
+    std::vector<unsigned char> models((size_t)K * MODEL_BYTES, 0);
+    for (int v = 0; v < K; v++) {
+      DevModel dm;
+      std::vector<float> hv_v;
+      std::vector<int> adj_v;
+      build_dev_model(hms[v], dm, v ? hv_v : hv, v ? adj_v : adj);
+      if (v) rebase_hull(*reinterpret_cast<const DevModel*>(models.data()), dm, hv_v, adj_v, hv, adj);
+      std::memcpy(models.data() + (size_t)v * MODEL_BYTES, &dm, sizeof dm);
+    }
+    s->d_model = (DevModel*)dalloc<unsigned char>(s.get(), models.size());
+    CU(cudaMemcpy(s->d_model, models.data(), models.size(), cudaMemcpyHostToDevice));
     s->d_hull = dalloc<float4>(s.get(), hv.size() / 4 + 1);
     CU(cudaMemcpy(s->d_hull, hv.data(), hv.size() * sizeof(float), cudaMemcpyHostToDevice));
     s->d_adj = dalloc<int>(s.get(), adj.size() + 1);
     CU(cudaMemcpy(s->d_adj, adj.data(), adj.size() * sizeof(int), cudaMemcpyHostToDevice));
     const size_t N = num_envs;
     SimBuffers& b = s->b;
-    b.n = num_envs; b.model = s->d_model; b.hull = s->d_hull; b.adj = s->d_adj;
+    b.n = num_envs; b.model = s->d_model; b.hull = s->d_hull; b.adj = s->d_adj; b.nobj = K;
     b.hull_count = (int)(hv.size() / 4); b.hull_smem = 0;
     b.state = dalloc<float>(s.get(), N * ST_STRIDE);
     b.info = dalloc<float>(s.get(), N * IN_STRIDE);
@@ -169,7 +197,17 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     b.achieved = dalloc<float>(s.get(), N * 2);
     b.desired = dalloc<float>(s.get(), N * 2);
     b.render_state = dalloc<float>(s.get(), N * RS_STRIDE);
-    b.reset_record = dalloc<float>(s.get(), ST_STRIDE + IN_STRIDE + RS_STRIDE);
+    b.reset_record = dalloc<float>(s.get(), (size_t)K * REC_STRIDE);
+    {
+      // both start as n % K; the first grs_reset below copies next_object into object
+      std::vector<int> first(N);
+      for (size_t e = 0; e < N; e++) first[e] = (int)(e % K);
+      int* next = dalloc<int>(s.get(), N);
+      CU(cudaMemcpy(next, first.data(), N * sizeof(int), cudaMemcpyHostToDevice));
+      b.next_object = next;
+      b.object = dalloc<int>(s.get(), N);
+      CU(cudaMemcpy(b.object, first.data(), N * sizeof(int), cudaMemcpyHostToDevice));
+    }
     b.debug = dalloc<float>(s.get(), N * DEBUG_STRIDE);
     b.queue = dalloc<int>(s.get(), 64);
     b.done_list = dalloc<int>(s.get(), N);
@@ -182,9 +220,9 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     const size_t obs_bytes = (size_t)s->C * s->H * s->W;
     s->d_obs = dalloc<unsigned char>(s.get(), N * obs_bytes);
     s->d_terminal_obs = dalloc<unsigned char>(s.get(), N * obs_bytes);
-    s->d_reset_obs = dalloc<unsigned char>(s.get(), obs_bytes);
+    s->d_reset_obs = dalloc<unsigned char>(s.get(), K * obs_bytes);
     s->d_actions = dalloc<float>(s.get(), N * 6);
-    s->d_hist = dalloc<float>(s.get(), N * 512 + 512);
+    s->d_hist = dalloc<float>(s.get(), (N + K) * 512);
     s->aa.astate = dalloc<int>(s.get(), N);
     s->aa.ctl = dalloc<int>(s.get(), AC_WORDS);
     s->aa.park = dalloc<float>(s.get(), N * PK_STRIDE);
@@ -206,20 +244,30 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     e.pos_tol = cfg.pos_tolerance; e.grasp_tol = cfg.grasp_tolerance; e.max_trans = cfg.max_translation; e.max_rot = cfg.max_rotation;
     // launch geometry of the per-environment kernels (k_substep, k_contacts, k_debug_step, k_camera_state): persistent blocks,
     // as many as fit (one WS per warp in shared memory)
-    s->smem = smem_bytes();
-    raise_dyn_smem((const void*)k_substep, s->smem, device);
-    raise_dyn_smem((const void*)k_contacts, s->smem, device);
-    raise_dyn_smem((const void*)k_debug_step, s->smem, device);
-    raise_dyn_smem((const void*)k_make_reset_record, s->smem, device);
+    s->kern = K > 1 ? multi_sim_kernels() : sim_kernels<false>();
+    const SimKernels& kn = s->kern;
+    s->smem = smem_bytes(K);
+    raise_dyn_smem((const void*)kn.substep, s->smem, device);
+    raise_dyn_smem((const void*)kn.contacts, s->smem, device);
+    raise_dyn_smem((const void*)kn.debug_step, s->smem, device);
+    raise_dyn_smem((const void*)kn.make_reset_record, s->smem, device);
+    raise_dyn_smem((const void*)kn.camera_state, s->smem, device);  // above the 48 KB default with several models
     int per_sm = 0, nsm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_substep, WARPS_PER_BLOCK * 32, s->smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kn.substep, WARPS_PER_BLOCK * 32, s->smem));
     CU(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
     if (per_sm < 1) throw std::runtime_error("substep kernel does not fit on this device");
     int want = (num_envs + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
     s->grid = std::min(want, per_sm * nsm);
     // step kernel geometry
     if (const char* e = getenv("GRS_STEP_WARPS")) s->ls_warps = std::max(1, std::min(LS_MAX_THREADS / 32, atoi(e)));
-    s->ls_smem = (sizeof(DevModel) + 15) / 16 * 16 + (size_t)s->ls_warps * sizeof(WS);
+    s->ls_smem = (size_t)K * MODEL_BYTES + (size_t)s->ls_warps * sizeof(WS);
+    {
+      int optin = 0;
+      CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+      if (s->ls_smem > (size_t)optin)
+        throw std::runtime_error(std::to_string(K) + " models and " + std::to_string(s->ls_warps) + " workspaces need " + std::to_string(s->ls_smem) +
+                                 " bytes of shared memory per block, more than the device's " + std::to_string(optin));
+    }
     {
       // hull vertices in shared memory when two blocks per SM still fit (227 KB per block, 228 KB per SM, 1 KB reserved each)
       const size_t with_hull = s->ls_smem + (size_t)s->b.hull_count * sizeof(float4);
@@ -230,45 +278,48 @@ extern "C" grs_sim* grs_create(const char* xml_path, int32_t num_envs, const grs
     // the observation phase needs RTHREADS-wide blocks and the observation tile in the block's shared memory
     s->fused_render = !s->ls_timing && s->ls_warps * 32 == RTHREADS && s->ls_smem >= render_phase_smem_bytes() && cfg.width <= TILE && cfg.height <= TILE;
     if (const char* e = getenv("GRS_FUSED_RENDER")) s->fused_render = s->fused_render && atoi(e) != 0;
-    raise_dyn_smem((const void*)k_env_step_ls<false, false>, s->ls_smem, device);
-    raise_dyn_smem((const void*)k_env_step_ls<false, true>, s->ls_smem, device);
-    raise_dyn_smem((const void*)k_env_step_ls<true, false>, s->ls_smem, device);
-    raise_dyn_smem((const void*)k_env_step_ls<false, false, true>, s->ls_smem, device);
+    raise_dyn_smem((const void*)kn.step, s->ls_smem, device);
+    raise_dyn_smem((const void*)kn.step_fused, s->ls_smem, device);
+    raise_dyn_smem((const void*)kn.step_timing, s->ls_smem, device);
+    raise_dyn_smem((const void*)kn.step_async, s->ls_smem, device);
     int ls_per_sm = 0;
-    if (s->fused_render) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, true>, s->ls_warps * 32, s->ls_smem));
-    else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, k_env_step_ls<false, false>, s->ls_warps * 32, s->ls_smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, s->fused_render ? kn.step_fused : kn.step, s->ls_warps * 32, s->ls_smem));
     if (ls_per_sm < 1) throw std::runtime_error("step kernel does not fit on this device");
     s->ls_grid = std::min((num_envs + s->ls_warps - 1) / s->ls_warps, ls_per_sm * nsm);
     for (int i = 0; i < grs_sim::NEV; i++) { CU(cudaEventCreate(&s->ev0[i])); CU(cudaEventCreate(&s->ev1[i])); }
-    render_scene_upload(s->hm, s->scene, s->owned);
-    // the reset record and the observation of a freshly reset environment (identical for every env and every episode)
-    k_make_reset_record<<<1, 32, s->smem, s->stream>>>(s->b, s->ecfg);
+    render_scene_upload(hms, s->scene, s->owned);
+    // the reset record and the observation of a freshly reset environment of each variant (identical for every env and every episode)
+    kn.make_reset_record<<<K, 32, s->smem, s->stream>>>(s->b, s->ecfg);
     CU(cudaGetLastError());
     s->launches++;
     ObsArgs& oa = s->obs_args;
     oa.obs = s->d_obs; oa.terminal_obs = s->d_terminal_obs; oa.reset_obs = s->d_reset_obs; oa.hist_prev = s->d_hist; oa.hist_reset = s->d_hist + N * 512;
+    oa.object = s->b.object;
     oa.C = s->C; oa.H = s->H; oa.W = s->W; oa.fovy = (float)s->hm.cam_fovy[e.obs_cam]; oa.auto_reset = e.auto_reset; oa.im_reward = e.im_reward;
     oa.obs_host = nullptr; oa.terminal_obs_host = nullptr;
     oa.info = s->b.info; oa.state = s->b.state; oa.info_stride = IN_STRIDE; oa.state_stride = ST_STRIDE;
     oa.in_reward = IN_REWARD; oa.in_ep_return = IN_EPISODE_RETURN; oa.st_ep_return = ST_EP_RETURN;
-    {
+    for (int v = 0; v < K; v++) {
       ObsArgs r = oa;  // the reset image: one environment, no previous histograms (they go to hist_reset), no reward
-      r.obs = s->d_reset_obs; r.terminal_obs = nullptr; r.reset_obs = nullptr; r.hist_prev = nullptr; r.auto_reset = 0; r.im_reward = 0;
-      r.info = nullptr; r.state = nullptr;
-      launch_render_obs(s->scene, r, s->b.reset_record + ST_STRIDE + IN_STRIDE, s->b.reset_record + ST_STRIDE, nullptr, nullptr, 1, s->stream);
+      r.obs = s->d_reset_obs + v * obs_bytes; r.terminal_obs = nullptr; r.reset_obs = nullptr; r.hist_prev = nullptr; r.hist_reset = oa.hist_reset + v * 512;
+      r.auto_reset = 0; r.im_reward = 0; r.info = nullptr; r.state = nullptr;
+      const float* rec = s->b.reset_record + (size_t)v * REC_STRIDE;
+      launch_render_obs(s->scene, r, rec + ST_STRIDE + IN_STRIDE, rec + ST_STRIDE, nullptr, nullptr, 1, s->stream);
+      s->launches++;
     }
-    s->launches++;
     CU(cudaStreamSynchronize(s->stream));
     {
       // reset randomisation: the new episode's observation is rendered per environment (object geom at its own pose)
-      float rinfo[IN_STRIDE];
-      CU(cudaMemcpy(rinfo, s->b.reset_record + ST_STRIDE, sizeof rinfo, cudaMemcpyDeviceToHost));
+      std::vector<float> rec((size_t)K * REC_STRIDE);
+      CU(cudaMemcpy(rec.data(), s->b.reset_record, rec.size() * sizeof(float), cudaMemcpyDeviceToHost));
       oa.reset_noise = (e.reset_noise_xy != 0.f || e.reset_noise_yaw != 0.f) ? 1 : 0;
-      oa.obj_geom = 0;
-      for (int g = 0; g < s->hm.ngeom; g++) if (s->hm.geom_bodyid[g] == s->hm.body_object) { oa.obj_geom = g; break; }
+      oa.obj_geom = s->scene.obj_geom;
       oa.reset_rs = s->b.reset_record + ST_STRIDE + IN_STRIDE;
       oa.reset_obj = s->b.reset_obj;
-      oa.reset_pad0 = (unsigned char)rinfo[IN_GRASP]; oa.reset_pad1 = (unsigned char)rinfo[IN_PHEROMONE];
+      for (int v = 0; v < K; v++) {
+        oa.reset_pad0[v] = (unsigned char)rec[(size_t)v * REC_STRIDE + ST_STRIDE + IN_GRASP];
+        oa.reset_pad1[v] = (unsigned char)rec[(size_t)v * REC_STRIDE + ST_STRIDE + IN_PHEROMONE];
+      }
     }
     if (grs_reset(s.get(), nullptr, nullptr) != 0) throw std::runtime_error(g_err);
     CU(cudaStreamSynchronize(s->stream));
@@ -293,6 +344,7 @@ extern "C" void grs_destroy(grs_sim* s) {
 }
 
 extern "C" int32_t grs_num_envs(const grs_sim* s) { return s ? s->n : 0; }
+extern "C" int32_t grs_num_scenes(const grs_sim* s) { return s ? (s->compile_only ? 1 : (int32_t)s->scenes.size()) : 0; }
 extern "C" int32_t grs_action_dim(const grs_sim* s) { return s ? s->adim : 0; }
 extern "C" int32_t grs_obs_shape(const grs_sim* s, int32_t* chw) {
   if (!s || !chw) return fail("null argument");
@@ -319,7 +371,7 @@ extern "C" int32_t grs_reset(grs_sim* s, const uint8_t* mask_dev, void* stream) 
     k_reset<<<(s->n + wpb - 1) / wpb, wpb * 32, 0, st>>>(s->b, s->ecfg, mask_dev);
     CU(cudaGetLastError());
     if (s->obs_args.reset_noise) launch_render_reset(s->scene, s->obs_args, mask_dev, s->n, st);
-    else launch_copy_reset_obs(s->d_obs, s->d_reset_obs, s->d_hist, s->d_hist + (size_t)s->n * 512, mask_dev, s->n, s->C * s->H * s->W, st);
+    else launch_copy_reset_obs(s->d_obs, s->d_reset_obs, s->d_hist, s->d_hist + (size_t)s->n * 512, s->b.object, mask_dev, s->n, s->C * s->H * s->W, st);
     s->launches += 2;
     return 0;
   } catch (const std::exception& e) { return fail(e.what()); }
@@ -348,9 +400,8 @@ extern "C" int32_t grs_step(grs_sim* s, const float* actions_dev, void* stream) 
     k_order_count<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
     k_order_envs<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
     s->launches += 2;
-    if (s->fused_render) k_env_step_ls<false, true><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
-    else if (s->ls_timing) k_env_step_ls<true, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
-    else k_env_step_ls<false, false><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
+    const StepKernel k = s->fused_render ? s->kern.step_fused : s->ls_timing ? s->kern.step_timing : s->kern.step;
+    k<<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
     CU(cudaGetLastError());
     CU(cudaEventRecord(s->ev1[s->ev_n], st));
     s->ev_n++;
@@ -437,7 +488,7 @@ extern "C" int32_t grs_substep(grs_sim* s, int32_t n, void* stream) {
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     if (st != s->stream) s->last_dev_stream = st;  // a later host-path call (own stream) must order itself behind this one
     launch_queue_kernel_prep(s, st);
-    k_substep<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, st>>>(s->b, n);
+    s->kern.substep<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, st>>>(s->b, n);
     CU(cudaGetLastError());
     s->launches++;
     return 0;
@@ -455,7 +506,9 @@ extern "C" int32_t grs_buffer(grs_sim* s, const char* name, void** ptr, uint64_t
   else if (k == "info") { p = s->b.info; sz = N * IN_STRIDE * 4; }
   else if (k == "obs") { p = s->d_obs; sz = N * ob; }
   else if (k == "terminal_obs") { p = s->d_terminal_obs; sz = N * ob; }
-  else if (k == "reset_obs") { p = s->d_reset_obs; sz = ob; }
+  else if (k == "reset_obs") { p = s->d_reset_obs; sz = s->scenes.size() * ob; }
+  else if (k == "object") { p = s->b.object; sz = N * 4; }
+  else if (k == "next_object") { p = const_cast<int*>(s->b.next_object); sz = N * 4; }
   else if (k == "reward") { p = s->b.reward; sz = N * 4; }
   else if (k == "done") { p = s->b.done; sz = N; }
   else if (k == "achieved") { p = s->b.achieved; sz = N * 8; }
@@ -519,7 +572,7 @@ extern "C" int32_t grs_get_contacts(grs_sim* s, int32_t* ncon, int32_t* geom, fl
   try {
     CU(cudaSetDevice(s->device));
     launch_queue_kernel_prep(s, s->stream);
-    k_contacts<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, s->stream>>>(s->b);
+    s->kern.contacts<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, s->stream>>>(s->b);
     CU(cudaGetLastError());
     s->launches++;
     CU(cudaStreamSynchronize(s->stream));
@@ -548,7 +601,7 @@ extern "C" int32_t grs_debug_step(grs_sim* s) {
   try {
     CU(cudaSetDevice(s->device));
     launch_queue_kernel_prep(s, s->stream);
-    k_debug_step<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, s->stream>>>(s->b);
+    s->kern.debug_step<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, s->stream>>>(s->b);
     CU(cudaGetLastError());
     s->launches++;
     CU(cudaStreamSynchronize(s->stream));
@@ -635,6 +688,7 @@ extern "C" int64_t grs_model_get_int(const grs_sim* s, const char* name, int32_t
     else if (k == "iterations") tmp = {m.iterations};
     else if (k == "cone_elliptic") tmp = {m.cone_elliptic};
     else if (k == "named_bodies") tmp = {m.body_ee, m.body_object, m.finger1[0], m.finger1[1], m.finger2[0], m.finger2[1]};
+    else if (k == "step_smem" && !s->compile_only) tmp = {(int)s->ls_smem, s->b.hull_smem, s->b.hull_count, s->ls_warps};
     else if (k.rfind("hull_adjadr:", 0) == 0 || k.rfind("hull_adj:", 0) == 0 || k.rfind("hull_faces:", 0) == 0) {
       std::string mn = k.substr(k.find(':') + 1);
       const HostMesh* hm = nullptr;
@@ -676,9 +730,9 @@ extern "C" int32_t grs_render(grs_sim* s, int32_t camera_id, int32_t width, int3
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     if (st != s->stream) s->last_dev_stream = st;  // a later host-path call (own stream) must order itself behind this one
     launch_queue_kernel_prep(s, st);
-    k_camera_state<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, st>>>(s->b, camera_id);
+    s->kern.camera_state<<<s->grid, WARPS_PER_BLOCK * 32, s->smem, st>>>(s->b, camera_id);
     CU(cudaGetLastError());
-    launch_render_raw(s->scene, s->b.debug, DEBUG_STRIDE, rgb_dev, depth_dev, s->n, height, width, s->hm.cam_fovy[camera_id], st);
+    launch_render_raw(s->scene, s->b.debug, DEBUG_STRIDE, s->b.object, rgb_dev, depth_dev, s->n, height, width, s->hm.cam_fovy[camera_id], st);
     s->launches += 2;
     return 0;
   } catch (const std::exception& e) { return fail(e.what()); }
@@ -760,7 +814,7 @@ extern "C" int32_t grs_async_recv(grs_sim* s, int32_t* out_ids_dev, void* stream
     k_async_order_envs<<<g, 256, 0, st>>>(s->b, s->aa, s->d_actions, s->adim, B);
     if (s->ev_n == grs_sim::NEV) harvest_events(s);
     CU(cudaEventRecord(s->ev0[s->ev_n], st));
-    k_env_step_ls<false, false, true><<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, s->d_actions, s->adim, s->scene, s->obs_args, s->aa);
+    s->kern.step_async<<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, s->d_actions, s->adim, s->scene, s->obs_args, s->aa);
     CU(cudaGetLastError());
     CU(cudaEventRecord(s->ev1[s->ev_n], st));
     s->ev_n++;

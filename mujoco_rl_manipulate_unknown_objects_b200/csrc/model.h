@@ -16,6 +16,7 @@ namespace grs {
 constexpr int NQ = 14, NV = 13, NU = 7;
 constexpr int MAXB = 10, MAXJ = 8, MAXG = 8, MAXPAIR = 16, MAXMESH = 6, MAXLEVEL = 6;
 constexpr int MAXCAM = 4, MAXLIGHT = 4;
+constexpr int MAXOBJ = 8;  // scenes (object variants) one simulator can hold
 
 enum GeomType { GEOM_PLANE = 0, GEOM_BOX = 6, GEOM_MESH = 7 };
 enum JointType { JNT_FREE = 0, JNT_SLIDE = 2, JNT_HINGE = 3 };
@@ -106,5 +107,15 @@ struct DevModel {
 // Flatten a HostModel into the device layout.  hull vertices (float4, w = 0) and the per-geom hull graph
 // ([nvert+1 offsets][neighbours], one block per geom) go to separate arrays.
 void build_dev_model(const HostModel& h, DevModel& d, std::vector<float>& hull_verts4, std::vector<int>& hull_adj);
+
+// Mixed simulators: several scenes that differ only in the object.  Returns the name of the first shared field (counts, tree,
+// joint / dof / actuator layout, named bodies, geoms and pairs, the gripper's hulls and render data, options, cameras' fovy,
+// lights and textures) in which `b` differs from `a`, or "" when the two can share one simulator.
+std::string scene_mismatch(const HostModel& a, const HostModel& b);
+
+// Appends the object geom's hull of variant `d` to the concatenated arrays and points every other geom of `d` at the hulls of
+// variant 0 (`d0`); `hv4` / `adj` are variant d's own arrays from build_dev_model.
+void rebase_hull(const DevModel& d0, DevModel& d, const std::vector<float>& hv4, const std::vector<int>& adj, std::vector<float>& all_hv4,
+                 std::vector<int>& all_adj);
 
 }  // namespace grs

@@ -18,6 +18,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <cstring>
 #include <stdexcept>
 #include <vector>
 
@@ -43,10 +44,24 @@ struct RenderScene {
   int light_directional[MAXLIGHT + 1];
   float light_pos[MAXLIGHT + 1][3], light_dir[MAXLIGHT + 1][3], light_diffuse[MAXLIGHT + 1][3], light_ambient[MAXLIGHT + 1][3], light_specular[MAXLIGHT + 1][3];
   float headlight_ambient[3], headlight_diffuse[3], headlight_specular[3];
-  float znear, zfar;  // metres (already scaled by the model extent)
+  // per variant: the object geom's triangles (variant 0's sit in the geom order, the others' follow every shared triangle) and
+  // the clip planes, in metres (scaled by the variant's model extent)
+  int obj_geom;
+  int obj_triadr[MAXOBJ], obj_trinum[MAXOBJ];
+  float znear[MAXOBJ], zfar[MAXOBJ];
 };
 
-inline void render_scene_upload(const HostModel& h, RenderScene& sc, std::vector<void*>& owned) {
+// triangles of geom g in variant v
+__device__ __forceinline__ void geom_tris(const RenderScene& sc, int g, int v, int& adr, int& num) {
+  const bool obj = g == sc.obj_geom;
+  adr = obj ? sc.obj_triadr[v] : sc.geom_triadr[g];
+  num = obj ? sc.obj_trinum[v] : sc.geom_trinum[g];
+}
+
+// hs: the variants of one simulator (scene_mismatch found them compatible); everything but the object geom's triangles and the
+// clip planes comes from hs[0]
+inline void render_scene_upload(const std::vector<HostModel>& hs, RenderScene& sc, std::vector<void*>& owned) {
+  const HostModel& h = hs[0];
   std::memset(&sc, 0, sizeof sc);
   std::vector<float> tri;
   sc.ngeom = h.ngeom;
@@ -65,6 +80,20 @@ inline void render_scene_upload(const HostModel& h, RenderScene& sc, std::vector
     for (int k = 0; k < 4; k++) sc.geom_rgba[g][k] = (float)h.geom_rgba[4 * g + k];
     sc.geom_emission[g] = (float)h.geom_matprop[4 * g]; sc.geom_specular[g] = (float)h.geom_matprop[4 * g + 1];
     sc.geom_shininess[g] = (float)h.geom_matprop[4 * g + 2]; sc.geom_textured[g] = h.geom_matprop[4 * g + 3] != 0;
+  }
+  sc.obj_geom = -1;
+  for (int g = 0; g < h.ngeom; g++) if (h.geom_bodyid[g] == h.body_object) { sc.obj_geom = g; break; }
+  if (sc.obj_geom < 0 || h.geom_meshid[sc.obj_geom] < 0) throw std::runtime_error("the object body has no mesh geom to render");
+  for (size_t v = 0; v < hs.size(); v++) {
+    if (v == 0) {
+      sc.obj_triadr[0] = sc.geom_triadr[sc.obj_geom]; sc.obj_trinum[0] = sc.geom_trinum[sc.obj_geom];
+    } else {
+      const auto& t = hs[v].meshes[hs[v].geom_meshid[sc.obj_geom]].tri;
+      sc.obj_triadr[v] = (int)tri.size() / 9;
+      tri.insert(tri.end(), t.begin(), t.end());
+      sc.obj_trinum[v] = (int)tri.size() / 9 - sc.obj_triadr[v];
+    }
+    sc.znear[v] = (float)(hs[v].znear * hs[v].extent); sc.zfar[v] = (float)(hs[v].zfar * hs[v].extent);
   }
   sc.ntri_total = (int)tri.size() / 9;
   if (sc.ntri_total >= (1 << 20)) throw std::runtime_error("too many render triangles");
@@ -89,15 +118,16 @@ inline void render_scene_upload(const HostModel& h, RenderScene& sc, std::vector
     }
   }
   for (int k = 0; k < 3; k++) { sc.headlight_ambient[k] = 0.1f; sc.headlight_diffuse[k] = 0.4f; sc.headlight_specular[k] = 0.5f; }  // mjVisual.headlight defaults
-  sc.znear = (float)(h.znear * h.extent); sc.zfar = (float)(h.zfar * h.extent);
 }
 
 // render state of an arbitrary camera for every environment -> first RS_STRIDE floats of each debug row
+template <bool MULTI>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32) k_camera_state(SimBuffers s, int cam) {
-  const DevModel& m = stage_model(s.model);
-  WS& w = my_ws();
+  stage_models<MULTI>(s);
+  WS& w = my_ws(MULTI ? s.nobj : 1);
   const int lane = threadIdx.x & 31;
   for (int env = next_env(s.queue, lane); env < s.n; env = next_env(s.queue, lane)) {
+    const DevModel& m = smem_model(MULTI ? s.object[env] : 0);
     EnvFlags f;
     load_state(w, f, s.state + (size_t)env * ST_STRIDE, lane);
     kinematics(m, w, lane);
@@ -230,12 +260,14 @@ __device__ __forceinline__ Shade shade_point(const RenderScene& sc, int g, const
 }
 
 // Renders one tile into shared memory: after the call zbuf[pix] low word = depth (float bits, metres along the optical axis),
-// and rgb8[pix] holds the packed colour.  rs = this environment's render state (geom poses + camera).
-__device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs, TileShared& sh, unsigned* rgb8, int W, int H, int tx0, int ty0, int tw, int th, float fovy) {
+// and rgb8[pix] holds the packed colour.  rs = this environment's render state (geom poses + camera), v = its variant.
+static __device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs, int v, TileShared& sh, unsigned* rgb8, int W, int H, int tx0, int ty0, int tw, int th,
+                            float fovy) {
   const int tid = threadIdx.x;
+  const float znear = sc.znear[v], zfar = sc.zfar[v];
   const float ify = tanf(0.5f * fovy * 0.017453292519943295f) /* MJCF fovy is always in degrees */, ifx = ify * (float)W / (float)H;
   const float fx = 1.0f / ifx, fy = 1.0f / ify;
-  for (int i = tid; i < TILE * TILE; i += RTHREADS) sh.zbuf[i] = pack_frag(sc.zfar, 0xffffffffu);
+  for (int i = tid; i < TILE * TILE; i += RTHREADS) sh.zbuf[i] = pack_frag(zfar, 0xffffffffu);
   if (tid < 12) sh.cam[tid] = rs[84 + tid];
   if (tid == 0) sh.nbig = 0;
   if (tid < TILE) sh.dxs[tid] = ((2.0f * ((tx0 + tid) + 0.5f)) / W - 1.0f) * ifx;
@@ -258,9 +290,10 @@ __device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs,
   __syncthreads();
   // ---- pass 1a: per-thread triangles
   for (int g = 0; g < sc.ngeom; g++) {
-    const int n = sc.geom_trinum[g], adr = sc.geom_triadr[g];
+    int n, adr;
+    geom_tris(sc, g, v, adr, n);
     for (int t = tid; t < n; t += RTHREADS) {
-      TriSetup s = tri_setup(sc.tri + (size_t)(adr + t) * 9, sh.xf[g], fx, fy, W, H, tx0, ty0, tw, th, sc.znear);
+      TriSetup s = tri_setup(sc.tri + (size_t)(adr + t) * 9, sh.xf[g], fx, fy, W, H, tx0, ty0, tw, th, znear);
       if (!s.ok) continue;
       int area = (s.x1 - s.x0 + 1) * (s.y1 - s.y0 + 1);
       unsigned id = (unsigned)(adr + t);
@@ -269,7 +302,7 @@ __device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs,
         if (q < BIGQ) { sh.bigq[q] = (g << 24) | t; continue; }
       }
       for (int py = s.y0; py <= s.y1; py++)
-        for (int px = s.x0; px <= s.x1; px++) raster_pixel(s, sh.dxs[px - tx0], sh.dys[py - ty0], px - tx0, py - ty0, sc.znear, sc.zfar, id, sh.zbuf);
+        for (int px = s.x0; px <= s.x1; px++) raster_pixel(s, sh.dxs[px - tx0], sh.dys[py - ty0], px - tx0, py - ty0, znear, zfar, id, sh.zbuf);
     }
   }
   __syncthreads();
@@ -277,17 +310,18 @@ __device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs,
   {
     const int nb = min(sh.nbig, BIGQ), warp = tid >> 5, lane = tid & 31;
     for (int q = warp; q < nb; q += RTHREADS / 32) {
-      int g = sh.bigq[q] >> 24, t = sh.bigq[q] & 0xffffff;
-      TriSetup s = tri_setup(sc.tri + (size_t)(sc.geom_triadr[g] + t) * 9, sh.xf[g], fx, fy, W, H, tx0, ty0, tw, th, sc.znear);
+      int g = sh.bigq[q] >> 24, t = sh.bigq[q] & 0xffffff, adr, n;
+      geom_tris(sc, g, v, adr, n);
+      TriSetup s = tri_setup(sc.tri + (size_t)(adr + t) * 9, sh.xf[g], fx, fy, W, H, tx0, ty0, tw, th, znear);
       if (!s.ok) continue;
-      unsigned id = (unsigned)(sc.geom_triadr[g] + t);
+      unsigned id = (unsigned)(adr + t);
       // dx(px) = A * px + B
       const float A = 2.0f * ifx / (float)W, B = (1.0f / (float)W - 1.0f) * ifx;
       for (int py = s.y0 + lane; py <= s.y1; py += 32) {  // one row per lane, only the columns the triangle can cover
         const float dy = sh.dys[py - ty0];
         int lo, hi;
         row_span(s, dy, A, B, lo, hi);
-        for (int px = lo; px <= hi; px++) raster_pixel(s, sh.dxs[px - tx0], dy, px - tx0, py - ty0, sc.znear, sc.zfar, id, sh.zbuf);
+        for (int px = lo; px <= hi; px++) raster_pixel(s, sh.dxs[px - tx0], dy, px - tx0, py - ty0, znear, zfar, id, sh.zbuf);
       }
     }
   }
@@ -307,7 +341,8 @@ __device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs,
     float nrm[3] = {0, 0, 1};
     if (id != 0xffffffffu) {
       int g = 0;
-      for (int k = 1; k < sc.ngeom; k++) if ((int)id >= sc.geom_triadr[k] && sc.geom_trinum[k] > 0) g = k;
+      for (int k = 1; k < sc.ngeom; k++) if (k != sc.obj_geom && (int)id >= sc.geom_triadr[k] && sc.geom_trinum[k] > 0) g = k;
+      if ((int)id >= sc.obj_triadr[v] && (int)id < sc.obj_triadr[v] + sc.obj_trinum[v]) g = sc.obj_geom;
       hit_geom = g;
       const float* tp = sc.tri + (size_t)id * 9;
       float a[3] = {__ldg(tp), __ldg(tp + 1), __ldg(tp + 2)}, e1[3] = {__ldg(tp + 3) - a[0], __ldg(tp + 4) - a[1], __ldg(tp + 5) - a[2]},
@@ -325,7 +360,7 @@ __device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs,
       float num = pn[0] * (pp[0] - cp[0]) + pn[1] * (pp[1] - cp[1]) + pn[2] * (pp[2] - cp[2]);
       if (denom != 0.0f) {
         float t = num / denom;
-        if (t >= sc.znear && t < depth) {
+        if (t >= znear && t < depth) {
           float hp[3] = {cp[0] + t * dw[0] - pp[0], cp[1] + t * dw[1] - pp[1], cp[2] + t * dw[2] - pp[2]};
           float u = hp[0] * pm[0] + hp[1] * pm[3] + hp[2] * pm[6], v = hp[0] * pm[1] + hp[1] * pm[4] + hp[2] * pm[7];
           bool inside = (sc.plane_size[0] <= 0 || fabsf(u) <= sc.plane_size[0]) && (sc.plane_size[1] <= 0 || fabsf(v) <= sc.plane_size[1]);
@@ -338,7 +373,7 @@ __device__ void render_tile(const RenderScene& sc, const float* __restrict__ rs,
       float m = fmaxf(fabsf(dw[0]), fmaxf(fabsf(dw[1]), fabsf(dw[2])));
       float f = 0.5f * (dw[2] / m + 1.0f);
       c.r = sc.sky_rgb2[0] + f * (sc.sky_rgb1[0] - sc.sky_rgb2[0]); c.g = sc.sky_rgb2[1] + f * (sc.sky_rgb1[1] - sc.sky_rgb2[1]); c.b = sc.sky_rgb2[2] + f * (sc.sky_rgb1[2] - sc.sky_rgb2[2]);
-      depth = sc.zfar;
+      depth = zfar;
     } else {
       float p[3] = {cp[0] + depth * dw[0], cp[1] + depth * dw[1], cp[2] + depth * dw[2]};
       float tex[3] = {1, 1, 1};
@@ -382,18 +417,19 @@ __device__ __forceinline__ float block_reduce(float v, float* red, int op /*0 su
 struct ObsArgs {
   unsigned char* obs;           // [n][C][H][W] uint8
   unsigned char* terminal_obs;  // likewise (SB3 terminal observation of environments that finished an episode)
-  const unsigned char* reset_obs;  // [C][H][W] observation of a freshly reset environment
+  const unsigned char* reset_obs;  // [nobj][C][H][W] observation of a freshly reset environment, per variant
   float* hist_prev;             // [n][2][256] float histograms (grey, depth) of each env's previous observation
-  float* hist_reset;            // the reset image's histograms
+  float* hist_reset;            // [nobj][2][256] the reset images' histograms
+  const int* object;            // [n] variant of each environment's current episode (the one a reset started)
   int C, H, W;
   float fovy;
   int auto_reset, im_reward;
   // reset randomisation: the observation of a new episode is rendered (reset record's scene with the object geom at its
   // per-environment pose) instead of copied from the constant reset image
   int reset_noise, obj_geom;
-  const float* reset_rs;   // [RS_STRIDE] render state of the reset record
+  const float* reset_rs;   // [nobj] render states of the reset records, REC_STRIDE apart
   const float* reset_obj;  // [n][12] object geom pose of each environment's current episode
-  unsigned char reset_pad0, reset_pad1;  // pad-channel scalars of a freshly reset environment
+  unsigned char reset_pad0[MAXOBJ], reset_pad1[MAXOBJ];  // pad-channel scalars of a freshly reset environment, per variant
   // host mirrors (grs_step_host with PINNED host buffers): device-visible addresses of the caller's pinned observation /
   // terminal-observation arrays, or NULL.  Each finished observation is stored there by the block that built it, so the
   // device-to-host transfer of the 20 KB images rides under the physics of the environments still integrating.
@@ -426,10 +462,10 @@ __device__ __forceinline__ void mirror_to_host(const unsigned char* src, unsigne
 //   reward   : per-env reward array (the intrinsic term is added in place), or NULL
 // rasterise + shade the scene `rs`, transform_depth, pack uint8 CHW with the two scalar channels into `dst`, histograms of the
 // grey image and of the depth channel into sh.hist
-__device__ __forceinline__ void render_and_pack(const RenderScene& sc, const ObsArgs& o, const float* rs, unsigned char* dst, unsigned char pad0, unsigned char pad1,
+__device__ __forceinline__ void render_and_pack(const RenderScene& sc, const ObsArgs& o, const float* rs, int v, unsigned char* dst, unsigned char pad0, unsigned char pad1,
                                                 TileShared& sh, unsigned* rgb8) {
   const int tid = threadIdx.x, C = o.C, H = o.H, W = o.W;
-  render_tile(sc, rs, sh, rgb8, W, H, 0, 0, W, H, o.fovy);
+  render_tile(sc, rs, v, sh, rgb8, W, H, 0, 0, W, H, o.fovy);
   const int npix = W * H;
   // transform_depth (utils.py:11-19): d -= min(d); d /= 2*mean(d[d <= 1]); 255*clip(d, 0, 1)
   float mn = 3.0e38f;
@@ -464,18 +500,20 @@ __device__ __forceinline__ void render_and_pack(const RenderScene& sc, const Obs
   __syncthreads();
 }
 
-// scene of a freshly reset environment with the object geom at this environment's pose -> rs2 (shared memory, RS_STRIDE floats)
-__device__ __forceinline__ void build_reset_scene(const ObsArgs& o, int env, float* rs2) {
+// scene of a freshly reset environment of variant v with the object geom at this environment's pose -> rs2 (shared memory,
+// RS_STRIDE floats)
+__device__ __forceinline__ void build_reset_scene(const ObsArgs& o, int env, int v, float* rs2) {
   const int tid = threadIdx.x;
   __syncthreads();
   if (tid < RS_STRIDE) {
     const int g = tid / 12;
-    rs2[tid] = (g == o.obj_geom && tid < 84) ? __ldcg(o.reset_obj + (size_t)env * 12 + (tid - 12 * g)) : o.reset_rs[tid];
+    rs2[tid] = (g == o.obj_geom && tid < 84) ? __ldcg(o.reset_obj + (size_t)env * 12 + (tid - 12 * g)) : o.reset_rs[(size_t)v * REC_STRIDE + tid];
   }
   __syncthreads();
 }
 
-__device__ __forceinline__ void render_obs_env(const RenderScene& sc, const ObsArgs& o, const float* rs, int env, unsigned char pad0, unsigned char pad1,
+// v: the variant of the episode the step belongs to (info IN_OBJECT); an auto-reset's new episode is o.object[env]
+__device__ __forceinline__ void render_obs_env(const RenderScene& sc, const ObsArgs& o, const float* rs, int v, int env, unsigned char pad0, unsigned char pad1,
                                                bool is_done, float* reward, TileShared& sh, unsigned* rgb8, float* rs2) {
   const int tid = threadIdx.x, C = o.C, auto_reset = o.auto_reset, im_reward = o.im_reward, npix = o.W * o.H;
   unsigned char* obs = o.obs;
@@ -484,7 +522,7 @@ __device__ __forceinline__ void render_obs_env(const RenderScene& sc, const ObsA
   float* hist_reset = o.hist_reset;
   const bool swap = is_done && auto_reset;
   unsigned char* dst = swap ? o.terminal_obs + (size_t)env * C * npix : obs + (size_t)env * C * npix;
-  render_and_pack(sc, o, rs, dst, pad0, pad1, sh, rgb8);
+  render_and_pack(sc, o, rs, v, dst, pad0, pad1, sh, rgb8);
   {
     unsigned char* hm = swap ? o.terminal_obs_host : o.obs_host;
     if (hm) mirror_to_host(dst, hm + (size_t)env * C * npix, C * npix);
@@ -515,12 +553,15 @@ __device__ __forceinline__ void render_obs_env(const RenderScene& sc, const ObsA
   __syncthreads();
   if (is_done && auto_reset) {
     // SB3 VecEnv: the returned observation is the first one of the next episode; the terminal one went to terminal_obs
+    const int vn = __ldcg(o.object + env);
     if (o.reset_noise) {
-      build_reset_scene(o, env, rs2);
-      render_and_pack(sc, o, rs2, obs + (size_t)env * C * npix, o.reset_pad0, o.reset_pad1, sh, rgb8);
+      build_reset_scene(o, env, vn, rs2);
+      render_and_pack(sc, o, rs2, vn, obs + (size_t)env * C * npix, o.reset_pad0[vn], o.reset_pad1[vn], sh, rgb8);
       if (o.obs_host) mirror_to_host(obs + (size_t)env * C * npix, o.obs_host + (size_t)env * C * npix, C * npix);
       if (hp) for (int i = tid; i < 512; i += RTHREADS) hp[i] = (float)(&sh.hist[0][0])[i];
     } else {
+      reset_obs += (size_t)vn * C * npix;
+      hist_reset += (size_t)vn * 512;
       const uint4* src = reinterpret_cast<const uint4*>(reset_obs);
       uint4* o4 = reinterpret_cast<uint4*>(obs + (size_t)env * C * npix);
       if ((C * npix) % 16 == 0) { for (int i = tid; i < C * npix / 16; i += RTHREADS) o4[i] = src[i]; }
@@ -541,7 +582,7 @@ __device__ __forceinline__ void render_obs_env(const RenderScene& sc, const ObsA
 // Standalone observation kernel: one block per environment.  info: per-env info rows; done: per-env done flags (NULL for
 // the reset image).  Used for the reset image and whenever the step kernel runs without its observation phase
 // (GRS_FUSED_RENDER=0, GRS_STEP_TIMING, other block widths than RTHREADS).
-__global__ void __launch_bounds__(RTHREADS) k_render_obs(RenderScene sc, ObsArgs o, const float* __restrict__ render_state, const float* __restrict__ info, int info_stride,
+static __global__ void __launch_bounds__(RTHREADS) k_render_obs(RenderScene sc, ObsArgs o, const float* __restrict__ render_state, const float* __restrict__ info, int info_stride,
                                                         const unsigned char* __restrict__ done, float* __restrict__ reward) {
   extern __shared__ __align__(16) unsigned char rsm[];
   TileShared& sh = *reinterpret_cast<TileShared*>(rsm);
@@ -549,12 +590,13 @@ __global__ void __launch_bounds__(RTHREADS) k_render_obs(RenderScene sc, ObsArgs
   float* rs2 = reinterpret_cast<float*>(rsm + sizeof(TileShared) + TILE * TILE * sizeof(unsigned));
   const int env = blockIdx.x;
   const float* inf = info + (size_t)env * info_stride;
-  render_obs_env(sc, o, render_state + (size_t)env * RS_STRIDE, env, (unsigned char)inf[IN_GRASP], (unsigned char)inf[IN_PHEROMONE], done ? done[env] != 0 : false, reward, sh, rgb8, rs2);
+  render_obs_env(sc, o, render_state + (size_t)env * RS_STRIDE, (int)inf[IN_OBJECT], env, (unsigned char)inf[IN_GRASP], (unsigned char)inf[IN_PHEROMONE],
+                 done ? done[env] != 0 : false, reward, sh, rgb8, rs2);
 }
 
 // The same over a list: block b builds the observation of environment list[b] for b < *count (the asynchronous step renders
 // the environments its launch finished; the grid is sized for the largest possible count).
-__global__ void __launch_bounds__(RTHREADS) k_render_obs_indexed(RenderScene sc, ObsArgs o, const float* __restrict__ render_state, const float* __restrict__ info,
+static __global__ void __launch_bounds__(RTHREADS) k_render_obs_indexed(RenderScene sc, ObsArgs o, const float* __restrict__ render_state, const float* __restrict__ info,
                                                                 int info_stride, const unsigned char* __restrict__ done, float* __restrict__ reward,
                                                                 const int* __restrict__ list, const int* __restrict__ count) {
   if ((int)blockIdx.x >= *count) return;
@@ -564,19 +606,21 @@ __global__ void __launch_bounds__(RTHREADS) k_render_obs_indexed(RenderScene sc,
   float* rs2 = reinterpret_cast<float*>(rsm + sizeof(TileShared) + TILE * TILE * sizeof(unsigned));
   const int env = list[blockIdx.x];
   const float* inf = info + (size_t)env * info_stride;
-  render_obs_env(sc, o, render_state + (size_t)env * RS_STRIDE, env, (unsigned char)inf[IN_GRASP], (unsigned char)inf[IN_PHEROMONE], done[env] != 0, reward, sh, rgb8, rs2);
+  render_obs_env(sc, o, render_state + (size_t)env * RS_STRIDE, (int)inf[IN_OBJECT], env, (unsigned char)inf[IN_GRASP], (unsigned char)inf[IN_PHEROMONE], done[env] != 0,
+                 reward, sh, rgb8, rs2);
 }
 
 // Explicit reset with reset randomisation: observation (and histograms) of the masked environments' new episodes
-__global__ void __launch_bounds__(RTHREADS) k_render_reset(RenderScene sc, ObsArgs o, const unsigned char* __restrict__ mask) {
+static __global__ void __launch_bounds__(RTHREADS) k_render_reset(RenderScene sc, ObsArgs o, const unsigned char* __restrict__ mask) {
   extern __shared__ __align__(16) unsigned char rsm[];
   TileShared& sh = *reinterpret_cast<TileShared*>(rsm);
   unsigned* rgb8 = reinterpret_cast<unsigned*>(rsm + sizeof(TileShared));
   float* rs2 = reinterpret_cast<float*>(rsm + sizeof(TileShared) + TILE * TILE * sizeof(unsigned));
   const int env = blockIdx.x, npix = o.W * o.H;
   if (mask && !mask[env]) return;
-  build_reset_scene(o, env, rs2);
-  render_and_pack(sc, o, rs2, o.obs + (size_t)env * o.C * npix, o.reset_pad0, o.reset_pad1, sh, rgb8);
+  const int v = o.object[env];
+  build_reset_scene(o, env, v, rs2);
+  render_and_pack(sc, o, rs2, v, o.obs + (size_t)env * o.C * npix, o.reset_pad0[v], o.reset_pad1[v], sh, rgb8);
   if (o.hist_prev) for (int i = threadIdx.x; i < 512; i += RTHREADS) o.hist_prev[(size_t)env * 512 + i] = (float)(&sh.hist[0][0])[i];
 }
 
@@ -628,9 +672,10 @@ __device__ __forceinline__ void render_phase(const RenderScene& sc, const ObsArg
     if (tid < RS_STRIDE) rs[tid] = __ldcg(s.render_state + (size_t)env * RS_STRIDE + tid);
     const float* inf = s.info + (size_t)env * IN_STRIDE;
     const unsigned char pad0 = (unsigned char)__ldcg(inf + IN_GRASP), pad1 = (unsigned char)__ldcg(inf + IN_PHEROMONE);
+    const int v = (int)__ldcg(inf + IN_OBJECT);
     const bool is_done = __ldcg(s.done + env) != 0;
     __syncthreads();
-    render_obs_env(sc, o, rs, env, pad0, pad1, is_done, s.reward, sh, rgb8, rs);  // rs is dead once the terminal image is packed
+    render_obs_env(sc, o, rs, v, env, pad0, pad1, is_done, s.reward, sh, rgb8, rs);  // rs is dead once the terminal image is packed
   }
 }
 
@@ -657,30 +702,31 @@ inline void launch_render_reset(const RenderScene& sc, const ObsArgs& o, const u
   if (cudaGetLastError() != cudaSuccess) throw std::runtime_error("k_render_reset launch failed");
 }
 
-// reset path: copy the constant reset image (and its histograms) into the masked environments
-__global__ void k_copy_reset_obs(unsigned char* __restrict__ obs, const unsigned char* __restrict__ reset_obs, float* __restrict__ hist, const float* __restrict__ hist_reset,
-                                 const unsigned char* __restrict__ mask, int bytes) {
+// reset path: copy the constant reset image of each masked environment's variant (and its histograms) into it
+static __global__ void k_copy_reset_obs(unsigned char* __restrict__ obs, const unsigned char* __restrict__ reset_obs, float* __restrict__ hist, const float* __restrict__ hist_reset,
+                                 const int* __restrict__ object, const unsigned char* __restrict__ mask, int bytes) {
   const int env = blockIdx.x;
   if (mask && !mask[env]) return;
-  for (int i = threadIdx.x; i < bytes; i += blockDim.x) obs[(size_t)env * bytes + i] = reset_obs[i];
-  for (int i = threadIdx.x; i < 512; i += blockDim.x) hist[(size_t)env * 512 + i] = hist_reset[i];
+  const int v = object[env];
+  for (int i = threadIdx.x; i < bytes; i += blockDim.x) obs[(size_t)env * bytes + i] = reset_obs[(size_t)v * bytes + i];
+  for (int i = threadIdx.x; i < 512; i += blockDim.x) hist[(size_t)env * 512 + i] = hist_reset[(size_t)v * 512 + i];
 }
-inline void launch_copy_reset_obs(unsigned char* obs, const unsigned char* reset_obs, float* hist, const float* hist_reset, const unsigned char* mask, int n, int bytes,
-                                  cudaStream_t st) {
-  k_copy_reset_obs<<<n, 256, 0, st>>>(obs, reset_obs, hist, hist_reset, mask, bytes);
+inline void launch_copy_reset_obs(unsigned char* obs, const unsigned char* reset_obs, float* hist, const float* hist_reset, const int* object, const unsigned char* mask, int n,
+                                  int bytes, cudaStream_t st) {
+  k_copy_reset_obs<<<n, 256, 0, st>>>(obs, reset_obs, hist, hist_reset, object, mask, bytes);
   if (cudaGetLastError() != cudaSuccess) throw std::runtime_error("k_copy_reset_obs launch failed");
 }
 
 // RobotEnv.render / physics.render for any camera and size: rgb u8[n][h][w][3], depth f32[n][h][w] in metres; grid (tiles, n)
-__global__ void __launch_bounds__(RTHREADS) k_render_raw(RenderScene sc, const float* __restrict__ render_state, int rs_stride, unsigned char* __restrict__ rgb,
-                                                        float* __restrict__ depth, int H, int W, float fovy) {
+static __global__ void __launch_bounds__(RTHREADS) k_render_raw(RenderScene sc, const float* __restrict__ render_state, int rs_stride, const int* __restrict__ object,
+                                                        unsigned char* __restrict__ rgb, float* __restrict__ depth, int H, int W, float fovy) {
   extern __shared__ __align__(16) unsigned char rsm[];
   TileShared& sh = *reinterpret_cast<TileShared*>(rsm);
   unsigned* rgb8 = reinterpret_cast<unsigned*>(rsm + sizeof(TileShared));
   const int env = blockIdx.y, tiles_x = (W + TILE - 1) / TILE;
   const int tx0 = (blockIdx.x % tiles_x) * TILE, ty0 = (blockIdx.x / tiles_x) * TILE;
   const int tw = min(TILE, W - tx0), th = min(TILE, H - ty0);
-  render_tile(sc, render_state + (size_t)env * rs_stride, sh, rgb8, W, H, tx0, ty0, tw, th, fovy);
+  render_tile(sc, render_state + (size_t)env * rs_stride, object[env], sh, rgb8, W, H, tx0, ty0, tw, th, fovy);
   for (int i = threadIdx.x; i < tw * th; i += RTHREADS) {
     int ly = i / tw, lx = i - ly * tw;
     size_t o = ((size_t)env * H + ty0 + ly) * W + tx0 + lx;
@@ -689,8 +735,8 @@ __global__ void __launch_bounds__(RTHREADS) k_render_raw(RenderScene sc, const f
     if (depth) depth[o] = __uint_as_float((unsigned)sh.zbuf[ly * TILE + lx]);
   }
 }
-inline void launch_render_raw(const RenderScene& sc, const float* render_state, int rs_stride, unsigned char* rgb, float* depth, int n, int H, int W, double fovy,
-                              cudaStream_t st) {
+inline void launch_render_raw(const RenderScene& sc, const float* render_state, int rs_stride, const int* object, unsigned char* rgb, float* depth, int n, int H, int W,
+                              double fovy, cudaStream_t st) {
   static bool attr_dev[64] = {};
   int dev_ = 0;
   cudaGetDevice(&dev_);
@@ -700,7 +746,7 @@ inline void launch_render_raw(const RenderScene& sc, const float* render_state, 
     attr = true;
   }
   dim3 grid(((W + TILE - 1) / TILE) * ((H + TILE - 1) / TILE), n);
-  k_render_raw<<<grid, RTHREADS, render_smem_bytes(), st>>>(sc, render_state, rs_stride, rgb, depth, H, W, fovy);
+  k_render_raw<<<grid, RTHREADS, render_smem_bytes(), st>>>(sc, render_state, rs_stride, object, rgb, depth, H, W, fovy);
   if (cudaGetLastError() != cudaSuccess) throw std::runtime_error("k_render_raw launch failed");
 }
 

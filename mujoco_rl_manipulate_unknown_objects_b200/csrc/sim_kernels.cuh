@@ -215,7 +215,7 @@ __device__ __noinline__ float chol_factor_solve(float* A, float* tmp, float b, i
 
 // -------------------------------------------------------------------------------- position stage
 // engine_core_smooth.c : mj_kinematics — lanes = bodies of one depth level
-__device__ __noinline__ void kinematics(const DevModel& m, WS& w, int lane) {
+static __device__ __noinline__ void kinematics(const DevModel& m, WS& w, int lane) {
   if (lane == 0) {
     // mj_normalizeQuat on the free joint
     for (int j = 0; j < m.njnt; j++)
@@ -285,7 +285,7 @@ __device__ __noinline__ void kinematics(const DevModel& m, WS& w, int lane) {
 }
 
 // engine_core_smooth.c : mj_comPos + mj_crb.  Leaves cdof, com, M (with armature) and the dyn scratch (cinert) filled.
-__device__ __noinline__ void com_pos_crb(const DevModel& m, WS& w, int lane) {
+static __device__ __noinline__ void com_pos_crb(const DevModel& m, WS& w, int lane) {
   const int nb = m.nbody;
   if (lane < nb) {
     int b = lane;
@@ -403,7 +403,7 @@ __device__ __forceinline__ unsigned sortable_key(float x) {
   return (k & 0x80000000u) ? ~k : (k | 0x80000000u);
 }
 // engine_collision_convex.c : mjccd_support for a hull — every lane scans a strided slice, arg-max by shuffles
-__device__ __noinline__ int support_geom(const DevModel& m, const WS& w, const float4* __restrict__ hv, int g, const float* dir, float* out, int lane) {
+static __device__ __noinline__ int support_geom(const DevModel& m, const WS& w, const float4* __restrict__ hv, int g, const float* dir, float* out, int lane) {
   const float* R = w.gmat[g];
   float l[3];
   mulmat3Tvec(l, R, dir);
@@ -431,7 +431,7 @@ __device__ __noinline__ int support_geom(const DevModel& m, const WS& w, const f
 // libccd support.c : __ccdSupport on obj1 - obj2, each inflated by margin/2; result into portal slot `slot`.
 // Both hull scans run in ONE loop (two independent compare chains per lane, two pairs of warp reductions back to back), so
 // a lone warp overlaps their latencies; vertex order, comparisons and tie rules are those of support_geom.
-__device__ __noinline__ void support_md(const DevModel& m, WS& w, const float4* hv, int g1, int g2, float margin, const float* dir, int slot, int lane) {
+static __device__ __noinline__ void support_md(const DevModel& m, WS& w, const float4* hv, int g1, int g2, float margin, const float* dir, int slot, int lane) {
   float n[3] = {dir[0], dir[1], dir[2]}, nd[3];
   normalize3(n);
   nd[0] = -n[0]; nd[1] = -n[1]; nd[2] = -n[2];
@@ -544,7 +544,7 @@ __device__ __forceinline__ void find_pos(const WS& w, float* pos) {
     pos[k] = inv * (b[0] * (SUPV1(0)[k] + SUPV2(0)[k]) + b[1] * (SUPV1(1)[k] + SUPV2(1)[k]) + b[2] * (SUPV1(2)[k] + SUPV2(2)[k]) + b[3] * (SUPV1(3)[k] + SUPV2(3)[k]));
 }
 // libccd mpr.c : ccdMPRPenetration (discoverPortal, refinePortal, findPenetr). All lanes carry the same portal.
-__device__ __noinline__ bool mpr_penetration(const DevModel& m, WS& w, const float4* hv, int g1, int g2, float margin,
+static __device__ __noinline__ bool mpr_penetration(const DevModel& m, WS& w, const float4* hv, int g1, int g2, float margin,
                                              float* depth, float* dir_out, float* pos, int lane) {
   float dir[3], va[3], vb[3];
   __syncwarp();
@@ -620,7 +620,7 @@ __device__ __noinline__ bool mpr_penetration(const DevModel& m, WS& w, const flo
 }
 
 // mju_makeFrame + contact bookkeeping (lane 0 writes)
-__device__ __noinline__ void add_contact(const DevModel& m, WS& w, int pair, float dist, const float* pos, const float* normal, int lane) {
+static __device__ __noinline__ void add_contact(const DevModel& m, WS& w, int pair, float dist, const float* pos, const float* normal, int lane) {
   int c = w.ncon;
   if (c >= MAXCON) { if (lane == 0) w.overflow = 1; return; }
   if (lane == 0) {
@@ -646,7 +646,7 @@ __device__ __noinline__ void add_contact(const DevModel& m, WS& w, int pair, flo
 }
 
 // engine_collision_driver.c : mj_collision over the candidate pair list (+ the bounding-sphere test of mj_collideGeoms)
-__device__ __noinline__ void collision(const DevModel& m, WS& w, const float4* hv, const int* __restrict__ adj, int lane) {
+static __device__ __noinline__ void collision(const DevModel& m, WS& w, const float4* hv, const int* __restrict__ adj, int lane) {
   if (lane == 0) { w.ncon = 0; w.overflow = 0; }
   // broadphase for every candidate pair at once (lane = pair): plane / bounding-sphere rejection of mj_collideGeoms
   bool cand = false;
@@ -764,7 +764,7 @@ __device__ __forceinline__ void forward_position(const DevModel& m, WS& w, const
 
 // -------------------------------------------------------------------------------- smooth dynamics
 // mj_comVel + mj_rne(flg_acc=0) + passive + actuation + xfrc -> fsmooth, asmooth.  Needs the dyn scratch from com_pos_crb.
-__device__ __noinline__ void smooth_forces(const DevModel& m, WS& w, int lane, bool actuation, float xfrc_z) {
+static __device__ __noinline__ void smooth_forces(const DevModel& m, WS& w, int lane, bool actuation, float xfrc_z) {
   const int nb = m.nbody;
   // forward pass by levels: cvel, cdof_dot, and cacc (kept in registers, written into cfrc as body force)
   if (lane == 0) for (int k = 0; k < 6; k++) { w.u.dyn.cvel[0][k] = 0; w.u.dyn.cfrc[0][k] = 0; }
@@ -842,7 +842,7 @@ __device__ __noinline__ void smooth_forces(const DevModel& m, WS& w, int lane, b
 }
 
 // -------------------------------------------------------------------------------- constraints
-__device__ __noinline__ float get_impedance(const float* solimp, float pos, float margin) {
+static __device__ __noinline__ float get_impedance(const float* solimp, float pos, float margin) {
   if (solimp[0] == solimp[1] || solimp[2] <= MINVAL) return 0.5f * (solimp[0] + solimp[1]);
   float x = fabsf((pos - margin) / solimp[2]);
   if (x >= 1) return solimp[1];
@@ -855,7 +855,7 @@ __device__ __noinline__ float get_impedance(const float* solimp, float pos, floa
 }
 
 // engine_core_constraint.c : mj_makeConstraint (limits + elliptic contacts), mj_makeImpedance, mj_referenceConstraint
-__device__ __noinline__ void make_constraint(const DevModel& m, WS& w, int lane) {
+static __device__ __noinline__ void make_constraint(const DevModel& m, WS& w, int lane) {
   // ---- joint limits: lane = joint
   bool active = false;
   float dist = 0, sign = 0;
@@ -1103,7 +1103,7 @@ __device__ __forceinline__ void make_hessian(WS& w, int lane) {
 
 // engine_solver.c : mj_solNewton (primal, elliptic cones, exact line search), fp32.
 // Returns the number of iterations. On exit w.qacc and w.fcon (= J^T f) are final.
-__device__ __noinline__ int solve_newton(const DevModel& m, WS& w, int lane, int max_iter) {
+static __device__ __noinline__ int solve_newton(const DevModel& m, WS& w, int lane, int max_iter) {
   const int nefc = w.nefc;
   float qa = 0;
   if (nefc == 0) {
@@ -1217,7 +1217,7 @@ __device__ __noinline__ int solve_newton(const DevModel& m, WS& w, int lane, int
 }
 
 // engine_forward.c : mj_Euler with implicit joint damping + mj_integratePos
-__device__ __noinline__ void euler_integrate(const DevModel& m, WS& w, int lane) {
+static __device__ __noinline__ void euler_integrate(const DevModel& m, WS& w, int lane) {
   const float h = m.timestep;
 #pragma unroll 1
   for (int e = lane; e < NV * NV; e += 32) {
@@ -1255,7 +1255,7 @@ __device__ __noinline__ void euler_integrate(const DevModel& m, WS& w, int lane)
 }
 
 // dm_control Physics.step() in legacy mode: mj_step2 on the already-computed position stage, then mj_step1.
-__device__ __noinline__ int physics_step(const DevModel& m, WS& w, const float4* hv, const int* adj, int lane, float xfrc_z, bool actuation) {
+static __device__ __noinline__ int physics_step(const DevModel& m, WS& w, const float4* hv, const int* adj, int lane, float xfrc_z, bool actuation) {
   smooth_forces(m, w, lane, actuation, xfrc_z);
   make_constraint(m, w, lane);
   int it = solve_newton(m, w, lane, m.iterations);

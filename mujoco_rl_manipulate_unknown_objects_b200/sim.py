@@ -10,7 +10,7 @@ import numpy as np
 
 from . import _native
 from ._native import INFO, DBG, GrsConfig
-from .config import make_config, scene_path
+from .config import make_config, scene_path, scene_paths
 
 NQ, NV, NU = 14, 13, 7
 
@@ -107,6 +107,11 @@ class GripperSim(CompiledModel):
     config: Namespace as produced by the reference's BaseConfig (or make_config()); `direction` is 0 or 45 as in the reference, or any other angle in degrees
     (robot_env.py:30-33).  auto_reset=True gives SB3 VecEnv semantics (an environment is reset inside the step
     that ends its episode; the terminal observation is kept in `terminal_obs`).
+
+    A list or tuple `config.sim_env` builds a mixed simulator: the scenes (variants 0..K-1, `scenes`) must differ only in the
+    object, and each environment runs one variant per episode.  `object_ids` holds the variant of every environment's current
+    episode, `next_object_ids` (writable; set_next_objects checks the values) the one its next reset starts; both start as n % K.  The model accessors (get, names,
+    sizes) answer for variant 0.
     """
 
     def __init__(self, config=None, num_envs=1, device=0, auto_reset=True, **overrides):
@@ -123,7 +128,9 @@ class GripperSim(CompiledModel):
         self.device = torch.device("cuda", self.device_index)
         lib = _native.load()
         cfg = _grs_config(config, auto_reset)
-        h = lib.grs_create(scene_path(config.sim_env).encode(), int(num_envs), C.byref(cfg), self.device_index)
+        self.scenes = scene_paths(config.sim_env)
+        paths = (C.c_char_p * len(self.scenes))(*[p.encode() for p in self.scenes])
+        h = lib.grs_create_scenes(paths, len(self.scenes), int(num_envs), C.byref(cfg), self.device_index)
         if not h:
             raise NativeError(_native.last_error())
         super().__init__(_handle=h)
@@ -136,7 +143,10 @@ class GripperSim(CompiledModel):
         N, (Cc, H, W) = self.num_envs, self.obs_shape
         self.obs = self._tensor("obs", (N, Cc, H, W), "|u1")
         self.terminal_obs = self._tensor("terminal_obs", (N, Cc, H, W), "|u1")
-        self.reset_obs = self._tensor("reset_obs", (Cc, H, W), "|u1")
+        K = lib.grs_num_scenes(h)
+        self.reset_obs = self._tensor("reset_obs", (Cc, H, W) if K == 1 else (K, Cc, H, W), "|u1")  # per variant in a mixed simulator
+        self.object_ids = self._tensor("object", (N,), "<i4")
+        self.next_object_ids = self._tensor("next_object", (N,), "<i4")
         self.reward = self._tensor("reward", (N,), "<f4")
         self.done = self._tensor("done", (N,), "|u1")
         self.achieved_goal = self._tensor("achieved", (N, 2), "<f4")
@@ -260,6 +270,19 @@ class GripperSim(CompiledModel):
         environment (row id), unchanged until the environment is sent again.  The synchronous step() need not write it."""
         N, a = self.num_envs, self.action_dim
         return self._tensor("actions", (N * 6,), "<f4")[:N * a].view(N, a)  # allocated N x 6, written with stride action_dim
+
+    def set_next_objects(self, variants, env_ids=None):
+        """Write `next_object_ids` (all environments, or those in `env_ids`) after checking that every value names a variant;
+        raises ValueError otherwise.  The check reads the values back to the host.  A value written straight into
+        next_object_ids that names no variant is ignored by the reset: the environment keeps its variant."""
+        t = self._torch
+        v = t.as_tensor(variants, device=self.device).to(t.int32)
+        if v.numel() and (int(v.min()) < 0 or int(v.max()) >= len(self.scenes)):
+            raise ValueError("next object variants must lie in 0..%d" % (len(self.scenes) - 1))
+        if env_ids is None:
+            self.next_object_ids.copy_(v.expand(self.num_envs))
+        else:
+            self.next_object_ids[t.as_tensor(env_ids, device=self.device).long()] = v
 
     @property
     def launch_count(self):

@@ -124,8 +124,9 @@ class LazyInfos(Sequence):
     stay valid until the next-but-one step() (the buffers flip every step); copy what has to live longer."""
 
     def __init__(self, rows, dones, terminal_obs, target_dir, t_start, extra=None, obs=None, prev_obs=None, episode_rewards=None,
-                 finished_rewards=None, truncation_key=False):
+                 finished_rewards=None, truncation_key=False, object_key=False):
         self._rows, self._dones, self._tobs, self._dir, self._t0 = rows, dones, terminal_obs, target_dir, t_start
+        self._object_key = object_key
         self._cache = {}
         self._extra = extra or {}
         self._obs, self._prev_obs, self._ep_rew, self._fin_rew, self._trunc = obs, prev_obs, episode_rewards, finished_rewards or {}, truncation_key
@@ -166,6 +167,8 @@ class LazyInfos(Sequence):
              "substeps": int(r[I["NSUB_A"]] + r[I["NSUB_B"]] + r[I["NSUB_C"]]),
              "achieved_goal": r[I["ACHIEVED"]:I["ACHIEVED"] + 2].copy(),
              "desired_goal": r[I["DESIRED"]:I["DESIRED"] + 2].copy()}
+        if self._object_key:  # mixed simulator: the variant (index into sim.scenes) of the episode the step belongs to
+            d["object_id"] = int(r[I["OBJECT"]])
         if done:
             if self._trunc:
                 d["TimeLimit.truncated"] = status == 2
@@ -276,7 +279,8 @@ class BatchedRobotVecEnv(_VecEnvBase):
             self._ep_rewards[idx] = 0
             self._ep_pos[idx] = 0
         infos = LazyInfos(b.info.copy() if self._copy else b.info, dones.copy() if self._copy else dones, tobs, self.target_direction, self._t_start,
-                          obs=b.obs, prev_obs=prev.obs, episode_rewards=self._ep_rewards, finished_rewards=finished, truncation_key=self._trunc)
+                          obs=b.obs, prev_obs=prev.obs, episode_rewards=self._ep_rewards, finished_rewards=finished, truncation_key=self._trunc,
+                          object_key=len(self.sim.scenes) > 1)
         if self._monitor is not None and tobs is not None:
             self._monitor.write_step(dones, infos)
         return self._obs_dict(b), (b.rew.copy() if self._copy else b.rew), (dones.copy() if self._copy else dones), infos

@@ -29,7 +29,7 @@ from mujoco_rl_manipulate_unknown_objects_b200.rollout import RolloutWorker, dis
 from mujoco_rl_manipulate_unknown_objects_b200.sac import SACLearner
 
 ap = argparse.ArgumentParser()
-ap.add_argument("--scene", default="sugar_cube"); ap.add_argument("--envs", type=int, default=4096); ap.add_argument("--capacity", type=int, default=128)
+ap.add_argument("--scene", default="sugar_cube", help="scene name, or several comma-separated for one mixed simulator"); ap.add_argument("--envs", type=int, default=4096); ap.add_argument("--capacity", type=int, default=128)
 ap.add_argument("--steps", type=int, default=16); ap.add_argument("--iters", type=int, default=3); ap.add_argument("--gradient-steps", type=int, default=16)
 ap.add_argument("--batch", type=int, default=256); ap.add_argument("--her-ratio", type=float, default=0.8); ap.add_argument("--launches", type=int, default=50)
 ap.add_argument("--pool-batch", type=int, default=0, help="run the asynchronous pool with this batch size (0: the synchronous step)")
@@ -43,7 +43,8 @@ if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     else:
         dist.init_process_group("gloo")
-cfg = make_config(sim_env="/xmls/%s_env.xml" % a.scene, her_buffer=True)
+scenes = ["/xmls/%s_env.xml" % x for x in a.scene.split(",")]  # several, comma-separated: one mixed simulator
+cfg = make_config(sim_env=scenes[0] if len(scenes) == 1 else scenes, her_buffer=True)
 plain = RolloutWorker(cfg, envs_per_gpu=a.envs, device=local, seed=0)
 w = RolloutWorker(cfg, envs_per_gpu=a.envs, device=local, seed=0)
 N, obs_shape, A = a.envs, w.sim.obs_shape, w.sim.action_dim
