@@ -925,7 +925,7 @@ static uint16_t f2bf(float f) {  // round to nearest even
   return (uint16_t)(u >> 16);
 }
 
-static uint16_t f2h(float f) {  // fp32 -> fp16, round to nearest even (conv1 weights; magnitudes far inside the normal range)
+static uint16_t f2h(float f) {  // fp32 -> fp16, round to nearest even, subnormals included (conv1 weights; grp_set_params refuses |w| >= 65520)
   uint32_t u;
   std::memcpy(&u, &f, 4);
   const uint32_t sign = (u >> 16) & 0x8000u;
@@ -1092,6 +1092,16 @@ extern "C" int32_t grp_set_params(grp_policy* p, const float* host, int64_t coun
     const Shape& s = p->sh;
     const ParamLayout L = layout_of(s);
     if (count != L.total) throw std::runtime_error("parameter count mismatch: expected " + std::to_string(L.total) + ", got " + std::to_string(count));
+    // conv1 multiplies in fp16: a weight that rounds to +-inf there (or is not finite) would make every action NaN.  Refused
+    // before anything is overwritten, so the policy keeps its previous parameters.
+    for (int64_t i = 0; i < 32LL * s.cin * 64; i++) {
+      const float w = host[L.c1w + i];
+      if (!(std::fabs(w) < 65520.0f)) {
+        const int64_t o = i / (s.cin * 64), c = i / 64 % s.cin, ky = i / 8 % 8, kx = i % 8;
+        throw std::runtime_error("features_extractor.cnn.0.weight[" + std::to_string(o) + ", " + std::to_string(c) + ", " + std::to_string(ky) + ", " +
+                                 std::to_string(kx) + "] = " + std::to_string(w) + " is outside the fp16 range conv1 computes in (|w| < 65520)");
+      }
+    }
     CU(cudaSetDevice(p->device));
     CU(cudaStreamSynchronize(p->stream));
     std::memcpy(p->params.data(), host, (size_t)count * 4);
