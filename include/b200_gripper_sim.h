@@ -40,7 +40,7 @@ typedef struct grs_config {
   int32_t her_buffer;       /* base_config.py:39  add exp(-|dg-ag|), robot_env.py:268-271 */
   int32_t direction;        /* base_config.py:42  0 -> (1,0), 45 -> (1,1), robot_env.py:30-33; any other angle (degrees) -> the unit
                                vector of the reference's disabled `_get_direction`, robot_env.py:46-54 */
-  int32_t width, height;    /* base_config.py:18-19 observation size (64 x 64) */
+  int32_t width, height;    /* base_config.py:18-19 observation size (64 x 64); each within 1..64, grs_create refuses more */
   int32_t auto_reset;       /* SB3 VecEnv semantics: reset an environment in the step that ends its episode */
   float pos_tolerance;      /* base_config.py:32 (0.002) */
   float grasp_tolerance;    /* base_config.py:31 (0.03) */

@@ -237,13 +237,19 @@ static __global__ void k_order_envs(SimBuffers s, const float* __restrict__ acti
   s.done_list[env] = -1;
 }
 
-// Launch bounds (320 threads, 2 blocks per SM) cap the kernel at 96 registers.  Measured in the steady state of the bench
-// workload (profiles/r2e_warps_regs_ab.log, r2f_regs.log): 113-120 registers (bounds 512, 1) 18.2 M substeps/s, 96 registers
-// 19.1 M, 80 registers 18.4 M, 72 registers 17.4 M, 64 registers 17.2 M; the stack frame grows by only 40 bytes at 96.
+// Launch bounds (320 threads, 2 blocks per SM) are a register cap, not a block width: they hold the kernel at 96 registers,
+// while every launch uses LS_WARPS * 32 = 256 threads (bounds of 256 x 2 would allow 128 registers).  Measured in the steady
+// state of the bench workload (profiles/r2e_warps_regs_ab.log, r2f_regs.log): 113-120 registers (bounds 512, 1) 18.2 M
+// substeps/s, 96 registers 19.1 M, 80 registers 18.4 M, 72 registers 17.4 M, 64 registers 17.2 M; the stack frame grows by
+// only 40 bytes at 96.
 constexpr int LS_MAX_THREADS = 320, LS_MIN_BLOCKS = 2;
+// Warps (= environments in flight) per block: the optimum between barrier max-ing (more warps) and instruction-cache diversity
+// (more blocks per SM), profiles/r2m_sweep.log.  The observation phase runs on the same blocks: it needs RTHREADS threads and
+// reuses the workspaces' shared memory for its tile.
+constexpr int LS_WARPS = 8;
+static_assert(LS_WARPS * 32 == RTHREADS, "the observation phase needs blocks of RTHREADS threads");
+static_assert(LS_WARPS * sizeof(WS) >= render_phase_smem_bytes(), "the observation tile must fit in the step kernel's shared memory");
 
-// TIMING = true: per-stage clock64 bookkeeping (sum over warps vs. per-round block maximum) into s.debug — a development
-// aid behind GRS_STEP_TIMING=1 that quantifies what the block barriers cost; the production instantiation carries none of it.
 __device__ __forceinline__ unsigned long long global_ns() {
   unsigned long long t;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -306,18 +312,18 @@ __device__ __forceinline__ void resume_env(const AsyncArgs& aa, WS& w, EnvCtl& t
   __syncwarp();
 }
 
-// FUSED = true: a block whose physics work is exhausted goes on to build observations (render_phase) instead of exiting, so
-// the rasteriser fills the SMs that idle while the longest substep chains finish.  Needs blockDim.x == RTHREADS.
-// ASYNC = true: the asynchronous step above (not FUSED: the observation phase would wait for environments that get parked).
+// Launched with LS_WARPS warps per block.  ASYNC = false, the synchronous step: a block whose physics work is exhausted goes on
+// to build observations (render_phase) instead of exiting, so the rasteriser fills the SMs that idle while the longest substep
+// chains finish, and the physics phase is timed on the device.  ASYNC = true: the asynchronous step above, without either (the
+// observation phase would wait for environments that get parked; k_render_obs_indexed renders its finished environments).
 // MULTI = true: a mixed simulator (SimBuffers::nobj > 1); each warp runs the model of its environment's variant.  The
 // single-scene instantiation keeps the model at a constant shared-memory address; the MULTI ones are compiled in
 // multi_kernels.cu only (see SimKernels below).
-template <bool TIMING, bool FUSED, bool ASYNC = false, bool MULTI = false>
+template <bool ASYNC, bool MULTI>
 __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(SimBuffers s, EnvCfg c, const float* __restrict__ actions, int adim, RenderScene sc, ObsArgs oa,
                                                                                   AsyncArgs aa) {
-  static_assert(!(ASYNC && (FUSED || TIMING)), "the asynchronous step has its own instantiation");
   unsigned smid = 0;
-  if (FUSED && threadIdx.x == 0) {
+  if (!ASYNC && threadIdx.x == 0) {
     atomicMin(s.tstamp, global_ns());
     atomicAdd(s.queue + 6, 1);  // blocks of this launch that are resident (render_phase)
     asm("mov.u32 %0, %%smid;" : "=r"(smid));
@@ -352,17 +358,6 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
   const DevModel* mp = &smem_model(0);  // the model of the warp's current environment (its variant, set when it is loaded)
   WS& w = my_ws(MULTI ? s.nobj : 1);
   const int lane = threadIdx.x & 31;
-  __shared__ unsigned long long t_sum[8], t_max[8], t_round[8];
-  __shared__ unsigned long long t_rounds, t_lone[8], t_lone_rounds;  // rounds in which exactly one warp of the block was active
-  __shared__ unsigned int t_hist[12];  // rounds with k active warps (k = 0..11)
-  __shared__ unsigned long long t_cyc[12];  // ... and the cycles they took
-  long long t_prev = 0;
-  int prev_active = 0;
-  const long long t_block0 = TIMING ? clock64() : 0;
-  if (TIMING) { if (threadIdx.x < 8) { t_sum[threadIdx.x] = 0; t_max[threadIdx.x] = 0; t_round[threadIdx.x] = 0; } if (threadIdx.x == 0) { t_rounds = 0; t_lone_rounds = 0; } if (threadIdx.x < 8) t_lone[threadIdx.x] = 0; if (threadIdx.x < 12) { t_hist[threadIdx.x] = 0; t_cyc[threadIdx.x] = 0; } __syncthreads(); }
-  long long t0 = 0;
-#define LS_T0() if (TIMING) t0 = clock64();
-#define LS_T1(p) if (TIMING) { unsigned long long d_ = (unsigned long long)(clock64() - t0); if (lane == 0) { atomicAdd(&t_sum[p], d_); atomicMax(&t_round[p], d_); } }
   EnvCtl t;
   t.stage = S_IDLE; t.env = -1;
   bool exhausted = false, first = true;
@@ -370,7 +365,6 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
 #pragma unroll 1
   for (;;) {
     // ---- controller round: finish / fetch / decide (per warp, no block-wide dependency)
-    LS_T0();
     bool dyn = false, pos = false, stop = false;
     if constexpr (ASYNC) {
       // stop rule: once `need` environments have finished in this launch (s.queue[3] counts them), nothing new is fetched and
@@ -425,35 +419,16 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
       }
     }
     pos = pos || dyn;
-    LS_T1(0);
-    const int n_active = TIMING ? __syncthreads_count(pos) >> 5 : __syncthreads_or(pos);
-    if (!n_active) break;
-    if (TIMING && threadIdx.x == 0) {
-      for (int p = 0; p < 8; p++) { t_max[p] += t_round[p]; if (prev_active == 1) t_lone[p] += t_round[p]; t_round[p] = 0; }
-      t_rounds++;
-      t_hist[min(n_active, 11)]++;
-      const long long now = clock64();
-      if (t_prev) t_cyc[min(prev_active, 11)] += (unsigned long long)(now - t_prev);  // the round that just ended ran with prev_active warps
-      t_prev = now;
-      if (prev_active == 1) t_lone_rounds++;
-    }
-    prev_active = n_active;
+    if (!__syncthreads_or(pos)) break;
     const DevModel& m = *mp;
     // ---- the substep pipeline, stage by stage, whole block in step (dm_control legacy step: mj_step2 then mj_step1)
-    LS_T0();
     if (dyn) smooth_forces(m, w, lane, true, t.f.xfrc_z);
-    LS_T1(1);
     // block barriers after the constraint rows, the Newton solve and CRB only (profiles/r2m_sweep.log: none 5 % slower)
-    LS_T0();
     if (dyn) make_constraint(m, w, lane);
-    LS_T1(2);
     __syncthreads();
     iters = 0;
-    LS_T0();
     if (dyn) iters = solve_newton(m, w, lane, m.iterations);
-    LS_T1(3);
     __syncthreads();
-    LS_T0();
     if (dyn) euler_integrate(m, w, lane);
     if constexpr (ASYNC) {
       if (pos) {  // PK_QPOS: what this position stage starts from, for a resume after a park in the next round
@@ -463,16 +438,11 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
       }
     }
     if (pos) kinematics(m, w, lane);
-    LS_T1(4);
-    LS_T0();
     if (pos) com_pos_crb(m, w, lane);
-    LS_T1(5);
     __syncthreads();
-    LS_T0();
     if (pos) collision(m, w, hull, s.adj, lane);
-    LS_T1(6);
   }
-  if (FUSED) {
+  if constexpr (!ASYNC) {
     if (threadIdx.x == 0) {  // end of this block's physics phase
       atomicMax(s.tstamp + 1, global_ns());
       atomicSub(s.sm_phys + (smid & 255), 1);
@@ -487,22 +457,6 @@ __global__ void __launch_bounds__(LS_MAX_THREADS, LS_MIN_BLOCKS) k_env_step_ls(S
       }
     }
   }
-  if (TIMING) {
-    __syncthreads();
-    if (threadIdx.x < 8) {
-      s.debug[(size_t)blockIdx.x * 32 + threadIdx.x] = (float)t_sum[threadIdx.x] / (float)(blockDim.x >> 5);
-      s.debug[(size_t)blockIdx.x * 32 + 8 + threadIdx.x] = (float)t_max[threadIdx.x];
-    }
-    if (threadIdx.x == 0) { s.debug[(size_t)blockIdx.x * 32 + 16] = (float)t_rounds; s.debug[(size_t)blockIdx.x * 32 + 17] = (float)t_lone_rounds; }
-    if (threadIdx.x < 8) s.debug[(size_t)blockIdx.x * 32 + 18 + threadIdx.x] = (float)t_lone[threadIdx.x];
-    // block-level record (second half of the debug buffer): physics-phase duration in cycles, then rounds with k active warps
-    float* bd = s.debug + (size_t)gridDim.x * 32 + (size_t)blockIdx.x * 32;
-    if (threadIdx.x == 0) { bd[0] = (float)(clock64() - t_block0); if (t_prev) t_cyc[min(prev_active, 11)] += (unsigned long long)(clock64() - t_prev); }
-    __syncthreads();
-    if (threadIdx.x >= 1 && threadIdx.x < 13) { bd[threadIdx.x] = (float)t_hist[threadIdx.x - 1]; bd[12 + threadIdx.x] = (float)t_cyc[threadIdx.x - 1]; }
-  }
-#undef LS_T0
-#undef LS_T1
 }
 
 // ---- the small kernels around the asynchronous step (grs_async_* in gripper_sim.cu)
@@ -588,7 +542,7 @@ static __global__ void k_async_recv(SimBuffers s, AsyncArgs aa, int* __restrict_
 // single-scene step kernel's narrowphase callees spill (DESIGN.md §3.6).
 using StepKernel = void (*)(SimBuffers, EnvCfg, const float*, int, RenderScene, ObsArgs, AsyncArgs);
 struct SimKernels {
-  StepKernel step, step_fused, step_timing, step_async;
+  StepKernel step, step_async;
   void (*make_reset_record)(SimBuffers, EnvCfg);
   void (*substep)(SimBuffers, int);
   void (*contacts)(SimBuffers);
@@ -597,9 +551,8 @@ struct SimKernels {
 };
 template <bool MULTI>
 inline SimKernels sim_kernels() {
-  return SimKernels{k_env_step_ls<false, false, false, MULTI>, k_env_step_ls<false, true, false, MULTI>, k_env_step_ls<true, false, false, MULTI>,
-                    k_env_step_ls<false, false, true, MULTI>, k_make_reset_record<MULTI>, k_substep<MULTI>, k_contacts<MULTI>, k_debug_step<MULTI>,
-                    k_camera_state<MULTI>};
+  return SimKernels{k_env_step_ls<false, MULTI>, k_env_step_ls<true, MULTI>, k_make_reset_record<MULTI>, k_substep<MULTI>, k_contacts<MULTI>,
+                    k_debug_step<MULTI>, k_camera_state<MULTI>};
 }
 SimKernels multi_sim_kernels();  // sim_kernels<true>(), multi_kernels.cu
 

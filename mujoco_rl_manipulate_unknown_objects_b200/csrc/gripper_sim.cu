@@ -6,7 +6,6 @@
 #include <cuda_runtime.h>
 
 #include <cmath>
-#include <cstdlib>
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
@@ -79,10 +78,8 @@ struct grs_sim {
   long ms_cnt = 0;
   int grid = 0;
   size_t smem = 0;
-  // step kernel geometry (GRS_STEP_WARPS warps per block)
-  int ls_warps = 8, ls_grid = 0;
-  bool ls_timing = false;
-  bool fused_render = false;  // observation phase inside the step kernel (env_lockstep.cuh : render_phase)
+  // step kernel geometry (LS_WARPS warps per block)
+  int ls_grid = 0;
   size_t ls_smem = 0;
   SimKernels kern{};  // single-scene or mixed-simulator instantiations (env_lockstep.cuh)
   ObsArgs obs_args{};
@@ -145,7 +142,8 @@ extern "C" grs_sim* grs_create_scenes(const char* const* xml_paths, int32_t coun
     grs_config cfg;
     if (cfg_in) cfg = *cfg_in; else grs_default_config(&cfg);
     if (cfg.direction < -360 || cfg.direction > 360) throw std::runtime_error("direction must be an angle in degrees within [-360, 360] (robot_env.py:30-33: 0 and 45 are the reference's cases)");
-    if (cfg.width <= 0 || cfg.height <= 0 || cfg.width > 256 || cfg.height > 256) throw std::runtime_error("observation size must be within 1..256");
+    // the observation is one rasteriser tile
+    if (cfg.width <= 0 || cfg.height <= 0 || cfg.width > TILE || cfg.height > TILE) throw std::runtime_error("observation size must be within 1.." + std::to_string(TILE));
     if (cfg.max_steps <= 0 || cfg.time_horizon <= 0) throw std::runtime_error("max_steps and time_horizon must be positive");
     int ndev = 0;
     cudaError_t ce = cudaGetDeviceCount(&ndev);
@@ -259,33 +257,25 @@ extern "C" grs_sim* grs_create_scenes(const char* const* xml_paths, int32_t coun
     int want = (num_envs + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
     s->grid = std::min(want, per_sm * nsm);
     // step kernel geometry
-    if (const char* e = getenv("GRS_STEP_WARPS")) s->ls_warps = std::max(1, std::min(LS_MAX_THREADS / 32, atoi(e)));
-    s->ls_smem = (size_t)K * MODEL_BYTES + (size_t)s->ls_warps * sizeof(WS);
+    s->ls_smem = (size_t)K * MODEL_BYTES + (size_t)LS_WARPS * sizeof(WS);
     {
       int optin = 0;
       CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
       if (s->ls_smem > (size_t)optin)
-        throw std::runtime_error(std::to_string(K) + " models and " + std::to_string(s->ls_warps) + " workspaces need " + std::to_string(s->ls_smem) +
+        throw std::runtime_error(std::to_string(K) + " models and " + std::to_string(LS_WARPS) + " workspaces need " + std::to_string(s->ls_smem) +
                                  " bytes of shared memory per block, more than the device's " + std::to_string(optin));
     }
     {
       // hull vertices in shared memory when two blocks per SM still fit (227 KB per block, 228 KB per SM, 1 KB reserved each)
       const size_t with_hull = s->ls_smem + (size_t)s->b.hull_count * sizeof(float4);
-      const bool want = getenv("GRS_HULL_SMEM") ? atoi(getenv("GRS_HULL_SMEM")) != 0 : true;
-      if (want && 2 * (with_hull + 1024) <= 228 * 1024) { s->ls_smem = with_hull; s->b.hull_smem = 1; }
+      if (2 * (with_hull + 1024) <= 228 * 1024) { s->ls_smem = with_hull; s->b.hull_smem = 1; }
     }
-    s->ls_timing = getenv("GRS_STEP_TIMING") != nullptr;
-    // the observation phase needs RTHREADS-wide blocks and the observation tile in the block's shared memory
-    s->fused_render = !s->ls_timing && s->ls_warps * 32 == RTHREADS && s->ls_smem >= render_phase_smem_bytes() && cfg.width <= TILE && cfg.height <= TILE;
-    if (const char* e = getenv("GRS_FUSED_RENDER")) s->fused_render = s->fused_render && atoi(e) != 0;
     raise_dyn_smem((const void*)kn.step, s->ls_smem, device);
-    raise_dyn_smem((const void*)kn.step_fused, s->ls_smem, device);
-    raise_dyn_smem((const void*)kn.step_timing, s->ls_smem, device);
     raise_dyn_smem((const void*)kn.step_async, s->ls_smem, device);
     int ls_per_sm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, s->fused_render ? kn.step_fused : kn.step, s->ls_warps * 32, s->ls_smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ls_per_sm, kn.step, LS_WARPS * 32, s->ls_smem));
     if (ls_per_sm < 1) throw std::runtime_error("step kernel does not fit on this device");
-    s->ls_grid = std::min((num_envs + s->ls_warps - 1) / s->ls_warps, ls_per_sm * nsm);
+    s->ls_grid = std::min((num_envs + LS_WARPS - 1) / LS_WARPS, ls_per_sm * nsm);
     for (int i = 0; i < grs_sim::NEV; i++) { CU(cudaEventCreate(&s->ev0[i])); CU(cudaEventCreate(&s->ev1[i])); }
     render_scene_upload(hms, s->scene, s->owned);
     // the reset record and the observation of a freshly reset environment of each variant (identical for every env and every episode)
@@ -400,12 +390,10 @@ extern "C" int32_t grs_step(grs_sim* s, const float* actions_dev, void* stream) 
     k_order_count<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
     k_order_envs<<<(s->n + 255) / 256, 256, 0, st>>>(s->b, actions_dev, s->adim);
     s->launches += 2;
-    const StepKernel k = s->fused_render ? s->kern.step_fused : s->ls_timing ? s->kern.step_timing : s->kern.step;
-    k<<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
+    s->kern.step<<<s->ls_grid, LS_WARPS * 32, s->ls_smem, st>>>(s->b, s->ecfg, actions_dev, s->adim, s->scene, s->obs_args, AsyncArgs{});
     CU(cudaGetLastError());
     CU(cudaEventRecord(s->ev1[s->ev_n], st));
     s->ev_n++;
-    if (!s->fused_render) { launch_render_obs(s->scene, s->obs_args, s->b.render_state, s->b.info, s->b.done, s->b.reward, s->n, st); s->launches++; }
     s->launches += 1;
     return 0;
   } catch (const std::exception& e) { return fail(e.what()); }
@@ -414,7 +402,7 @@ extern "C" int32_t grs_step(grs_sim* s, const float* actions_dev, void* stream) 
 // Device-visible address of a caller's host buffer if it is page-locked (cudaHostAlloc / cudaHostRegister, e.g. torch's
 // pin_memory()): the observation phase then stores finished observations straight into it.  NULL for pageable memory.
 static unsigned char* mapped_host_ptr(void* host) {
-  if (!host || getenv("GRS_NO_HOST_MIRROR")) return nullptr;
+  if (!host) return nullptr;
   cudaPointerAttributes a{};
   if (cudaPointerGetAttributes(&a, host) != cudaSuccess) { cudaGetLastError(); return nullptr; }
   if (a.type != cudaMemoryTypeHost || !a.devicePointer) return nullptr;
@@ -688,7 +676,7 @@ extern "C" int64_t grs_model_get_int(const grs_sim* s, const char* name, int32_t
     else if (k == "iterations") tmp = {m.iterations};
     else if (k == "cone_elliptic") tmp = {m.cone_elliptic};
     else if (k == "named_bodies") tmp = {m.body_ee, m.body_object, m.finger1[0], m.finger1[1], m.finger2[0], m.finger2[1]};
-    else if (k == "step_smem" && !s->compile_only) tmp = {(int)s->ls_smem, s->b.hull_smem, s->b.hull_count, s->ls_warps};
+    else if (k == "step_smem" && !s->compile_only) tmp = {(int)s->ls_smem, s->b.hull_smem, s->b.hull_count, LS_WARPS};
     else if (k.rfind("hull_adjadr:", 0) == 0 || k.rfind("hull_adj:", 0) == 0 || k.rfind("hull_faces:", 0) == 0) {
       std::string mn = k.substr(k.find(':') + 1);
       const HostMesh* hm = nullptr;
@@ -745,15 +733,16 @@ extern "C" float grs_step_kernel_ms(grs_sim* s, int32_t reset_counters) {
   cudaSetDevice(s->device);
   harvest_events(s);
   float avg = s->ms_cnt ? (float)(s->ms_sum / s->ms_cnt) : 0.0f;
-  if (s->fused_render) {
-    // fused kernel: the physics phase is timed on the device (globaltimer: first block start -> last block leaving the
-    // substep loop, accumulated by the last block of every launch); the events above cover physics + observation phases
-    unsigned long long t[4] = {0, 0, 0, 0};
-    if (cudaStreamSynchronize(s->stream) == cudaSuccess && cudaMemcpy(t, s->b.tstamp, sizeof t, cudaMemcpyDeviceToHost) == cudaSuccess && t[3])
-      avg = (float)((double)t[2] / (double)t[3] * 1e-6);
-    if (reset_counters) cudaMemset(s->b.tstamp + 2, 0, 2 * sizeof(unsigned long long));
+  // the synchronous step kernel times its physics phase on the device (globaltimer: first block start -> last block leaving the
+  // substep loop, accumulated by the last block of every launch); the events above cover physics + observation phases and are
+  // the answer when only asynchronous launches ran since the last reset
+  unsigned long long t[4] = {0, 0, 0, 0};
+  if (cudaStreamSynchronize(s->stream) == cudaSuccess && cudaMemcpy(t, s->b.tstamp, sizeof t, cudaMemcpyDeviceToHost) == cudaSuccess && t[3])
+    avg = (float)((double)t[2] / (double)t[3] * 1e-6);
+  if (reset_counters) {
+    cudaMemset(s->b.tstamp + 2, 0, 2 * sizeof(unsigned long long));
+    s->ms_sum = 0; s->ms_cnt = 0;
   }
-  if (reset_counters) { s->ms_sum = 0; s->ms_cnt = 0; }
   return avg;
 }
 
@@ -814,7 +803,7 @@ extern "C" int32_t grs_async_recv(grs_sim* s, int32_t* out_ids_dev, void* stream
     k_async_order_envs<<<g, 256, 0, st>>>(s->b, s->aa, s->d_actions, s->adim, B);
     if (s->ev_n == grs_sim::NEV) harvest_events(s);
     CU(cudaEventRecord(s->ev0[s->ev_n], st));
-    s->kern.step_async<<<s->ls_grid, s->ls_warps * 32, s->ls_smem, st>>>(s->b, s->ecfg, s->d_actions, s->adim, s->scene, s->obs_args, s->aa);
+    s->kern.step_async<<<s->ls_grid, LS_WARPS * 32, s->ls_smem, st>>>(s->b, s->ecfg, s->d_actions, s->adim, s->scene, s->obs_args, s->aa);
     CU(cudaGetLastError());
     CU(cudaEventRecord(s->ev1[s->ev_n], st));
     s->ev_n++;

@@ -580,8 +580,8 @@ __device__ __forceinline__ void render_obs_env(const RenderScene& sc, const ObsA
 }
 
 // Standalone observation kernel: one block per environment.  info: per-env info rows; done: per-env done flags (NULL for
-// the reset image).  Used for the reset image and whenever the step kernel runs without its observation phase
-// (GRS_FUSED_RENDER=0, GRS_STEP_TIMING, other block widths than RTHREADS).
+// the reset image).  Renders the reset images; the synchronous step builds its observations in the step kernel's observation
+// phase (render_phase) and the asynchronous one with k_render_obs_indexed.
 static __global__ void __launch_bounds__(RTHREADS) k_render_obs(RenderScene sc, ObsArgs o, const float* __restrict__ render_state, const float* __restrict__ info, int info_stride,
                                                         const unsigned char* __restrict__ done, float* __restrict__ reward) {
   extern __shared__ __align__(16) unsigned char rsm[];
@@ -624,8 +624,8 @@ static __global__ void __launch_bounds__(RTHREADS) k_render_reset(RenderScene sc
   if (o.hist_prev) for (int i = threadIdx.x; i < 512; i += RTHREADS) o.hist_prev[(size_t)env * 512 + i] = (float)(&sh.hist[0][0])[i];
 }
 
-inline size_t render_smem_bytes() { return sizeof(TileShared) + TILE * TILE * sizeof(unsigned); }
-inline size_t render_phase_smem_bytes() { return render_smem_bytes() + RS_STRIDE * sizeof(float); }
+constexpr size_t render_smem_bytes() { return sizeof(TileShared) + TILE * TILE * sizeof(unsigned); }
+constexpr size_t render_phase_smem_bytes() { return render_smem_bytes() + RS_STRIDE * sizeof(float); }
 
 // Observation phase of the fused step kernel (env_lockstep.cuh).  A block whose physics work is exhausted turns into an
 // observation builder: it takes tickets from a global counter and renders environments in the order in which their
@@ -682,7 +682,6 @@ __device__ __forceinline__ void render_phase(const RenderScene& sc, const ObsArg
 // obs == reset image path: done = NULL, n = 1, hist_prev = NULL -> histograms go to hist_reset
 inline void launch_render_obs(const RenderScene& sc, const ObsArgs& o, const float* render_state, const float* info, const unsigned char* done, float* reward, int n,
                               cudaStream_t st) {
-  if (o.W > TILE || o.H > TILE) throw std::runtime_error("observation size above 64x64 is not supported by the fused observation kernel");
   static bool attr_dev[64] = {};
   int dev_ = 0;
   cudaGetDevice(&dev_);

@@ -66,6 +66,19 @@ def test_no_cpu_fallback():
     assert lib.grp_create(2, 5, 64, 64, 6, 0) is None and b"CUDA" in lib.grp_last_error()
 
 
+def test_create_refuses_observations_larger_than_one_tile():
+    """The observation is rasterised as one 64 x 64 tile: a larger width or height is refused by the configuration checks,
+    before the device is looked at (so with or without a GPU)."""
+    from mujoco_rl_manipulate_unknown_objects_b200 import _native
+    lib = _native.load()
+    for w, h in ((65, 64), (64, 65), (0, 64)):
+        c = _native.GrsConfig()
+        lib.grs_default_config(C.byref(c))
+        c.width, c.height = w, h
+        assert lib.grs_create(b"/xmls/sugar_cube_env.xml", 2, C.byref(c), 0) is None
+        assert b"observation size must be within 1..64" in lib.grs_last_error(), lib.grs_last_error()
+
+
 def test_config_struct_layout_is_the_same_in_header_binding_and_integration_stub():
     """grs_config is passed by pointer: the header, the package's ctypes binding and the stub shown in INTEGRATION.md must list the
     same fields in the same order with the same types, and the defaults of the trailing (non-reference) fields must be neutral."""

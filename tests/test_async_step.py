@@ -44,7 +44,10 @@ CASES = [("acorn", 4096, 1024, {}), ("acorn", 512, 64, {}), ("acorn", 512, 1, {}
 @pytest.mark.parametrize("scene,n,batch,extra", CASES, ids=["%s-%d-%d%s" % (c[0], c[1], c[2], "-im-noise-45" if c[3] else "") for c in CASES])
 def test_async_transitions_equal_synchronous_steps(scene, n, batch, extra):
     """A fixed action tape tape[k, e]; environment e's k-th send uses tape[k, e].  Its first K returned transitions must be
-    bit-equal to row e of the synchronous steps 1..K (time_horizon=2, so auto-resets and terminal observations are covered)."""
+    bit-equal to row e of the synchronous steps 1..K (time_horizon=2, so auto-resets and terminal observations are covered).
+    The synchronous step builds its observations in the step kernel's fused observation phase, the pool with the standalone
+    observation kernel (k_render_obs_indexed), so this also holds the two observation paths against each other, terminal_obs
+    included."""
     import torch
     from mujoco_rl_manipulate_unknown_objects_b200 import AsyncGripperEnv
     K = 4

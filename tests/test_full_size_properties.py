@@ -1,10 +1,11 @@
 """GPU: size-independent properties at BASELINE.json's full batch sizes (4 096 and 8 192 environments per GPU), where
 the fp64 oracle is too slow to follow.
 
-* scheduling independence: which warp / block / wave integrates an environment, in which order environments leave the
-  work queue (longest-first order, 8 or 10 warps per block), and whether the observation is built by the fused phase
-  or by the standalone kernel must not change a single bit of any output;
+* scheduling independence: which warp / block / wave integrates an environment and in which order environments leave the
+  work queue (longest-first order; a permutation of the environments moves each to another queue position, warp and
+  block) must not change a single bit of any output;
 * determinism: two runs of the same action tape are bit-identical; identical environments stay identical;
+* host path: grs_step_host into pageable and into pinned host arrays returns what the device step computes, bit for bit;
 * conservation-style sanity: every environment takes between 1 and 3 x max_steps substeps, finite state, rewards in
   the progress reward's range [0, 3] (reward.py:18-41 with the unreachable bonus gate), done only on the time limit
   or FAIL.
@@ -17,7 +18,8 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 
-def _run(n, scene, steps, env=None, seed=0):
+def _run(n, scene, steps, env=None, seed=0, perm=None):
+    """`steps` agent steps of a seeded action tape; with `perm`, environment j takes the actions of environment perm[j]"""
     import torch
     from mujoco_rl_manipulate_unknown_objects_b200 import GripperSim, make_config
     old = {k: os.environ.get(k) for k in (env or {})}
@@ -33,7 +35,8 @@ def _run(n, scene, steps, env=None, seed=0):
     gen = torch.Generator(device="cuda").manual_seed(seed)
     out = []
     for _ in range(steps):
-        sim.step(torch.rand((n, 6), device="cuda", generator=gen) * 2 - 1)
+        a = torch.rand((n, 6), device="cuda", generator=gen) * 2 - 1
+        sim.step(a if perm is None else a[perm])
         out.append(dict(obs=sim.obs.clone(), reward=sim.reward.clone(), done=sim.done.clone(), info=sim.info.clone(), state=sim.state.clone(),
                         ag=sim.achieved_goal.clone(), tobs=sim.terminal_obs.clone()))
     sim.close()
@@ -45,19 +48,67 @@ def test_results_do_not_depend_on_scheduling(n, scene):
     import torch
     steps = 4 if n <= 8192 else 3
     base = _run(n, scene, steps)
-    # 10 warps per block hands the queue entries to other warps and blocks; GRS_GAP_SKIP=0 evaluates every cached separating
-    # axis instead of skipping those whose separation budget is still positive (sim_kernels.cuh : collision) — the skip is
-    # exact, so not a bit may change
-    variants = (dict(GRS_FUSED_RENDER="0"), dict(GRS_STEP_WARPS="10", GRS_HULL_SMEM="0"), dict(GRS_GAP_SKIP="0", GRS_NO_HOST_MIRROR="1"))
-    for env in (variants if n <= 8192 else variants[1:]):
-        other = _run(n, scene, steps, env)
-        for t in range(steps):
-            for k in base[t]:
-                assert torch.equal(base[t][k], other[t][k]), "%s differs at step %d under %s" % (k, t, env)
+    # permuted environments: with the default (zero) reset noise a reset does not depend on the environment id, so environment
+    # j of the second run is environment perm[j] of the first, now at another queue position and in another warp and block
+    perm = torch.randperm(n, generator=torch.Generator().manual_seed(7)).cuda()
+    other = _run(n, scene, steps, perm=perm)
+    for t in range(steps):
+        for k in base[t]:
+            assert torch.equal(base[t][k][perm], other[t][k]), "%s differs at step %d with the environments permuted" % (k, t)
+    # GRS_GAP_SKIP=0 evaluates every cached separating axis instead of skipping those whose separation budget is still positive
+    # (sim_kernels.cuh : collision) — the skip is exact, so not a bit may change
+    other = _run(n, scene, steps, dict(GRS_GAP_SKIP="0"))
+    for t in range(steps):
+        for k in base[t]:
+            assert torch.equal(base[t][k], other[t][k]), "%s differs at step %d with GRS_GAP_SKIP=0" % (k, t)
     again = _run(n, scene, steps)
     for t in range(steps):
         for k in base[t]:
             assert torch.equal(base[t][k], again[t][k]), "run-to-run difference in %s at step %d" % (k, t)
+
+
+def test_host_step_equals_device_step():
+    """grs_step_host copies the outputs into pageable host arrays after the step kernel, while into pinned arrays the
+    observation phase stores each image itself as it finishes.  Both must return what the device step leaves in its buffers.
+    The copy of the terminal observations takes the done rows one by one when at most N/8 environments are done and the
+    whole array otherwise; the tape reaches both (time_horizon=2, every 16th environment starts one step before it)."""
+    import torch
+    from mujoco_rl_manipulate_unknown_objects_b200 import GripperSim, make_config
+    from mujoco_rl_manipulate_unknown_objects_b200._native import INFO as I
+    n, th = 4096, 2
+    sims = [GripperSim(make_config(sim_env="/xmls/acorn_env.xml", time_horizon=th), num_envs=n, auto_reset=True) for _ in range(3)]
+    for s in sims:
+        flags = s.get_state()["flags"]
+        flags[::16, 1] = th - 1  # episode step
+        s.set_state(flags=flags)
+    Cc, H, W = sims[0].obs_shape
+
+    def host_arrays(alloc):
+        return dict(obs=alloc((n, Cc, H, W), np.uint8), achieved=alloc((n, 2), np.float32), desired=alloc((n, 2), np.float32),
+                    reward=alloc((n,), np.float32), done=alloc((n,), np.uint8), info=alloc((n, I["STRIDE"]), np.float32),
+                    terminal_obs=alloc((n, Cc, H, W), np.uint8))
+    pageable = host_arrays(np.zeros)
+    pinned = host_arrays(lambda shape, dt: torch.from_numpy(np.zeros(shape, dt)).pin_memory().numpy())
+    rng = np.random.default_rng(5)
+    ndone = []
+    for t in range(2):
+        a = (rng.random((n, 6), dtype=np.float32) * 2 - 1) * 0.3
+        sims[0].step_host(a, **pageable)
+        sims[1].step_host(a, **pinned)
+        dev = sims[2]
+        dev.step(torch.from_numpy(a).cuda())
+        ref = dict(obs=dev.obs, achieved=dev.achieved_goal, desired=dev.desired_goal, reward=dev.reward, done=dev.done, info=dev.info)
+        ref = {k: v.cpu().numpy() for k, v in ref.items()}
+        done = ref["done"] != 0
+        ndone.append(int(done.sum()))
+        tobs = dev.terminal_obs.cpu().numpy()
+        for name, h in (("pageable", pageable), ("pinned", pinned)):
+            for k, v in ref.items():
+                assert h[k].tobytes() == v.tobytes(), "%s differs at step %d (%s host arrays)" % (k, t, name)
+            assert np.array_equal(h["terminal_obs"][done], tobs[done]), "terminal_obs differs at step %d (%s host arrays)" % (t, name)
+    assert ndone[0] <= n // 8 < ndone[1], "the tape missed a terminal-observation copy branch: %s environments done" % ndone
+    for s in sims:
+        s.close()
 
 
 def test_separation_budget_skip_is_exact():

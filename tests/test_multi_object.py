@@ -1,7 +1,9 @@
 """GPU: mixed simulators (grs_create_scenes) — several object scenes in one simulator, one variant per environment and episode.
 
 * bit-identity: environment n of a mixed simulator computes exactly what environment n of the single-scene simulator of its
-  variant computes (step outputs with auto-resets and reset noise, renders of every camera, a substep);
+  variant computes (step outputs with auto-resets and reset noise, renders of every camera, a substep); the mixed simulator
+  reads the convex hulls from global memory and the single-scene ones from shared memory, so this also holds the two hull
+  placements of the step kernel against each other;
 * next_object: a written variant takes effect at that environment's next auto-reset or explicit reset, and nowhere else;
 * the asynchronous pool and SAC work over a mixed simulator unchanged;
 * create errors: no scenes, too many scenes, a scene that differs in a shared field.
@@ -46,6 +48,9 @@ def test_mixed_rows_equal_single_scene_rows():
     singles = [_sim(s, N, **cfg) for s in SCENES]
     assert mixed.scenes[2].endswith("bread_crumb_env.xml") and len(mixed.scenes) == 4
     assert tuple(mixed.reset_obs.shape) == (4,) + mixed.obs_shape and tuple(singles[0].reset_obs.shape) == singles[0].obs_shape
+    # step_smem[1]: hull vertices staged in shared memory (DESIGN.md §3.6: the four hulls together do not fit beside the models)
+    assert mixed.get("step_smem")[1] == 0, "the mixed simulator no longer reads the hull from global memory"
+    assert all(s.get("step_smem")[1] == 1 for s in singles), "a single-scene simulator no longer stages the hull in shared memory"
     obj = mixed.object_ids.long()
     assert torch.equal(obj.cpu(), torch.arange(N) % 4) and torch.equal(mixed.next_object_ids.long(), obj)
     rows = torch.arange(N, device="cuda")
